@@ -9,6 +9,7 @@ hot path over the whole resident database shard for all queries.
   python bench.py [--gpus N] [--steps K] [--warmup W]            our arm
   python bench.py --impl reference [...]                         CPU arm (oracle port, all host threads)
   torchrun --nproc-per-node N bench.py --gpus N ...              one rank per GPU, no collective on the data path
+  python bench.py ... --dump-outputs DIR                         also write the last timed step's scores to DIR/*.npy
 
 Prints ONE JSON line (rank 0).  `value` = device-resident kernel throughput (CUDA events on
 the launching stream, max over ranks); `e2e` = the same metric through sw_score_batch /
@@ -35,6 +36,7 @@ SEED = 20160912
 SM_COUNT = 148
 PIPE_PROFILE = "profiles/r01_pipe_pairs_1024thr.json"
 SASS_PROFILE = "profiles/r02_sass_hotloop.json"
+DUMP_BYTES = 60_000_000
 
 
 def measured_r_int():
@@ -170,8 +172,10 @@ def run_reference(args, rank, world):
                                        nthreads=host_threads())
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        _, used = o.score_batch_packed(q[0], q[1], q[2], db[0], db[1], db[2], nthreads=host_threads())
+        scores, used = o.score_batch_packed(q[0], q[1], q[2], db[0], db[1], db[2], nthreads=host_threads())
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, scores)
     gcups = cells * args.steps / dt / 1e9
     sample = (f"each step scores the first {ns} of the {args.subjects} synthetic 150-nt subjects x {args.queries} "
               f"queries ({cells:.3g} cells); GCUPS is a rate, so the bounded sample does not change the metric")
@@ -219,6 +223,20 @@ def log(*a):
 def matrices_equal(a, b):
     """Row-wise comparison of two score matrices of possibly different integer width."""
     return a.shape == b.shape and all(np.array_equal(a[i], b[i]) for i in range(a.shape[0]))
+
+
+def dump_outputs(path, scores):
+    """Writes the [queries, subjects] score matrix the timed path returned as float32, which holds every
+    score exactly.  A matrix above DUMP_BYTES (the default GPU workload's is 4 GB) is cut to a fixed-seed
+    sample of its columns, sorted; subject_index.npy names the columns kept.  Two builds run with the
+    same arguments score the same inputs, so their files compare element for element."""
+    nq, ns = scores.shape
+    ncol = min(ns, DUMP_BYTES // (4 * nq + 8))
+    idx = np.sort(np.random.default_rng(SEED).choice(ns, size=ncol, replace=False))
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, "scores.npy"), scores[:, idx].astype(np.float32))
+    np.save(os.path.join(path, "subject_index.npy"), idx.astype(np.float64))
+    log(f"wrote scores of {ncol} of {ns} subjects x {nq} queries to {path}")
 
 
 def e2e_loop(eng, hdb, out, steps):
@@ -279,7 +297,7 @@ def main():
     capture_stdout()
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=3)
+    ap.add_argument("--steps", type=int, default=3, help="timed steps (at least 1)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--subjects", type=int, default=10_000_000, help="subjects per GPU")
@@ -295,7 +313,12 @@ def main():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-single-handle", action="store_true")
     ap.add_argument("--no-configs", action="store_true", help="skip the configs{} / latency{} blocks")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="after the timed steps, write the score matrix of the last one (rank 0's shard; a "
+                         "fixed-seed sample of its columns) to DIR/scores.npy + DIR/subject_index.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
 
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -370,6 +393,8 @@ def main():
     # spot check: the timed output is the real thing (compare a slice with an independent launch)
     chk = eng.fetch_db()
     checksum = int(chk[:, :: max(1, args.subjects // 4096)].astype(np.int64).sum())
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, chk)
 
     # ---- end-to-end arm: host buffers in, host scores out, every step -----------------------
     e2e = None
