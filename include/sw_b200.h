@@ -151,7 +151,8 @@ int sw_fetch_best(sw_handle_t *h, int32_t *best_score, uint64_t *best_index, int
 
 /* ---- output path ------------------------------------------------------------
  * The bank returns a 12-bit score per (ID) slot (ScoreBank_v2.v:39-41); the result buffer the
- * reference planned (CAPI_template/ResBuffer.v:11-22) has ports only.  Three shapes here:
+ * reference planned (CAPI_template/ResBuffer.v:11-22) has ports only.  Four shapes here (the fourth, the hit
+ * list of sw_set_hits, is described below):
  *   SW_OUTPUT_I32   int32 matrix [rows][ns]                     (default; sw_fetch / sw_fetch_db)
  *   SW_OUTPUT_I16   int16 matrix [rows][ns]: half the HBM and half the D2H bytes.  A score above
  *                   32767 is stored as -1 in the matrix and returned exactly by sw_fetch_overflow
@@ -178,6 +179,28 @@ int sw_fetch_overflow(sw_handle_t *h, uint64_t *flat_index, int32_t *score, size
  * cap = entries both arrays hold (>= rows * k). */
 int sw_fetch_topk(sw_handle_t *h, int32_t *scores, uint64_t *index, size_t cap, int timeout_ms);
 int sw_fetch_db_topk(sw_handle_t *h, int32_t *scores, uint64_t *index, size_t cap);
+
+/* Hit list: every (row, subject) pair with score >= min_score, in place of a matrix.  Replaces the bank's
+ * (IDs, results, vld) stream (ScoreBank_v2.v:39-41), filtered on `results`.  min_score >= 1 turns it on,
+ * 0 turns it off (back to matrices).  Each GPU's list holds max_hits entries per batch slot.
+ *   Entries: exactly the entries of the int32 matrix that are >= min_score -- row = query row (row nq + i =
+ *   reverse complement of query i with sw_set_strands(h, 1)), index = input index within the batch (ids via
+ *   sw_fetch_ids), score = the exact int32 score, above 32767 too -- in row-major order (row ascending, then
+ *   index ascending), the same for every kernel, work order and GPU count.  The int16 / int32 output setting is
+ *   ignored while hits are on.
+ *   Setting: like the other modes, only while no batch is in flight (SW_EAGAIN), and scored batches become
+ *   stale.  Hits and top-k exclude each other (SW_EINVAL either way round); min_score < 0, min_score > 0 with
+ *   max_hits == 0 or max_hits > 2^31 - 1 is SW_EINVAL.  Submitting with the forced 32-bit scorer
+ *   (sw_set_kernel_choice force32) is SW_EINVAL; nothing is enqueued then.
+ *   Fetching: *count = the exact number of hits.  cap < *count: SW_ECAPACITY, nothing written, the batch stays
+ *   fetchable and a retry with larger arrays returns the same list without rescoring (cap = 0 with null arrays
+ *   is the size query).  A GPU that found more than max_hits hits, or more scores beyond 16 bits than the side
+ *   list holds: SW_ERANGE, nothing written, the batch is consumed (raise max_hits or min_score and score
+ *   again).  Fetching a hits batch with a matrix / top-k / best-hit call, or a batch of another mode with these
+ *   two, is SW_ESTATE. */
+int sw_set_hits(sw_handle_t *h, int32_t min_score, size_t max_hits);
+int sw_fetch_hits(sw_handle_t *h, uint32_t *row, uint64_t *index, int32_t *score, size_t cap, size_t *count, int timeout_ms);
+int sw_fetch_db_hits(sw_handle_t *h, uint32_t *row, uint64_t *index, int32_t *score, size_t cap, size_t *count);
 
 /* ---- introspection --------------------------------------------------------- */
 const char *sw_strerror(int code);

@@ -11,6 +11,7 @@ capi_sample_aligner/software-C,C++/src/main_test.c:290-528):
     Engine.set_queries(...)                          <- type-01 record, ld_q
     Engine.score_batch(...)                          <- stream of type-10 records
     Engine.fetch(timeout_ms)                         <- (IDs, results, vld) + WED poll, result-2048
+    Engine.fetch_hits(timeout_ms)                    <- the same stream filtered on results >= min_score
 """
 import ctypes as C
 import os
@@ -103,6 +104,9 @@ def load_library():
     L.sw_fetch_overflow.argtypes = [vp, vp, vp, sz, C.POINTER(sz)]
     L.sw_fetch_topk.argtypes = [vp, vp, vp, sz, i32]
     L.sw_fetch_db_topk.argtypes = [vp, vp, vp, sz]
+    L.sw_set_hits.argtypes = [vp, C.c_int32, sz]
+    L.sw_fetch_hits.argtypes = [vp, vp, vp, vp, sz, C.POINTER(sz), i32]
+    L.sw_fetch_db_hits.argtypes = [vp, vp, vp, vp, sz, C.POINTER(sz)]
     L.sw_device_error_bits.argtypes = [vp]
     L.sw_device_error_bits.restype = C.c_uint
     L.sw_is_check_build.restype = i32
@@ -153,6 +157,7 @@ class Engine:
         self._batch_ns = []  # subjects of the batches in flight, oldest first
         self.out_mode = SW_OUTPUT_I32
         self.topk = 0
+        self.hits = 0        # min_score of the hit-list mode (0 = off)
         self._ids_ns = 0     # subjects of the batch sw_fetch_ids refers to (last loaded / fetched)
 
     # -- plumbing ---------------------------------------------------------------------
@@ -253,6 +258,37 @@ class Engine:
         ix = np.empty((self.nq, self.topk), dtype=np.uint64)
         self._check(self.lib.sw_fetch_db_topk(self.h, _ptr(sc), _ptr(ix), sc.size))
         return sc, ix
+
+    def set_hits(self, min_score, max_hits=1 << 24):
+        """min_score >= 1: instead of a matrix, list every (row, subject) pair scoring >= min_score
+        (fetch_hits / fetch_db_hits); each GPU's list holds max_hits entries.  0 = back to matrices."""
+        self._check(self.lib.sw_set_hits(self.h, int(min_score), int(max_hits)))
+        self.hits = int(min_score)
+
+    def _hits(self, call):
+        cnt = C.c_size_t(0)
+        rc = call(None, None, None, 0, C.byref(cnt))            # size query (SW_OK with no hits at all)
+        row = np.empty(cnt.value if rc == SW_ECAPACITY else 0, dtype=np.uint32)
+        idx = np.empty(row.size, dtype=np.uint64)
+        sc = np.empty(row.size, dtype=np.int32)
+        if rc == SW_ECAPACITY:
+            rc = call(_ptr(row), _ptr(idx), _ptr(sc), row.size, C.byref(cnt))
+        return rc, row, idx, sc
+
+    def fetch_hits(self, timeout_ms=-1):
+        """(row uint32, index uint64, score int32) of the oldest batch in flight: every entry of its int32
+        matrix >= min_score, row-major order; index = input index in the batch."""
+        rc, row, idx, sc = self._hits(lambda r, i, s, cap, cnt: self.lib.sw_fetch_hits(self.h, r, i, s, cap, cnt, timeout_ms))
+        if self._batch_ns and rc in (SW_OK, SW_ERANGE):          # SW_ERANGE consumes the batch too
+            self._ids_ns = self._batch_ns.pop(0)
+        self._check(rc)
+        return row, idx, sc
+
+    def fetch_db_hits(self):
+        """fetch_hits for the resident database (after score_db)."""
+        rc, row, idx, sc = self._hits(lambda r, i, s, cap, cnt: self.lib.sw_fetch_db_hits(self.h, r, i, s, cap, cnt))
+        self._check(rc)
+        return row, idx, sc
 
     def set_jit(self, mode):
         self._check(self.lib.sw_set_jit(self.h, mode))

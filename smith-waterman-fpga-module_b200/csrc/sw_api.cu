@@ -21,6 +21,8 @@
 #include "sw_jit.h"
 #include "sw_kernels.h"
 
+#include <cub/device/device_radix_sort.cuh>
+
 #include <algorithm>
 #include <atomic>
 #include <chrono>
@@ -117,9 +119,10 @@ struct Slot {
     size_t s0 = 0, s1 = 0;            // global subject range [s0, s1) of this GPU's shard
     DevBuf d_raw, d_off, d_len, d_pair_subj, d_pair_len, d_tile_woff, d_tp, d_out;
     DevBuf d_ovf_count, d_ovf_list, d_ovf_score, d_topk_out;
+    DevBuf d_hits_key, d_hits_score, d_hits_count;   // hit list of the last scoring (reserved at the first one in hits mode)
     uint32_t npairs = 0, max_len = 0;
     uint64_t sum_len = 0, tp_words = 0;
-    PinnedBuf h_stage_a, h_stage_b, h_stage_c, h_stage_d, h_topk, h_ovf;
+    PinnedBuf h_stage_a, h_stage_b, h_stage_c, h_stage_d, h_topk, h_ovf, h_hits;
     cudaEvent_t ev_start = nullptr, ev_stop = nullptr, ev_upload = nullptr;
     std::vector<cudaEvent_t> ev_pool;  // chunk-done events, created once
     std::vector<QueryChunk> chunks;
@@ -132,6 +135,7 @@ struct Slot {
     bool ovf_used = false;
     int out_mode = SW_OUT_I32;         // of the last scoring
     int topk_k = 0;
+    int hits_shift = 0;                // hit keys: row << hits_shift | shard-local subject
     // small (latency) path: one staging buffer in, mapped scores out
     bool is_small = false;
     PinnedBuf h_small_in, h_small_out, h_small_flag;
@@ -158,7 +162,8 @@ struct GpuCtx {
     DevBuf d_wave_bnd, d_wave_state;  // band-pipelined kernel: boundary rows; progress / best / done words
     int wave_bps[16] = {0};           // resident blocks per SM of its instances (0 = not asked yet)
     DevBuf d_wave32_bnd, d_wave32_state;   // 32-bit band-pipelined scorer of the overflow list
-    DevBuf d_wave_rows;               // top-k mode: one scratch score row per band-pipelined query
+    DevBuf d_wave_rows;               // top-k / hits mode: one scratch score row per band-pipelined query
+    DevBuf d_hits_key2, d_hits_score2, d_sort_tmp;   // fetch of a hit list: radix-sort output and temp storage (copy stream)
     uint32_t wave32_epoch = 0;        // 8-bit tag field: 1 .. 255, boundary rows zeroed when it restarts
     int wave32_bps = 0;
     uint32_t wave_epoch = 0;          // launches so far: the tag of the boundary elements (20 bits)
@@ -176,6 +181,12 @@ struct Batch {
     int nq = 0;                       // query rows the scores of this batch have
     bool loaded = false, scored = false, small = false;
     int out_mode = SW_OUT_I32, topk_k = 0;
+    int32_t hits_min = 0;             // > 0: scored in hits mode with this threshold
+    size_t hits_max = 0;
+    bool hits_staged = false;         // the stitched list below waits for a fetch with enough room
+    std::vector<uint32_t> hits_row;
+    std::vector<uint64_t> hits_index;
+    std::vector<int32_t> hits_score;
     std::vector<uint64_t> ids;
     bool have_ids = false;
     uint64_t cells = 0;
@@ -202,6 +213,8 @@ struct sw_handle {
     int last_slot = 0;                // slot of the most recent load / fetch (ids, cells, overflow list)
     int out_mode = SW_OUT_I32;        // SW_OUTPUT_I32 / SW_OUTPUT_I16 for the next scoring
     int topk_k = 0;                   // > 0: fused top-k instead of a matrix
+    int32_t hits_min = 0;             // > 0: hit list (scores >= hits_min) instead of a matrix
+    size_t hits_max = 0;              // entries of each GPU's hit list
     bool small_path = true;
     bool small_timing = true;         // record CUDA events around the latency path's kernel (sw_last_kernel_ms)
     int jit = 1;                      // run-time specialisation of gap penalties: 0 off, 1 large jobs, 2 always
@@ -276,10 +289,12 @@ std::vector<DevBuf *> all_devbufs(GpuCtx &g)
 {
     std::vector<DevBuf *> v = {&g.d_qpacked, &g.d_qoff, &g.d_qlen, &g.d_qidx, &g.d_bnd, &g.d_counters, &g.d_scratch32,
                                &g.d_best_score, &g.d_best_index, &g.d_topk_keys, &g.d_err, &g.d_wave_bnd, &g.d_wave_state, &g.d_wave32_bnd, &g.d_wave32_state, &g.d_wave_rows,
-                               &g.d_bnd_aux[0], &g.d_bnd_aux[1], &g.d_bnd_aux[2], &g.d_part_done, &g.d_part_best};
+                               &g.d_bnd_aux[0], &g.d_bnd_aux[1], &g.d_bnd_aux[2], &g.d_part_done, &g.d_part_best,
+                               &g.d_hits_key2, &g.d_hits_score2, &g.d_sort_tmp};
     for (Slot &b : g.slot) {
         DevBuf *bufs[] = {&b.d_raw, &b.d_off, &b.d_len, &b.d_pair_subj, &b.d_pair_len, &b.d_tile_woff, &b.d_tp, &b.d_out,
-                          &b.d_ovf_count, &b.d_ovf_list, &b.d_ovf_score, &b.d_topk_out, &b.d_small_in, &b.d_small_done};
+                          &b.d_ovf_count, &b.d_ovf_list, &b.d_ovf_score, &b.d_topk_out, &b.d_small_in, &b.d_small_done,
+                          &b.d_hits_key, &b.d_hits_score, &b.d_hits_count};
         v.insert(v.end(), std::begin(bufs), std::end(bufs));
     }
     return v;
@@ -293,7 +308,7 @@ void free_gpu(GpuCtx &g)
         for (cudaEvent_t e : b.ev_pool) cudaEventDestroy(e);
         b.ev_pool.clear();
         b.chunks.clear();
-        PinnedBuf *pins[] = {&b.h_stage_a, &b.h_stage_b, &b.h_stage_c, &b.h_stage_d, &b.h_topk, &b.h_ovf, &b.h_small_in, &b.h_small_out,
+        PinnedBuf *pins[] = {&b.h_stage_a, &b.h_stage_b, &b.h_stage_c, &b.h_stage_d, &b.h_topk, &b.h_ovf, &b.h_hits, &b.h_small_in, &b.h_small_out,
                              &b.h_small_flag};
         for (PinnedBuf *p : pins) p->release();
         if (b.ev_start) cudaEventDestroy(b.ev_start);
@@ -845,13 +860,27 @@ int score_gpu(sw_handle *h, GpuCtx &gc, Slot &g)
     g.chunks.clear();
     g.scored = true;
     g.ovf_used = false;
-    g.out_mode = h->topk_k > 0 ? SW_OUT_TOPK : h->out_mode;
+    g.out_mode = h->topk_k > 0 ? SW_OUT_TOPK : h->hits_min > 0 ? SW_OUT_HITS : h->out_mode;
     g.topk_k = h->topk_k;
     if (n == 0 || nq == 0) return SW_OK;
     const bool topk = g.out_mode == SW_OUT_TOPK;
+    const bool hits = g.out_mode == SW_OUT_HITS;
     const size_t esz = g.out_mode == SW_OUT_I16 ? sizeof(int16_t) : sizeof(int32_t);
 
-    if (!topk) {
+    // hit list: keys row << hits_shift | shard-local subject (the fetch sorts them: row-major order)
+    SwHitList hl;
+    if (hits) {
+        int sb = 0;
+        while ((1ull << sb) < (uint64_t)n) ++sb;
+        g.hits_shift = sb;
+        SW_CUDA(h, g.d_hits_count.reserve(sizeof(unsigned long long)));
+        SW_CUDA(h, g.d_hits_key.reserve(h->hits_max * sizeof(unsigned long long)));
+        SW_CUDA(h, g.d_hits_score.reserve(h->hits_max * sizeof(int32_t)));
+        SW_CUDA(h, cudaMemsetAsync(g.d_hits_count.p, 0, sizeof(unsigned long long), gc.st_compute));
+        hl.keys = g.d_hits_key.as<unsigned long long>(); hl.score = g.d_hits_score.as<int32_t>();
+        hl.count = g.d_hits_count.as<unsigned long long>(); hl.cap = (unsigned)h->hits_max;
+        hl.min_score = h->hits_min; hl.shift = sb;
+    } else if (!topk) {
         SW_CUDA(h, g.d_out.reserve((size_t)nq * n * esz));
         SW_CUDA(h, cudaMemsetAsync(g.d_out.p, 0, (size_t)nq * n * esz, gc.st_compute));
     } else {
@@ -937,7 +966,9 @@ int score_gpu(sw_handle *h, GpuCtx &gc, Slot &g)
 
     SwStripLaunch base;
     base.db = db; base.q = dq; base.sc = sc;
-    base.out = topk ? nullptr : g.d_out.p; base.out_stride = n; base.out_elems = (size_t)nq * n; base.out_mode = g.out_mode;
+    base.out = (topk || hits) ? nullptr : g.d_out.p; base.out_stride = n; base.out_elems = hits ? h->hits_max : (size_t)nq * n;
+    base.out_mode = g.out_mode;
+    base.hits = hl;
     base.dev_err = gc.d_err.as<unsigned>();
     if (may_overflow) {
         SW_CUDA(h, g.d_ovf_count.reserve(sizeof(unsigned)));
@@ -978,7 +1009,7 @@ int score_gpu(sw_handle *h, GpuCtx &gc, Slot &g)
                 // the last round partly empty.  With the pass split that round costs a fraction of a part, so a
                 // one-lane variant is the faster one as soon as its chains fill the GPU once
                 // (scripts/split_ab.py: 10 kb x 120 000 x 1 kb: R38x1_G4 7 014, band-pipelined 7 340, R32x2_G1 8 390 GCUPS).
-                const int nchunks_est = (topk || may_overflow || !wave_q.empty()) ? 1 : std::max(1, std::min(std::min(nq, 8), (int)(est_ms_all / 50.0)));
+                const int nchunks_est = (topk || hits || may_overflow || !wave_q.empty()) ? 1 : std::max(1, std::min(std::min(nq, 8), (int)(est_ms_all / 50.0)));
                 const uint64_t nql_launch = (uint64_t)std::max(1, nq / nchunks_est);
                 for (int cand : ranked) {
                     const SwStripVariant *cv = sw_strip_variant(cand);
@@ -1002,7 +1033,10 @@ int score_gpu(sw_handle *h, GpuCtx &gc, Slot &g)
                 for (uint64_t x : parts) { key ^= x; key *= 1099511628211ull; }
                 if (gc.tune_key != key || gc.tune_choice < 0) {
                     int choice = vidx;
-                    rc = autotune_variant(h, gc, g, base, ranked, nq, same_len, &choice);
+                    // the sample launches append nothing: a pair they score is scored again by the real launch
+                    SwStripLaunch sample = base;
+                    if (hits) { sample.hits.keys = nullptr; sample.ovf_list = nullptr; sample.ovf_count = nullptr; }
+                    rc = autotune_variant(h, gc, g, sample, ranked, nq, same_len, &choice);
                     if (rc != SW_OK) return rc;
                     gc.tune_choice = choice;
                     gc.tune_key = key;
@@ -1012,7 +1046,7 @@ int score_gpu(sw_handle *h, GpuCtx &gc, Slot &g)
             // query chunks: a handful of launches so that D2H of finished rows overlaps compute
             // (each launch has its own tail: aim for >= ~50 ms of work per launch, at ~6 TCUPS)
             int nchunks = std::max(1, std::min(std::min(nq, 8), (int)(est_ms_all / 50.0)));
-            if (topk || may_overflow || !wave_q.empty()) nchunks = 1;
+            if (topk || hits || may_overflow || !wave_q.empty()) nchunks = 1;
             // the device work counter is 32-bit: (pair blocks) x (queries per launch) must stay below 2^31
             while (nchunks < nq && (uint64_t)(g.npairs / 4 + 1) * (uint64_t)((nq + nchunks - 1) / nchunks) >= (1ull << 31)) nchunks *= 2;
             nchunks = std::min(nchunks, nq);
@@ -1185,15 +1219,17 @@ int score_gpu(sw_handle *h, GpuCtx &gc, Slot &g)
     const bool use32 = !have_strip && wave_q.empty();        // forced 32-bit scorer
     if (topk) {
         if (!have_strip && wave_q.empty()) return SW_EINVAL;  // the 32-bit scorer has no top-k epilogue
-        if (!wave_q.empty()) {
-            max_grid = std::max(max_grid, 1);                 // list 0 also takes the rows of the band-pipelined queries
-            const size_t rb = wave_q.size() * (size_t)n * sizeof(int32_t);
-            SW_CUDA(h, gc.d_wave_rows.reserve(rb));
-            SW_CUDA(h, cudaMemsetAsync(gc.d_wave_rows.p, 0xFF, rb, gc.st_compute));    // -1 = not scored here
-        }
+        if (!wave_q.empty()) max_grid = std::max(max_grid, 1);      // list 0 also takes the rows of the band-pipelined queries
         const size_t bytes = (size_t)max_grid * nq * g.topk_k * sizeof(unsigned long long);
         SW_CUDA(h, gc.d_topk_keys.reserve(bytes));
         SW_CUDA(h, cudaMemsetAsync(gc.d_topk_keys.p, 0, bytes, gc.st_compute));
+    }
+
+    if (hits && use32) return SW_EINVAL;                      // (rejected at submit: the 32-bit scorer has no hit list)
+    if ((topk || hits) && !wave_q.empty()) {
+        const size_t rb = wave_q.size() * (size_t)n * sizeof(int32_t);
+        SW_CUDA(h, gc.d_wave_rows.reserve(rb));
+        SW_CUDA(h, cudaMemsetAsync(gc.d_wave_rows.p, 0xFF, rb, gc.st_compute));    // -1 = not scored here
     }
 
     // 32-bit scratch (force32, or the overflow fix-up of the few listed pairs)
@@ -1208,12 +1244,12 @@ int score_gpu(sw_handle *h, GpuCtx &gc, Slot &g)
         SW_CUDA(h, gc.d_scratch32.reserve((size_t)2 * max_cols * threads32 * sizeof(int32_t)));
     }
     SwScore32Launch s32;
-    s32.db = db; s32.q = dq; s32.sc = sc; s32.out = topk ? nullptr : g.d_out.p; s32.out_stride = n; s32.out_mode = g.out_mode;
+    s32.db = db; s32.q = dq; s32.sc = sc; s32.out = (topk || hits) ? nullptr : g.d_out.p; s32.out_stride = n; s32.out_mode = g.out_mode;
     s32.scratch = gc.d_scratch32.as<int32_t>(); s32.max_cols = max_cols; s32.threads_total = threads32;
 
     size_t nev = 0;
     if (!use32) {
-        const bool chunk_events = simple && plan.size() > 1 && !may_overflow && !topk;
+        const bool chunk_events = simple && plan.size() > 1 && !may_overflow && !topk && !hits;
         bool forked[kStreams] = {false, false, false, false};
         for (size_t i = 0; i < plan.size(); ++i) {
             Planned &p = plan[i];
@@ -1290,9 +1326,9 @@ int score_gpu(sw_handle *h, GpuCtx &gc, Slot &g)
                 W.db = db; W.q = dq; W.query = q; W.sc = sc;
                 W.npass = (int)((h->q_len[q] + rows - 1) / rows);
                 W.out = g.d_out.p; W.out_stride = n; W.out_mode = g.out_mode;
-                if (topk) { W.out = gc.d_wave_rows.p; W.out_mode = SW_OUT_I32; W.out_row = wave_row; }
+                if (topk || hits) { W.out = gc.d_wave_rows.p; W.out_mode = SW_OUT_I32; W.out_row = wave_row; }
                 W.bnd = gc.d_wave_bnd.p; W.cols_stride = cols_stride;
-                W.bnd_elems = (size_t)g.npairs * 2 * cols_stride; W.out_elems = topk ? wave_q.size() * (size_t)n : (size_t)nq * n;
+                W.bnd_elems = (size_t)g.npairs * 2 * cols_stride; W.out_elems = (topk || hits) ? wave_q.size() * (size_t)n : (size_t)nq * n;
                 gc.wave_epoch = (gc.wave_epoch % 0xFFFFEu) + 1u;            // 1 .. 2^20 - 2
                 if (gc.wave_epoch == 1u && gc.counter_next > 0) {
                     // the epoch wrapped (or first use): stale tags must not match again
@@ -1316,6 +1352,11 @@ int score_gpu(sw_handle *h, GpuCtx &gc, Slot &g)
                     // scorer keep the sentinel here and reach the merge through the overflow list)
                     SW_CUDA(h, sw_launch_topk_row(gc.st_compute, (const int32_t *)gc.d_wave_rows.p + (size_t)wave_row * n, (uint32_t)n, q,
                                                   g.topk_k, gc.d_topk_keys.as<unsigned long long>()));
+                    h->launches++;
+                }
+                if (hits) {
+                    // the row's entries >= min_score join the list (flagged pairs come from the overflow list)
+                    SW_CUDA(h, sw_launch_hits_row(gc.st_compute, (const int32_t *)gc.d_wave_rows.p + (size_t)wave_row * n, (uint32_t)n, q, hl));
                     h->launches++;
                 }
                 if (&gc == &h->gpus[0] && label_v < 0)
@@ -1373,6 +1414,10 @@ int score_gpu(sw_handle *h, GpuCtx &gc, Slot &g)
             }
             SW_CUDA(h, sw_launch_score32(gc.st_compute, s32));
             h->launches++;
+            if (hits) {
+                SW_CUDA(h, sw_launch_hits_ovf(gc.st_compute, s32.list_count, s32.list, s32.list_score, kOvfCap, hl));
+                h->launches++;
+            }
         }
         if (topk) {
             SW_CUDA(h, sw_launch_topk_merge(gc.st_compute, gc.d_topk_keys.as<unsigned long long>(), max_grid, nq, g.topk_k,
@@ -1457,6 +1502,7 @@ int fetch_slot(sw_handle *h, int si, FetchKind kind, void *scores, uint64_t *ind
     const bool forever = timeout_ms < 0;
     const auto t_fetch0 = std::chrono::steady_clock::now();
     const auto t_end = t_fetch0 + std::chrono::milliseconds(forever ? 0 : timeout_ms);
+    if (bt.hits_min > 0) return SW_ESTATE;                  // a hits batch has no matrix / top-k lists
     if (kind == FETCH_TOPK) {
         if (bt.topk_k <= 0) return SW_ESTATE;
         if (cap < nq * (size_t)bt.topk_k) return SW_ECAPACITY;
@@ -1637,6 +1683,116 @@ int fetch_slot(sw_handle *h, int si, FetchKind kind, void *scores, uint64_t *ind
     return SW_OK;
 }
 
+// Hit list of a batch: per GPU wait for the kernels, read the count, radix-sort the list by (row, subject) and copy
+// it to pinned staging -- on the copy stream, so that the next batch's kernels keep running -- then stitch the
+// shards on the host.  Shards are contiguous input ranges in GPU order, so row-major order = for every row, the
+// run of GPU 0, then of GPU 1, ...  The stitched list stays in the Batch until a fetch has room for it.
+int fetch_hits_slot(sw_handle *h, int si, uint32_t *row, uint64_t *index, int32_t *score, size_t cap, size_t *count, int timeout_ms)
+{
+    Batch &bt = h->batch[si];
+    if (bt.hits_min <= 0) return SW_ESTATE;
+    const bool forever = timeout_ms < 0;
+    const auto t_fetch0 = std::chrono::steady_clock::now();
+    const auto t_end = t_fetch0 + std::chrono::milliseconds(forever ? 0 : timeout_ms);
+    if (!bt.hits_staged) {
+        const size_t ng = h->gpus.size();
+        std::vector<unsigned long long> cnt(ng, 0);
+        bool too_many = false;
+        for (size_t gi = 0; gi < ng; ++gi) {
+            GpuCtx &g = h->gpus[gi];
+            Slot &b = g.slot[si];
+            if (b.s1 == b.s0 || bt.nq == 0 || b.chunks.empty()) continue;
+            SW_CUDA(h, cudaSetDevice(g.dev));
+            int rc = wait_event(h, b.chunks.back().done, t_end, forever);
+            if (rc != SW_OK) return rc;
+            SW_CUDA(h, cudaMemcpy(&cnt[gi], b.d_hits_count.p, sizeof(unsigned long long), cudaMemcpyDeviceToHost));
+            too_many |= cnt[gi] > bt.hits_max;
+            if (b.ovf_used) {
+                unsigned novf = 0;
+                SW_CUDA(h, cudaMemcpy(&novf, b.d_ovf_count.p, sizeof novf, cudaMemcpyDeviceToHost));
+                too_many |= novf > kOvfCap;
+            }
+        }
+        const auto t_fetch1 = std::chrono::steady_clock::now();
+        *count = 0;
+        for (unsigned long long c : cnt) *count += (size_t)c;
+        if (too_many) return SW_ERANGE;
+        int row_bits = 0;
+        while ((1ull << row_bits) < (uint64_t)bt.nq) ++row_bits;
+        for (size_t gi = 0; gi < ng; ++gi) {
+            GpuCtx &g = h->gpus[gi];
+            Slot &b = g.slot[si];
+            const size_t c = (size_t)cnt[gi];
+            if (c == 0) continue;
+            SW_CUDA(h, cudaSetDevice(g.dev));
+            const int end_bit = std::max(1, b.hits_shift + row_bits);          // only the key bits in use
+            // sized for max_hits (a count never exceeds it here): a buffer that grows would be freed, and cudaFree
+            // waits for the whole device -- the next batch's kernels included
+            if (g.d_hits_key2.cap < bt.hits_max * sizeof(unsigned long long) || g.d_hits_score2.cap < bt.hits_max * sizeof(int32_t)) {
+                SW_CUDA(h, g.d_hits_key2.reserve(bt.hits_max * sizeof(unsigned long long)));
+                SW_CUDA(h, g.d_hits_score2.reserve(bt.hits_max * sizeof(int32_t)));
+            }
+            size_t tmp = 0;
+            SW_CUDA(h, cub::DeviceRadixSort::SortPairs(nullptr, tmp, b.d_hits_key.as<unsigned long long>(), g.d_hits_key2.as<unsigned long long>(),
+                                                      b.d_hits_score.as<int32_t>(), g.d_hits_score2.as<int32_t>(), (int)bt.hits_max, 0, 64, g.st_copy));
+            SW_CUDA(h, g.d_sort_tmp.reserve(tmp));
+            tmp = g.d_sort_tmp.cap;
+            SW_CUDA(h, cub::DeviceRadixSort::SortPairs(g.d_sort_tmp.p, tmp, b.d_hits_key.as<unsigned long long>(), g.d_hits_key2.as<unsigned long long>(),
+                                                      b.d_hits_score.as<int32_t>(), g.d_hits_score2.as<int32_t>(), (int)c, 0, end_bit, g.st_copy));
+            h->launches++;
+            SW_CUDA(h, b.h_hits.reserve((size_t)c * (sizeof(unsigned long long) + sizeof(int32_t))));
+            SW_CUDA(h, cudaMemcpyAsync(b.h_hits.p, g.d_hits_key2.p, (size_t)c * sizeof(unsigned long long), cudaMemcpyDeviceToHost, g.st_copy));
+            SW_CUDA(h, cudaMemcpyAsync((unsigned long long *)b.h_hits.p + c, g.d_hits_score2.p, (size_t)c * sizeof(int32_t),
+                                       cudaMemcpyDeviceToHost, g.st_copy));
+        }
+        double ms_max = 0.0, ms_min = 1e300;
+        size_t total = 0;
+        for (size_t gi = 0; gi < ng; ++gi) {
+            GpuCtx &g = h->gpus[gi];
+            Slot &b = g.slot[si];
+            SW_CUDA(h, cudaSetDevice(g.dev));
+            SW_CUDA(h, cudaStreamSynchronize(g.st_copy));
+            total += cnt[gi];
+            if (b.scored && b.s1 > b.s0 && bt.nq) {
+                SW_CUDA(h, cudaEventSynchronize(b.ev_stop));
+                float ms = 0.f;
+                SW_CUDA(h, cudaEventElapsedTime(&ms, b.ev_start, b.ev_stop));
+                ms_max = std::max(ms_max, (double)ms);
+                ms_min = std::min(ms_min, (double)ms);
+            }
+        }
+        bt.hits_row.resize(total); bt.hits_index.resize(total); bt.hits_score.resize(total);
+        std::vector<size_t> cur(ng, 0);
+        size_t o = 0;
+        for (int r = 0; r < bt.nq && o < total; ++r) {
+            for (size_t gi = 0; gi < ng; ++gi) {
+                const Slot &b = h->gpus[gi].slot[si];
+                if (cnt[gi] == 0) continue;
+                const unsigned long long *keys = (const unsigned long long *)b.h_hits.p;
+                const int32_t *sc = (const int32_t *)(keys + cnt[gi]);
+                const unsigned long long mask = (1ull << b.hits_shift) - 1ull;
+                for (size_t &k = cur[gi]; k < cnt[gi] && (keys[k] >> b.hits_shift) == (unsigned long long)r; ++k, ++o) {
+                    bt.hits_row[o] = (uint32_t)r; bt.hits_index[o] = b.s0 + (keys[k] & mask); bt.hits_score[o] = sc[k];
+                }
+            }
+        }
+        bt.hits_staged = true;
+        bt.ovf_index.clear(); bt.ovf_score.clear();          // sw_fetch_overflow: nothing for a hits batch
+        finish_timing(h, si, t_fetch0, t_fetch1, ms_max, ms_min);
+        if (device_error_bits(h)) { bt.hits_staged = false; return SW_EDEVICE; }
+    }
+    *count = bt.hits_row.size();
+    if (cap < *count) return SW_ECAPACITY;
+    if (*count) {
+        std::memcpy(row, bt.hits_row.data(), *count * sizeof(uint32_t));
+        std::memcpy(index, bt.hits_index.data(), *count * sizeof(uint64_t));
+        std::memcpy(score, bt.hits_score.data(), *count * sizeof(int32_t));
+    }
+    bt.hits_staged = false;
+    h->last_slot = si;
+    return SW_OK;
+}
+
 int load_batch(sw_handle *h, int si, const uint8_t *packed, const uint32_t *len, const uint64_t *off,
                const uint64_t *ids, size_t ns)
 {
@@ -1685,6 +1841,7 @@ int score_batch_slot(sw_handle *h, int si)
     bt.nq = (int)h->q_len.size();
     bt.out_mode = h->out_mode;
     bt.topk_k = h->topk_k;
+    bt.hits_min = h->hits_min; bt.hits_max = h->hits_max; bt.hits_staged = false;
     h->last_cells = bt.cells;
     const size_t ng = h->gpus.size();
     std::vector<int> rcs(ng, SW_OK);
@@ -1740,7 +1897,8 @@ int small_submit(sw_handle *h, int si, const uint8_t *packed, const uint32_t *le
     *taken = false;
     const int nq = (int)h->q_len.size();
     if (!h->small_path || ns == 0 || nq == 0 || ns > 8192 || (size_t)nq * ns > (1u << 20)) return SW_OK;
-    if (h->topk_k > 0 || h->out_mode != SW_OUT_I32 || h->params.score_width != 0) return SW_OK;
+    // (hits mode: the completion protocol below reads a fixed number of result words, a list has no such end)
+    if (h->topk_k > 0 || h->hits_min > 0 || h->out_mode != SW_OUT_I32 || h->params.score_width != 0) return SW_OK;
     uint64_t bmin = ~0ull, bmax = 0, sum = 0;
     uint32_t maxlen = 0;
     size_t n_empty = 0;
@@ -1774,7 +1932,7 @@ int small_submit(sw_handle *h, int si, const uint8_t *packed, const uint32_t *le
     bt.ns = ns; bt.loaded = true; bt.scored = true; bt.small = true;
     bt.have_ids = ids != nullptr;
     if (ids) bt.ids.assign(ids, ids + ns); else bt.ids.clear();
-    bt.nq = nq; bt.out_mode = SW_OUT_I32; bt.topk_k = 0;
+    bt.nq = nq; bt.out_mode = SW_OUT_I32; bt.topk_k = 0; bt.hits_min = 0; bt.hits_staged = false;
     bt.cells = sum * h->q_sum_len;
     h->last_cells = bt.cells;
     for (auto &gg : h->gpus) { gg.slot[si].s0 = 0; gg.slot[si].s1 = 0; gg.slot[si].chunks.clear(); gg.slot[si].ovf_used = false; }
@@ -1889,6 +2047,9 @@ int fetch_db_common(sw_handle_t *h, FetchKind kind, void *scores, uint64_t *inde
     if (!h->batch[0].loaded || !h->batch[0].scored) return SW_ESTATE;
     return fetch_slot(h, 0, kind, scores, index, cap, -1);
 }
+
+// hits mode with the forced 32-bit scorer: refused before anything is enqueued (that scorer has no hit list)
+bool hits_need_strip(const sw_handle *h) { return h->hits_min > 0 && h->force32; }
 
 int fetch_common(sw_handle_t *h, FetchKind kind, void *scores, uint64_t *index, size_t cap, int timeout_ms)
 {
@@ -2062,11 +2223,40 @@ int sw_set_output(sw_handle_t *h, int mode)
 
 int sw_set_topk(sw_handle_t *h, int k)
 {
-    if (!h || k < 0 || k > SW_MAX_TOPK) return SW_EINVAL;
+    if (!h || k < 0 || k > SW_MAX_TOPK || (k > 0 && h->hits_min > 0)) return SW_EINVAL;
     if (h->n_inflight) return SW_EAGAIN;
     h->topk_k = k;
     for (Batch &bt : h->batch) bt.scored = false;
     return SW_OK;
+}
+
+int sw_set_hits(sw_handle_t *h, int32_t min_score, size_t max_hits)
+{
+    // (the device counter is 32-bit and counts past the list's end; the radix sort takes an int count)
+    if (!h || min_score < 0 || (min_score > 0 && (max_hits == 0 || max_hits > 0x7FFFFFFFu))) return SW_EINVAL;
+    if (min_score > 0 && h->topk_k > 0) return SW_EINVAL;
+    if (h->n_inflight) return SW_EAGAIN;
+    h->hits_min = min_score;
+    h->hits_max = min_score > 0 ? max_hits : 0;
+    for (Batch &bt : h->batch) bt.scored = false;
+    return SW_OK;
+}
+
+int sw_fetch_hits(sw_handle_t *h, uint32_t *row, uint64_t *index, int32_t *score, size_t cap, size_t *count, int timeout_ms)
+{
+    if (!h || !count || (cap && (!row || !index || !score))) return SW_EINVAL;
+    *count = 0;
+    if (h->n_inflight == 0) return SW_ESTATE;
+    return pop_fifo(h, fetch_hits_slot(h, h->fifo[0], row, index, score, cap, count, timeout_ms));
+}
+
+int sw_fetch_db_hits(sw_handle_t *h, uint32_t *row, uint64_t *index, int32_t *score, size_t cap, size_t *count)
+{
+    if (!h || !count || (cap && (!row || !index || !score))) return SW_EINVAL;
+    *count = 0;
+    if (h->n_inflight) return SW_EAGAIN;
+    if (!h->batch[0].loaded || !h->batch[0].scored) return SW_ESTATE;
+    return fetch_hits_slot(h, 0, row, index, score, cap, count, -1);
 }
 
 int sw_set_queries(sw_handle_t *h, const uint8_t *packed, const uint32_t *len, const uint64_t *off, int nq)
@@ -2142,6 +2332,7 @@ int sw_score_db(sw_handle_t *h)
     if (!h) return SW_EINVAL;
     if (h->n_inflight) return SW_EAGAIN;
     if (!h->batch[0].loaded || h->batch[0].small) return SW_ESTATE;
+    if (hits_need_strip(h)) return SW_EINVAL;
     return score_batch_slot(h, 0);
 }
 
@@ -2180,6 +2371,7 @@ int sw_score_batch(sw_handle_t *h, const uint8_t *packed, const uint32_t *len, c
 {
     if (!h || (ns > 0 && (!packed || !len || !off))) return SW_EINVAL;
     if (h->n_inflight >= 2) return SW_EAGAIN;          // both buffers busy: the bank's `full`
+    if (hits_need_strip(h)) return SW_EINVAL;
     // take the slot that is not in flight; this replaces whatever sw_load_db left there
     const int si = (h->n_inflight == 1) ? (1 - h->fifo[0]) : 0;
     bool taken = false;
@@ -2237,7 +2429,7 @@ int sw_fetch_best(sw_handle_t *h, int32_t *best_score, uint64_t *best_index, int
     if (h->n_inflight) return SW_EAGAIN;
     const Batch &bt = h->batch[0];
     const int nq = bt.nq;
-    if (!bt.loaded || !bt.scored || bt.small || bt.topk_k > 0 || bt.out_mode != SW_OUT_I32) return SW_ESTATE;
+    if (!bt.loaded || !bt.scored || bt.small || bt.topk_k > 0 || bt.hits_min > 0 || bt.out_mode != SW_OUT_I32) return SW_ESTATE;
     if (nq_cap < nq) return SW_ECAPACITY;
     for (int q = 0; q < nq; ++q) { best_score[q] = 0; best_index[q] = 0; }
     std::vector<int32_t> hs(nq);

@@ -7,6 +7,7 @@
 
 #include <stdint.h>
 
+#include <algorithm>
 #include <vector>
 
 namespace swk {
@@ -337,12 +338,15 @@ cudaError_t sw_launch_strip(cudaStream_t st, const SwStripLaunch &L)
     a.raw = L.db.raw; a.off = L.db.off; a.pair_desc = L.db.pair_desc;
     a.ovf_count = L.ovf_count; a.ovf_list = L.ovf_list; a.ovf_cap = L.ovf_cap;
     a.topk_keys = L.topk_keys; a.topk_k = L.topk_k; a.topk_nq = L.topk_nq;
+    a.hits = L.hits.keys; a.hits_score = L.hits.score; a.hits_count = L.hits.count; a.hits_cap = L.hits.cap;
+    a.min_score = L.hits.min_score; a.hits_shift = L.hits.shift;
     a.dev_err = L.dev_err;
     a.done_count = L.done_count; a.done_flag = L.done_flag; a.done_seq = L.done_seq;
 #ifdef SW_BOUNDS_CHECK
     a.tp_words = L.db.tp_words; a.bnd_elems = L.bnd_elems; a.out_elems = L.out_elems;
 #endif
     if (L.out_mode == SW_OUT_TOPK && (L.topk_k < 1 || L.topk_k > kMaxTopK || !L.topk_keys)) return cudaErrorInvalidValue;
+    if (L.out_mode == SW_OUT_HITS && (L.direct || (L.hits.keys && (!L.hits.score || !L.hits.count)))) return cudaErrorInvalidValue;
     const size_t smem = sw_strip_smem_bytes(L.vidx, L.chunk_passes);
     if (L.jit_kernel && !L.direct && !sc.limit) {
         void *params[] = {&a};
@@ -538,6 +542,55 @@ cudaError_t sw_launch_topk_row(cudaStream_t st, const int32_t *row, uint32_t n, 
 {
     if (k <= 0) return cudaSuccess;
     topk_row_kernel<<<1, 256, 0, st>>>(row, n, k, keys + (size_t)q * k);
+    return cudaGetLastError();
+}
+
+namespace {
+// hit-list entries of one materialised score row (the band-pipelined kernel's) / of the overflow list; grid-stride,
+// so a warp's lanes look at consecutive entries and the warp appends with one atomicAdd (hits_slots)
+__global__ void __launch_bounds__(256) hits_row_kernel(const int32_t *row, uint32_t n, int q, const SwHitList hl)
+{
+    const unsigned long long key_row = (unsigned long long)(unsigned)q << hl.shift;
+    const uint32_t stride = gridDim.x * blockDim.x;
+    for (uint32_t i0 = blockIdx.x * blockDim.x; i0 < n; i0 += stride) {       // warp-uniform trip count
+        const uint32_t i = i0 + threadIdx.x;
+        const int32_t v = i < n ? row[i] : -1;
+        const bool take = v >= 0 && v >= hl.min_score;                         // < 0: not scored here / sentinel
+        unsigned long long p = 0, unused = 0;
+        if (hits_slots(hl.count, take, false, p, unused) && take && p < hl.cap) { hl.keys[p] = key_row | i; hl.score[p] = v; }
+    }
+}
+
+__global__ void __launch_bounds__(256) hits_ovf_kernel(const unsigned *ovf_count, const uint2 *ovf_list, const int32_t *ovf_score,
+                                                       unsigned ovf_cap, const SwHitList hl)
+{
+    const unsigned c = *ovf_count, n = c < ovf_cap ? c : ovf_cap;
+    const unsigned stride = gridDim.x * blockDim.x;
+    for (unsigned i0 = blockIdx.x * blockDim.x; i0 < n; i0 += stride) {
+        const unsigned i = i0 + threadIdx.x;
+        const bool take = i < n && ovf_score[i] >= hl.min_score;
+        unsigned long long p = 0, unused = 0;
+        if (hits_slots(hl.count, take, false, p, unused) && take && p < hl.cap) {
+            hl.keys[p] = ((unsigned long long)ovf_list[i].x << hl.shift) | ovf_list[i].y;
+            hl.score[p] = ovf_score[i];
+        }
+    }
+}
+}  // namespace
+
+cudaError_t sw_launch_hits_row(cudaStream_t st, const int32_t *row, uint32_t n, int q, const SwHitList &hl)
+{
+    if (n == 0 || !hl.keys) return cudaSuccess;
+    const uint32_t grid = std::min<uint32_t>((n + 255) / 256, 1024);
+    hits_row_kernel<<<grid, 256, 0, st>>>(row, n, q, hl);
+    return cudaGetLastError();
+}
+
+cudaError_t sw_launch_hits_ovf(cudaStream_t st, const unsigned *ovf_count, const uint2 *ovf_list, const int32_t *ovf_score,
+                               unsigned ovf_cap, const SwHitList &hl)
+{
+    if (!hl.keys) return cudaSuccess;
+    hits_ovf_kernel<<<std::max<unsigned>(1, std::min<unsigned>((ovf_cap + 255) / 256, 256)), 256, 0, st>>>(ovf_count, ovf_list, ovf_score, ovf_cap, hl);
     return cudaGetLastError();
 }
 

@@ -13,6 +13,7 @@
 #define SW_OUT_I32  0
 #define SW_OUT_I16  1
 #define SW_OUT_TOPK 2
+#define SW_OUT_HITS 3
 #define SW_MAX_TOPK 32
 
 /* Database shard resident in HBM.  Layout (DESIGN.md "data layout"):
@@ -76,6 +77,16 @@ size_t sw_strip_smem_bytes(int idx, int chunk_passes);
 /* Resident blocks per SM of variant idx with smem_bytes of dynamic shared memory. */
 cudaError_t sw_strip_occupancy(int idx, size_t smem_bytes, int *blocks_per_sm);
 
+/* Hit list (SW_OUT_HITS): keys[i] = row << shift | shard-local subject, score[i] = its score, for every pair
+ * scoring >= min_score; *count counts past cap, stores stop there.  keys == null: append nothing. */
+struct SwHitList {
+    unsigned long long *keys = nullptr;
+    int32_t *score = nullptr;
+    unsigned long long *count = nullptr;   /* 64-bit: it counts past cap, and a shard can have >= 2^32 pairs */
+    unsigned cap = 0;
+    int min_score = 1, shift = 0;
+};
+
 /* One strip-kernel launch: queries qidx[0..nql) (or q0 .. q0+nql-1 when qidx is null) against all
  * pairs of db.  bnd: scratch for pass boundaries, grid * bnd_cols * (block_threads/G) uint2.
  * counter: zeroed device word (work queue) or null for a static schedule.  chunk_passes: passes (of
@@ -110,6 +121,7 @@ struct SwStripLaunch {
     unsigned ovf_cap = 0;
     unsigned long long *topk_keys = nullptr;
     int topk_k = 0, topk_nq = 0;
+    SwHitList hits{};             /* SW_OUT_HITS; out_elems is then the list's allocated length (bounds-check build) */
     unsigned *dev_err = nullptr;
     unsigned *done_count = nullptr, *done_flag = nullptr;   /* latency path: completion flag in mapped host memory */
     unsigned done_seq = 0;
@@ -227,5 +239,13 @@ cudaError_t sw_launch_topk_row(cudaStream_t st, const int32_t *row, uint32_t n, 
 cudaError_t sw_launch_topk_merge(cudaStream_t st, const unsigned long long *keys, int nlists, int nq, int k,
                                  const unsigned *ovf_count, const uint2 *ovf_list, const int32_t *ovf_score,
                                  unsigned ovf_cap, unsigned long long *out_keys);
+
+/* Hit-list entries that do not come from the strip epilogue, appended with one atomicAdd per warp like
+ * there: hits_row = the entries >= min_score of one materialised score row of query row q
+ * (entries < 0 are skipped: not scored here, or the overflow sentinel) -- the band-pipelined kernel's rows;
+ * hits_ovf = the overflow-list entries whose exact 32-bit score (ovf_score) is >= min_score. */
+cudaError_t sw_launch_hits_row(cudaStream_t st, const int32_t *row, uint32_t n, int q, const SwHitList &hl);
+cudaError_t sw_launch_hits_ovf(cudaStream_t st, const unsigned *ovf_count, const uint2 *ovf_list, const int32_t *ovf_score,
+                               unsigned ovf_cap, const SwHitList &hl);
 
 #endif

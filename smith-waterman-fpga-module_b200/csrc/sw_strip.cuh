@@ -53,6 +53,7 @@
 #define SW_OUT_I32  0               /* int32 out[q][subject]                                     */
 #define SW_OUT_I16  1               /* int16 out[q][subject]                                     */
 #define SW_OUT_TOPK 2               /* no matrix: per-block private top-k lists, merged later    */
+#define SW_OUT_HITS 3               /* no matrix: (row << hits_shift | subject, score) of every score >= min_score */
 
 /* device-side error word (bit set = which check failed); only written by SW_BOUNDS_CHECK builds
  * and by the wave kernel's spin-wait guard */
@@ -209,6 +210,13 @@ struct StripArgs {
     unsigned *done_count;
     unsigned *done_flag;
     unsigned done_seq;
+    // hit list (SW_OUT_HITS): hits[i] = row << hits_shift | subject, hits_score[i] = score, for every pair with
+    // score >= min_score that is not on the overflow list; hits_count counts past hits_cap, stores stop there
+    unsigned long long *hits;  // null = append nothing (autotune's sample launches)
+    int32_t *hits_score;
+    unsigned long long *hits_count;   // 64-bit: a shard of 10 M subjects x 1 000 rows has 10^10 pairs
+    unsigned hits_cap;
+    int min_score, hits_shift;
 #ifdef SW_BOUNDS_CHECK
     unsigned long long tp_words, bnd_elems, out_elems;
 #endif
@@ -221,6 +229,22 @@ struct StripArgs {
 #define SW_CHECK(cond, bit, args) do { } while (0)
 #define SW_CHECKED(cond, bit, args) (true)
 #endif
+
+// Hit-list slots of up to two entries per lane (take0, take1): one atomicAdd per warp on *count.  Every
+// lane of the warp calls it.  Returns false when the warp has nothing to append.
+__device__ __forceinline__ bool hits_slots(unsigned long long *count, bool take0, bool take1, unsigned long long &p0,
+                                           unsigned long long &p1)
+{
+    const unsigned b0 = __ballot_sync(0xFFFFFFFFu, take0), b1 = __ballot_sync(0xFFFFFFFFu, take1);
+    if ((b0 | b1) == 0u) return false;
+    const unsigned lane = threadIdx.x & 31u, below = (1u << lane) - 1u, n0 = __popc(b0);
+    unsigned long long base = 0;
+    if (lane == 0) base = atomicAdd(count, (unsigned long long)(n0 + __popc(b1)));
+    base = __shfl_sync(0xFFFFFFFFu, base, 0);
+    p0 = base + __popc(b0 & below);
+    p1 = base + n0 + __popc(b1 & below);
+    return true;
+}
 
 // Column codes: 0..15 = t_lo | t_hi << 2 (both members have a base in this column);
 // 16..19 = 16 + t_lo (the shorter member, always the high lane, has ended: its lane sees PAD);
@@ -855,6 +879,22 @@ __global__ void __launch_bounds__(BT, MINB) sw_strip_kernel(const StripArgs a)
                 SW_CHECK((unsigned long long)eq * a.out_stride + subj_lo < a.out_elems, SW_DEVERR_OUT, a);
                 orow[subj_lo] = (int16_t)(ov0 ? SW_OVERFLOW_SENTINEL : sc0);
                 if (has1) orow[subj_hi] = (int16_t)(ov1 ? SW_OVERFLOW_SENTINEL : sc1);
+            }
+        } else if (a.out_mode == SW_OUT_HITS) {
+            // every thread of the block is here (the item loop is block-uniform); flagged pairs reach the
+            // list from their exact score (hits_ovf_kernel), never from here
+            unsigned long long p0 = 0, p1 = 0;
+            const bool t0 = owner && !ov0 && sc0 >= a.min_score, t1 = has1 && !ov1 && sc1 >= a.min_score;
+            if (a.hits && hits_slots(a.hits_count, t0, t1, p0, p1)) {
+                const unsigned long long row = (unsigned long long)(unsigned)eq << a.hits_shift;
+                if (t0 && p0 < a.hits_cap) {
+                    SW_CHECK(p0 < a.out_elems, SW_DEVERR_OUT, a);
+                    a.hits[p0] = row | subj_lo; a.hits_score[p0] = sc0;
+                }
+                if (t1 && p1 < a.hits_cap) {
+                    SW_CHECK(p1 < a.out_elems, SW_DEVERR_OUT, a);
+                    a.hits[p1] = row | subj_hi; a.hits_score[p1] = sc1;
+                }
             }
         } else {
             // fused top-k: candidates = keys above the block's current K-th key for this query
