@@ -133,9 +133,7 @@ struct Slot {
     std::vector<uint32_t> pair_tmp;    // latency path: pairing scratch before the descriptors are written
     bool scored = false;
     bool ovf_used = false;
-    int out_mode = SW_OUT_I32;         // of the last scoring
-    int topk_k = 0;
-    int hits_shift = 0;                // hit keys: row << hits_shift | shard-local subject
+    int hits_shift = 0;               // hit keys: row << hits_shift | shard-local subject
     // small (latency) path: one staging buffer in, mapped scores out
     bool is_small = false;
     PinnedBuf h_small_in, h_small_out, h_small_flag;
@@ -180,8 +178,10 @@ struct Batch {
     size_t ns = 0;
     int nq = 0;                       // query rows the scores of this batch have
     bool loaded = false, scored = false, small = false;
+    // output of the scoring, fixed at submit: SW_OUT_I32 / I16 / TOPK (topk_k lists) / HITS (scores >= hits_min,
+    // at most hits_max per GPU)
     int out_mode = SW_OUT_I32, topk_k = 0;
-    int32_t hits_min = 0;             // > 0: scored in hits mode with this threshold
+    int32_t hits_min = 0;
     size_t hits_max = 0;
     bool hits_staged = false;         // the stitched list below waits for a fetch with enough room
     std::vector<uint32_t> hits_row;
@@ -244,7 +244,7 @@ struct sw_handle {
     double last_ms = 0.0;
     sw_stats_t stats{};               // host-visible phase times of the last submit / fetch
     char last_kernel[96] = "none";
-    int force_R = 0, force_G = 0, force32 = 0, force_arith = -1;
+    int force_R = 0, force_G = 0, force32 = 0;
     int force_variant = -1;
     bool autotune = true;             // time the model's top candidates on a sample of large jobs
 };
@@ -258,6 +258,8 @@ const int kMaxCounters = 4096;
         cudaError_t e__ = (call);                                               \
         if (e__ != cudaSuccess) { (h)->last_cuda.store((int)e__); return (e__ == cudaErrorMemoryAllocation) ? SW_ENOMEM : SW_ECUDA; } \
     } while (0)
+// propagates the status of a failed SW_* call
+#define SW_TRY(call) do { const int rc__ = (call); if (rc__ != SW_OK) return rc__; } while (0)
 
 int validate_params(const sw_params_t *p)
 {
@@ -408,6 +410,16 @@ void build_segments(Slot &g, const uint32_t *pair_len, size_t np)
     }
 }
 
+SwDevDb dev_db(const Slot &g)
+{
+    SwDevDb db{};
+    db.raw = g.d_raw.as<uint8_t>(); db.off = g.d_off.as<uint64_t>(); db.len = g.d_len.as<uint32_t>();
+    db.ns = (uint32_t)(g.s1 - g.s0); db.pair_subj = g.d_pair_subj.as<uint32_t>();
+    db.pair_len = g.d_pair_len.as<uint32_t>(); db.tile_woff = g.d_tile_woff.as<uint64_t>();
+    db.tp = g.d_tp.as<uint32_t>(); db.tp_words = g.tp_words; db.npairs = g.npairs; db.max_len = g.max_len;
+    return db;
+}
+
 // Length-sorts the shard's subjects, pairs neighbours in length order, lays out 32-pair tiles, uploads.
 int load_shard(sw_handle *h, GpuCtx &gc, Slot &g, const uint8_t *packed, const uint32_t *len, const uint64_t *off)
 {
@@ -488,25 +500,9 @@ int load_shard(sw_handle *h, GpuCtx &gc, Slot &g, const uint8_t *packed, const u
     SW_CUDA(h, cudaMemcpyAsync(g.d_tile_woff.p, tile_woff, (ntiles + 1) * sizeof(uint64_t), cudaMemcpyHostToDevice, cs));
     SW_CUDA(h, cudaEventRecord(g.ev_upload, cs));
     SW_CUDA(h, cudaStreamWaitEvent(gc.st_compute, g.ev_upload, 0));
-
-    SwDevDb db{};
-    db.raw = g.d_raw.as<uint8_t>(); db.off = g.d_off.as<uint64_t>(); db.len = g.d_len.as<uint32_t>();
-    db.ns = (uint32_t)n; db.pair_subj = g.d_pair_subj.as<uint32_t>(); db.pair_len = g.d_pair_len.as<uint32_t>();
-    db.tile_woff = g.d_tile_woff.as<uint64_t>(); db.tp = g.d_tp.as<uint32_t>(); db.tp_words = g.tp_words;
-    db.npairs = g.npairs; db.max_len = g.max_len;
-    SW_CUDA(h, sw_launch_build_tp(gc.st_compute, db));
+    SW_CUDA(h, sw_launch_build_tp(gc.st_compute, dev_db(g)));
     h->launches++;
     return SW_OK;
-}
-
-SwDevDb dev_db(const Slot &g)
-{
-    SwDevDb db{};
-    db.raw = g.d_raw.as<uint8_t>(); db.off = g.d_off.as<uint64_t>(); db.len = g.d_len.as<uint32_t>();
-    db.ns = (uint32_t)(g.s1 - g.s0); db.pair_subj = g.d_pair_subj.as<uint32_t>();
-    db.pair_len = g.d_pair_len.as<uint32_t>(); db.tile_woff = g.d_tile_woff.as<uint64_t>();
-    db.tp = g.d_tp.as<uint32_t>(); db.tp_words = g.tp_words; db.npairs = g.npairs; db.max_len = g.max_len;
-    return db;
 }
 
 SwDevQueries dev_queries(const sw_handle *h, const GpuCtx &gc)
@@ -516,6 +512,19 @@ SwDevQueries dev_queries(const sw_handle *h, const GpuCtx &gc)
     dq.nq = (int)h->q_len.size(); dq.max_len = h->q_max_len;
     return dq;
 }
+
+// Pair blocks (block_threads / G pairs each) of a strip launch over npairs pairs.
+uint32_t pair_blocks(const SwStripVariant *v, uint64_t npairs)
+{
+    const uint64_t ppb = (uint64_t)(v->block_threads / v->G);
+    return (uint32_t)((npairs + ppb - 1) / ppb);
+}
+
+// Passes of variant vidx in one profile chunk when the chunk may use 48 KB of shared memory.
+int budget_passes(int vidx) { return std::max<int>(1, (int)((48 * 1024) / sw_strip_smem_bytes(vidx, 1))); }
+
+// Passes per profile chunk of a query that needs need_passes passes.
+int chunk_passes_for(int vidx, int need_passes) { return std::max(1, std::min(need_passes, budget_passes(vidx))); }
 
 // Measured steady-state speed of each variant in GCUPS over PADDED cells (150-nt reads,
 // profiles/r01_variant_sweep.txt); only the ratios matter for the choice below.
@@ -567,9 +576,9 @@ double variant_speed_at(const GpuCtx &gc, const SwStripVariant *v, uint32_t max_
 // pairs can keep busy, plus half the time of the longest work item running at its share of an SM:
 // with few, long items the tail of the launch is what matters.
 // split: the launch may use the pass split (plan_pass_split), which cuts the item -- and the tail -- into parts.
-double variant_cost(const GpuCtx &gc, const Slot &g, const SwStripVariant *v, const uint32_t *qlens, size_t nql, uint32_t maxq,
-                    bool split = false)
+double variant_cost(const GpuCtx &gc, const Slot &g, int vidx, const uint32_t *qlens, size_t nql, uint32_t maxq, bool split = false)
 {
+    const SwStripVariant *v = sw_strip_variant(vidx);
     const int P = v->R * v->G;
     double rows = 0;                      // padded rows over all queries
     for (size_t i = 0; i < nql; ++i) rows += (double)((qlens[i] + P - 1) / P) * P;
@@ -586,10 +595,9 @@ double variant_cost(const GpuCtx &gc, const Slot &g, const SwStripVariant *v, co
     double item = qrows * cols * 2.0 * ppb * ((double)gc.num_sms * v->min_blocks) / speed;
     if (split) {
         // the same arithmetic as plan_pass_split: parts of whole profile chunks, about 20 rounds of items
-        const size_t pass_bytes = (size_t)v->G * v->S * ((v->R / v->S + 1) / 2) * 32 * sizeof(uint2);
-        const double chunk_rows = (double)std::max<size_t>(1, (48 * 1024) / pass_bytes) * P;
+        const double chunk_rows = (double)budget_passes(vidx) * P;
         const double chunks = std::ceil(qrows / chunk_rows);
-        const double rounds = std::ceil((double)g.npairs / ppb) * (double)std::max<size_t>(nql, 1) / ((double)gc.num_sms * v->min_blocks);
+        const double rounds = (double)pair_blocks(v, g.npairs) * (double)std::max<size_t>(nql, 1) / ((double)gc.num_sms * v->min_blocks);
         if (chunks >= 2.0 && rounds >= 1.0 && rounds < 16.0) item /= std::min(chunks, std::ceil(20.0 / rounds));
     }
     return job + 0.5 * item;
@@ -622,7 +630,7 @@ int choose_variant(const sw_handle *h, const GpuCtx &gc, const Slot &g, const ui
     double best_cost = 0;
     std::vector<std::pair<double, int>> costs;
     for (int i = 0; i < nv; ++i) {
-        const double cost = variant_cost(gc, g, sw_strip_variant(i), qlens, nql, maxq, split);
+        const double cost = variant_cost(gc, g, i, qlens, nql, maxq, split);
         if (best < 0 || cost < best_cost) { best = i; best_cost = cost; }
         costs.emplace_back(cost, i);
     }
@@ -643,6 +651,16 @@ int cached_occupancy(sw_handle *h, GpuCtx &gc, int vidx, int chunk_passes, int *
     return SW_OK;
 }
 
+// Grows a scratch buffer that the GPU's launch streams share, after draining them: kernels queued on
+// the compute stream or a side stream may still read the old allocation.
+cudaError_t grow_shared(GpuCtx &gc, DevBuf &buf, size_t bytes)
+{
+    if (bytes <= buf.cap && buf.p) return cudaSuccess;
+    cudaError_t e = cudaStreamSynchronize(gc.st_compute);
+    for (cudaStream_t st : gc.st_aux) if (st && e == cudaSuccess) e = cudaStreamSynchronize(st);
+    return e == cudaSuccess ? buf.reserve(bytes) : e;
+}
+
 // Launch geometry of a strip variant for `npairs` pairs with subjects up to max_len and queries up to
 // maxq rows; also grows the pass-boundary scratch.
 int strip_setup(sw_handle *h, GpuCtx &gc, DevBuf &bnd_buf, uint32_t npairs, uint32_t max_len, uint32_t maxq, int nql, int vidx,
@@ -651,17 +669,14 @@ int strip_setup(sw_handle *h, GpuCtx &gc, DevBuf &bnd_buf, uint32_t npairs, uint
     const SwStripVariant *v = sw_strip_variant(vidx);
     const int P = v->R * v->G;
     const int need_passes = (int)((maxq + P - 1) / P);
-    const size_t pass_bytes = sw_strip_smem_bytes(vidx, 1);
-    const int budget_passes = std::max<int>(1, (int)((48 * 1024) / pass_bytes));
-    *chunk_passes = std::max(1, std::min(need_passes, budget_passes));
+    *chunk_passes = chunk_passes_for(vidx, need_passes);
     int bps = 0;
-    int rc = cached_occupancy(h, gc, vidx, *chunk_passes, &bps);
-    if (rc != SW_OK) return rc;
+    SW_TRY(cached_occupancy(h, gc, vidx, *chunk_passes, &bps));
     if (bps < 1) return SW_ECUDA;
     const int ppb = v->block_threads / v->G;
-    const uint32_t npb = (npairs + ppb - 1) / ppb;
     // persistent blocks: as many as there are work items (pair blocks x queries), at most a full GPU
-    *grid = (int)std::min<uint64_t>(std::max<uint64_t>((uint64_t)npb * (uint64_t)std::max(nql, 1), 1), (uint64_t)gc.num_sms * bps);
+    *grid = (int)std::min<uint64_t>(std::max<uint64_t>((uint64_t)pair_blocks(v, npairs) * (uint64_t)std::max(nql, 1), 1),
+                                    (uint64_t)gc.num_sms * bps);
     *bnd_elems = 0;
     if (need_passes > 1) {
         // pass-boundary scratch: one (H, G) per column of the longest subject, per pair slot, per
@@ -672,11 +687,7 @@ int strip_setup(sw_handle *h, GpuCtx &gc, DevBuf &bnd_buf, uint32_t npairs, uint
         if (per_block > budget) return SW_ENOMEM;
         *grid = (int)std::min<size_t>((size_t)*grid, std::max<size_t>(1, budget / per_block));
         // (a buffer shared by the launches of one stream only ever grows: earlier launches keep fitting)
-        if (bnd_buf.cap < (size_t)*grid * per_block) {
-            SW_CUDA(h, cudaStreamSynchronize(gc.st_compute));
-            for (cudaStream_t st : gc.st_aux) if (st) SW_CUDA(h, cudaStreamSynchronize(st));
-            SW_CUDA(h, bnd_buf.reserve((size_t)*grid * per_block));
-        }
+        SW_CUDA(h, grow_shared(gc, bnd_buf, (size_t)*grid * per_block));
         *bnd_elems = (size_t)*grid * per_block / sizeof(uint2);
     }
     return SW_OK;
@@ -723,21 +734,16 @@ int plan_pass_split(sw_handle *h, GpuCtx &gc, SwStripLaunch &L, uint32_t npairs,
     const int chunks = (npass + L.chunk_passes - 1) / L.chunk_passes;       // a part is whole profile chunks
     if (chunks < 2) return SW_OK;
     const int ppb = v->block_threads / v->G;
-    const uint64_t npb = (npairs + ppb - 1) / ppb;
-    const uint64_t chains = npb * (uint64_t)std::max(nql_max, 1);
+    const uint64_t chains = (uint64_t)pair_blocks(v, npairs) * (uint64_t)std::max(nql_max, 1);
     int nparts = 0, part_passes = 0;
     if (!plan_pass_parts(npass, L.chunk_passes, chains, L.grid, h->pass_split, &nparts, &part_passes)) return SW_OK;
     const size_t bnd_bytes = (size_t)chains * (size_t)max_len * ppb * sizeof(uint2);
     size_t free_b = 0, total_b = 0;
     SW_CUDA(h, cudaMemGetInfo(&free_b, &total_b));
     if (bnd_bytes > ((size_t)16 << 30) || (gc.d_bnd.cap < bnd_bytes && bnd_bytes - gc.d_bnd.cap > free_b / 2)) return SW_OK;
-    if (gc.d_bnd.cap < bnd_bytes || gc.d_part_done.cap < chains * sizeof(unsigned) || gc.d_part_best.cap < chains * v->block_threads * sizeof(uint32_t)) {
-        SW_CUDA(h, cudaStreamSynchronize(gc.st_compute));
-        for (cudaStream_t st : gc.st_aux) if (st) SW_CUDA(h, cudaStreamSynchronize(st));
-        SW_CUDA(h, gc.d_bnd.reserve(bnd_bytes));
-        SW_CUDA(h, gc.d_part_done.reserve(chains * sizeof(unsigned)));
-        SW_CUDA(h, gc.d_part_best.reserve(chains * v->block_threads * sizeof(uint32_t)));
-    }
+    SW_CUDA(h, grow_shared(gc, gc.d_bnd, bnd_bytes));
+    SW_CUDA(h, grow_shared(gc, gc.d_part_done, chains * sizeof(unsigned)));
+    SW_CUDA(h, grow_shared(gc, gc.d_part_best, chains * v->block_threads * sizeof(uint32_t)));
     L.nparts = nparts; L.part_passes = part_passes;
     L.part_done = gc.d_part_done.as<unsigned>(); L.part_best = gc.d_part_best.as<uint32_t>();
     L.bnd_elems = bnd_bytes / sizeof(uint2);
@@ -750,8 +756,7 @@ int plan_pass_split(sw_handle *h, GpuCtx &gc, SwStripLaunch &L, uint32_t npairs,
 // than two full grids, or consecutive items of a thread block stop sharing the query profile.
 uint32_t superblock_for(const SwStripVariant *v, uint32_t npairs, uint64_t tp_words, int grid, double sb_mb)
 {
-    const uint32_t ppb = (uint32_t)(v->block_threads / v->G);
-    const uint32_t npb = (npairs + ppb - 1) / ppb;
+    const uint32_t npb = pair_blocks(v, npairs);
     if (npb == 0 || tp_words == 0) return 0;
     const double bytes_per_block = (double)tp_words * 4.0 / (double)npb;
     uint32_t b = (uint32_t)std::max(1.0, (sb_mb * 1024 * 1024) / std::max(bytes_per_block, 1.0));
@@ -818,8 +823,7 @@ int autotune_variant(sw_handle *h, GpuCtx &gc, Slot &g, SwStripLaunch base, cons
     float best_ms = 0.f;
     for (int c = 0; c < ncand; ++c) {
         base.vidx = ranked[c];
-        int rc = strip_setup(h, gc, gc.d_bnd, base.db.npairs, g.max_len, h->q_max_len, nqs, base.vidx, &base.grid, &base.chunk_passes, &base.bnd_elems);
-        if (rc != SW_OK) return rc;
+        SW_TRY(strip_setup(h, gc, gc.d_bnd, base.db.npairs, g.max_len, h->q_max_len, nqs, base.vidx, &base.grid, &base.chunk_passes, &base.bnd_elems));
         base.bnd = gc.d_bnd.as<uint2>();
         float ms = 0.f;
         for (int rep = 0; rep < 2; ++rep) {  // first run warms caches and the instruction cache
@@ -836,406 +840,509 @@ int autotune_variant(sw_handle *h, GpuCtx &gc, Slot &g, SwStripLaunch base, cons
     return SW_OK;
 }
 
-cudaEvent_t pool_event(sw_handle *h, Slot &g, size_t i, int *rc)
+// Marks queries [q0, q1) finished at this point of the compute stream (the slot's chunk-done events are created once).
+int push_chunk(sw_handle *h, GpuCtx &gc, Slot &g, int q0, int q1)
 {
-    *rc = SW_OK;
+    const size_t i = g.chunks.size();
     while (g.ev_pool.size() <= i) {
         cudaEvent_t e = nullptr;
         cudaError_t ce = cudaEventCreateWithFlags(&e, cudaEventDisableTiming);
-        if (ce != cudaSuccess) { h->last_cuda.store((int)ce); *rc = SW_ECUDA; return nullptr; }
+        if (ce != cudaSuccess) { h->last_cuda.store((int)ce); return SW_ECUDA; }
         g.ev_pool.push_back(e);
     }
-    return g.ev_pool[i];
+    QueryChunk c{q0, q1, g.ev_pool[i]};
+    SW_CUDA(h, cudaEventRecord(c.done, gc.st_compute));
+    g.chunks.push_back(c);
+    return SW_OK;
 }
 
-// One group of queries that run with the same variant (q empty = all queries, contiguous).
-struct QueryGroup { int vidx; std::vector<int> q; uint64_t rows; };
+// What the stages of one GPU's scoring share.
+struct ScoreJob {
+    GpuCtx &gc; Slot &g; const Batch &bt;   // bt: the output settings
+    int nq = 0; size_t n = 0;               // n: subjects of the shard
+    bool topk = false, hits = false, may_overflow = false;
+    SwScoring sc{}; SwDevDb db{}; SwDevQueries dq{}; SwHitList hl{};
+    std::vector<int> wave_q, strip_q;       // queries of the band-pipelined kernel / of the strip kernel
+    SwStripLaunch base;                     // what every strip launch of the scoring has in common
+};
 
-int score_gpu(sw_handle *h, GpuCtx &gc, Slot &g)
+// One strip launch of a plan: queries [q0, q1) (query chunks), launch stream, time of its longest work item.
+struct Planned { SwStripLaunch L; int q0, q1; int stream; double item_s; };
+
+// The strip queries' launch plan.
+struct StripPlan {
+    std::vector<Planned> launches;
+    std::vector<uint32_t> qlen; uint32_t maxq = 0; uint64_t rows = 0;   // the strip queries' lengths, longest, sum
+    bool same_len = false, simple = false, jit_used = false;
+    int max_grid = 0, label_v = -1;   // label_v: the variant last_kernel names
+    size_t n_groups = 0;              // launches of the length-group plan
+};
+
+// Output buffers of a scoring, zeroed on the compute stream: the matrix, the top-k lists or the hit list.
+int reserve_outputs(sw_handle *h, ScoreJob &j)
 {
-    if (&gc == &h->gpus[0]) h->last_parts = 1;
-    SW_CUDA(h, cudaSetDevice(gc.dev));
-    const int nq = (int)h->q_len.size();
-    const size_t n = g.s1 - g.s0;
-    g.chunks.clear();
-    g.scored = true;
-    g.ovf_used = false;
-    g.out_mode = h->topk_k > 0 ? SW_OUT_TOPK : h->hits_min > 0 ? SW_OUT_HITS : h->out_mode;
-    g.topk_k = h->topk_k;
-    if (n == 0 || nq == 0) return SW_OK;
-    const bool topk = g.out_mode == SW_OUT_TOPK;
-    const bool hits = g.out_mode == SW_OUT_HITS;
-    const size_t esz = g.out_mode == SW_OUT_I16 ? sizeof(int16_t) : sizeof(int32_t);
-
-    // hit list: keys row << hits_shift | shard-local subject (the fetch sorts them: row-major order)
-    SwHitList hl;
-    if (hits) {
+    GpuCtx &gc = j.gc; Slot &g = j.g;
+    if (j.hits) {
+        // hit list: keys row << hits_shift | shard-local subject (the fetch sorts them: row-major order)
         int sb = 0;
-        while ((1ull << sb) < (uint64_t)n) ++sb;
+        while ((1ull << sb) < (uint64_t)j.n) ++sb;
         g.hits_shift = sb;
         SW_CUDA(h, g.d_hits_count.reserve(sizeof(unsigned long long)));
-        SW_CUDA(h, g.d_hits_key.reserve(h->hits_max * sizeof(unsigned long long)));
-        SW_CUDA(h, g.d_hits_score.reserve(h->hits_max * sizeof(int32_t)));
+        SW_CUDA(h, g.d_hits_key.reserve(j.bt.hits_max * sizeof(unsigned long long)));
+        SW_CUDA(h, g.d_hits_score.reserve(j.bt.hits_max * sizeof(int32_t)));
         SW_CUDA(h, cudaMemsetAsync(g.d_hits_count.p, 0, sizeof(unsigned long long), gc.st_compute));
-        hl.keys = g.d_hits_key.as<unsigned long long>(); hl.score = g.d_hits_score.as<int32_t>();
-        hl.count = g.d_hits_count.as<unsigned long long>(); hl.cap = (unsigned)h->hits_max;
-        hl.min_score = h->hits_min; hl.shift = sb;
-    } else if (!topk) {
-        SW_CUDA(h, g.d_out.reserve((size_t)nq * n * esz));
-        SW_CUDA(h, cudaMemsetAsync(g.d_out.p, 0, (size_t)nq * n * esz, gc.st_compute));
+        j.hl.keys = g.d_hits_key.as<unsigned long long>(); j.hl.score = g.d_hits_score.as<int32_t>();
+        j.hl.count = g.d_hits_count.as<unsigned long long>(); j.hl.cap = (unsigned)j.bt.hits_max;
+        j.hl.min_score = j.bt.hits_min; j.hl.shift = sb;
+    } else if (!j.topk) {
+        const size_t bytes = (size_t)j.nq * j.n * (j.bt.out_mode == SW_OUT_I16 ? sizeof(int16_t) : sizeof(int32_t));
+        SW_CUDA(h, g.d_out.reserve(bytes));
+        SW_CUDA(h, cudaMemsetAsync(g.d_out.p, 0, bytes, gc.st_compute));
     } else {
-        SW_CUDA(h, g.d_topk_out.reserve((size_t)nq * g.topk_k * sizeof(unsigned long long)));
-        SW_CUDA(h, cudaMemsetAsync(g.d_topk_out.p, 0, (size_t)nq * g.topk_k * sizeof(unsigned long long), gc.st_compute));
+        const size_t bytes = (size_t)j.nq * j.bt.topk_k * sizeof(unsigned long long);
+        SW_CUDA(h, g.d_topk_out.reserve(bytes));
+        SW_CUDA(h, cudaMemsetAsync(g.d_topk_out.p, 0, bytes, gc.st_compute));
     }
-    SW_CUDA(h, cudaEventRecord(g.ev_start, gc.st_compute));
-    int rc = SW_OK;
-    if (g.npairs == 0) {
-        SW_CUDA(h, cudaEventRecord(g.ev_stop, gc.st_compute));
-        g.ev_stop_deferred = false;
-        QueryChunk c{0, nq, pool_event(h, g, 0, &rc)};
-        if (rc != SW_OK) return rc;
-        SW_CUDA(h, cudaEventRecord(c.done, gc.st_compute));
-        g.chunks.push_back(c);
-        return SW_OK;
-    }
+    return SW_OK;
+}
 
-    const SwScoring sc = scoring_of(h);
-    const SwDevDb db = dev_db(g);
-    const SwDevQueries dq = dev_queries(h, gc);
-
-    // Value range: the packed 16-bit kernel is always used; when match * min(m, n) could exceed
-    // the 16-bit range it flags the (rare) pairs whose running maximum got near 32767: they go to
-    // the overflow list and the 32-bit kernel recomputes exactly those.
-    const uint64_t smax = (uint64_t)sc.match * std::min<uint64_t>(h->q_max_len, g.max_len);
-    const bool may_overflow = !sc.limit && (smax + (uint64_t)sc.match >= 32000ull);
-    SW_CUDA(h, gc.d_counters.reserve(kMaxCounters * sizeof(unsigned)));
-
-    // ---- few, long pairs: the bands of a long query become concurrent work items (sw_wave.cuh) ----
-    std::vector<int> wave_q, strip_q;
-    {
-        // (top-k: the band-pipelined kernel fills a scratch row per query, whose top k then join the key lists)
-        const bool wave_ok = h->wave && !sc.limit && !h->force32 && !variant_forced(h);
-        // Besides "few pairs": whenever the long queries' work items (128 pairs x all passes) would
-        // leave the strip kernel's last round mostly empty.  Measured (profiles/r02_wave_vs_strip_mid.txt):
-        // the band-pipelined kernel holds 7.2-7.5 TCUPS from 3 000 to 100 000 pairs, the strip kernel
-        // 8.1 TCUPS at exactly two full rounds but 4.9-6.9 below and between whole rounds.
-        size_t n_long = 0;
-        for (int q = 0; q < nq; ++q) n_long += (h->q_len[q] >= 2 * SW_WAVE_ROWS_PER_BAND && h->q_len[q] <= 4000u * 256u) ? 1 : 0;
-        const double rounds = (double)((g.npairs + 127) / 128) * (double)n_long / ((double)gc.num_sms * 2.0);
-        // (only when every query is long: shorter ones in the same launch fill the strip kernel's rounds)
-        // With the pass split (one launch, equally long queries) the strip kernel no longer pays for a
-        // partly filled last round, so from one full round on it is the faster one
-        // (profiles/r02_pass_split_ab.txt: 8.4-8.8 TCUPS against the band-pipelined 7.2-7.6).
-        // -- when ONE query's items fill kSplitMinRounds rounds (the queries of a call may go out as separate
-        // launches: 3 x 4 kb queries x 60 000 x 2 kb, 0.79 rounds per query, strip + split 6 160 vs 7 794 GCUPS).
-        // scripts/split_ab.py, profiles/r02_pass_split_ab.txt: 10 kb x 100 000 x 1 kb (1.32 rounds) 7 340 -> 8 492,
-        // x 120 000 (1.58) 7 343 -> 8 660, x 151 552 (2.00) 8 327 -> 8 758, x 260 000 (3.43) 8 417 -> 8 756.
-        bool split_possible = h->pass_split != 0 && n_long > 0 && rounds / (double)std::max<size_t>(n_long, 1) >= kSplitMinRounds;
-        for (int q = 1; q < nq; ++q) split_possible = split_possible && h->q_len[q] == h->q_len[0];
-        const bool underfilled = n_long == (size_t)nq &&
-                                 (rounds < 1.05 || (!split_possible && rounds < 4.0 && rounds / std::ceil(rounds) < 0.85));
-        const double bnd_bytes = (double)g.npairs * 2.0 * ((double)g.max_len + 64.0) * 16.0;      // tagged boundary rows of all pairs
-        const bool bnd_fits = bnd_bytes <= 4.0e9, bnd_fits_few = bnd_bytes <= 16.0e9;
-        for (int q = 0; q < nq; ++q) {
-            const uint32_t ql = h->q_len[q];
-            bool w = false;
-            if (wave_ok && ql > SW_WAVE_ROWS_PER_BAND && ql <= 4000u * 256u) {
-                if (h->wave >= 2) w = true;
-                else w = (bnd_fits_few && ((g.npairs <= 1536 && ql >= 2 * SW_WAVE_ROWS_PER_BAND) || g.npairs <= 64)) ||
-                         (ql >= 2 * SW_WAVE_ROWS_PER_BAND && underfilled && bnd_fits);
-            }
-            (w ? wave_q : strip_q).push_back(q);
+// Few, long pairs: the bands of a long query become concurrent work items (sw_wave.cuh).  Splits the
+// queries into those of the band-pipelined kernel and those of the strip kernel.
+void route_queries(const sw_handle *h, const GpuCtx &gc, const Slot &g, std::vector<int> &wave_q, std::vector<int> &strip_q)
+{
+    const int nq = (int)h->q_len.size();
+    // (top-k: the band-pipelined kernel fills a scratch row per query, whose top k then join the key lists)
+    const bool wave_ok = h->wave && !scoring_of(h).limit && !h->force32 && !variant_forced(h);
+    // Besides "few pairs": whenever the long queries' work items (128 pairs x all passes) would
+    // leave the strip kernel's last round mostly empty.  Measured (profiles/r02_wave_vs_strip_mid.txt):
+    // the band-pipelined kernel holds 7.2-7.5 TCUPS from 3 000 to 100 000 pairs, the strip kernel
+    // 8.1 TCUPS at exactly two full rounds but 4.9-6.9 below and between whole rounds.
+    size_t n_long = 0;
+    for (int q = 0; q < nq; ++q) n_long += (h->q_len[q] >= 2 * SW_WAVE_ROWS_PER_BAND && h->q_len[q] <= 4000u * 256u) ? 1 : 0;
+    const double rounds = (double)((g.npairs + 127) / 128) * (double)n_long / ((double)gc.num_sms * 2.0);
+    // (only when every query is long: shorter ones in the same launch fill the strip kernel's rounds)
+    // With the pass split (one launch, equally long queries) the strip kernel no longer pays for a
+    // partly filled last round, so from one full round on it is the faster one
+    // (profiles/r02_pass_split_ab.txt: 8.4-8.8 TCUPS against the band-pipelined 7.2-7.6).
+    // -- when ONE query's items fill kSplitMinRounds rounds (the queries of a call may go out as separate
+    // launches: 3 x 4 kb queries x 60 000 x 2 kb, 0.79 rounds per query, strip + split 6 160 vs 7 794 GCUPS).
+    // scripts/split_ab.py, profiles/r02_pass_split_ab.txt: 10 kb x 100 000 x 1 kb (1.32 rounds) 7 340 -> 8 492,
+    // x 120 000 (1.58) 7 343 -> 8 660, x 151 552 (2.00) 8 327 -> 8 758, x 260 000 (3.43) 8 417 -> 8 756.
+    bool split_possible = h->pass_split != 0 && n_long > 0 && rounds / (double)std::max<size_t>(n_long, 1) >= kSplitMinRounds;
+    for (int q = 1; q < nq; ++q) split_possible = split_possible && h->q_len[q] == h->q_len[0];
+    const bool underfilled = n_long == (size_t)nq &&
+                             (rounds < 1.05 || (!split_possible && rounds < 4.0 && rounds / std::ceil(rounds) < 0.85));
+    const double bnd_bytes = (double)g.npairs * 2.0 * ((double)g.max_len + 64.0) * 16.0;      // tagged boundary rows of all pairs
+    const bool bnd_fits = bnd_bytes <= 4.0e9, bnd_fits_few = bnd_bytes <= 16.0e9;
+    for (int q = 0; q < nq; ++q) {
+        const uint32_t ql = h->q_len[q];
+        bool w = false;
+        if (wave_ok && ql > SW_WAVE_ROWS_PER_BAND && ql <= 4000u * 256u) {
+            if (h->wave >= 2) w = true;
+            else w = (bnd_fits_few && ((g.npairs <= 1536 && ql >= 2 * SW_WAVE_ROWS_PER_BAND) || g.npairs <= 64)) ||
+                     (ql >= 2 * SW_WAVE_ROWS_PER_BAND && underfilled && bnd_fits);
         }
+        (w ? wave_q : strip_q).push_back(q);
     }
+}
 
-    // ---- launch plan ---------------------------------------------------------------------------
-    // Simple case (one length group, every query on one variant -- the bulk case, config 3): query
-    // chunks on the compute stream, D2H of finished rows overlapping the next chunk, the model's top
-    // candidates timed on a sample.  General case: every (length group, query group) gets its own
-    // launch and variant; launches run on several streams so that the tail of one overlaps the
-    // start of the next, longest work items first.
-    struct Planned { SwStripLaunch L; int q0, q1; int stream; double item_s; };
-    std::vector<Planned> plan;
-    std::vector<int> &qidx_host = g.qidx_host;     // stays alive until this slot is scored again
-    qidx_host.clear();
+// Workload signature of an autotune decision (FNV-1a over shape, penalties and the effective output mode).
+uint64_t tune_signature(const sw_handle *h, const Slot &g, int nq, int out_mode)
+{
+    uint64_t key = 1469598103934665603ull;
+    auto log2b = [](uint64_t x) { uint64_t b = 0; while (x >>= 1) ++b; return b; };
+    const uint64_t parts[] = {h->q_max_len, h->q_sum_len, (uint64_t)nq, g.max_len, log2b(g.npairs), log2b(g.sum_len),
+                              (uint64_t)(uint16_t)h->params.match, (uint64_t)(uint16_t)h->params.mismatch,
+                              (uint64_t)(uint16_t)h->params.gap_open, (uint64_t)(uint16_t)h->params.gap_extend,
+                              (uint64_t)h->params.score_width, (uint64_t)out_mode};
+    for (uint64_t x : parts) { key ^= x; key *= 1099511628211ull; }
+    return key;
+}
+
+// Simple case (one length group, every query on one variant -- the bulk case, config 3): query chunks on
+// the compute stream, D2H of finished rows overlapping the next chunk, the model's top candidates timed
+// on a sample.
+int plan_one_launch(sw_handle *h, ScoreJob &j, StripPlan &p)
+{
+    GpuCtx &gc = j.gc; Slot &g = j.g;
+    const int nq = j.nq;
     std::vector<int> ranked;
-    int max_grid = 0;
-    bool simple = false, jit_used = false, sticky_ok = false;
-    int label_v = -1;
-    size_t n_groups_total = 0;
-
-    SwStripLaunch base;
-    base.db = db; base.q = dq; base.sc = sc;
-    base.out = (topk || hits) ? nullptr : g.d_out.p; base.out_stride = n; base.out_elems = hits ? h->hits_max : (size_t)nq * n;
-    base.out_mode = g.out_mode;
-    base.hits = hl;
-    base.dev_err = gc.d_err.as<unsigned>();
-    if (may_overflow) {
-        SW_CUDA(h, g.d_ovf_count.reserve(sizeof(unsigned)));
-        SW_CUDA(h, g.d_ovf_list.reserve((size_t)kOvfCap * sizeof(uint2)));
-        SW_CUDA(h, g.d_ovf_score.reserve((size_t)kOvfCap * sizeof(int32_t)));
-        SW_CUDA(h, cudaMemsetAsync(g.d_ovf_count.p, 0, sizeof(unsigned), gc.st_compute));
-        base.ovf_count = g.d_ovf_count.as<unsigned>(); base.ovf_list = g.d_ovf_list.as<uint2>(); base.ovf_cap = kOvfCap;
-        g.ovf_used = true;
-    }
-
-    if (!h->force32 && !strip_q.empty()) {
-        std::vector<uint32_t> sl;
-        uint32_t smaxq = 0;
-        uint64_t srows = 0;
-        for (int q : strip_q) { sl.push_back(h->q_len[q]); smaxq = std::max(smaxq, h->q_len[q]); srows += h->q_len[q]; }
-        const bool all_strip = (int)strip_q.size() == nq;
-        const bool same_len = std::all_of(sl.begin(), sl.end(), [&](uint32_t x) { return x == sl[0]; });
-        std::vector<Seg> segs = g.segs;
-        bool use_segs = h->plan_segs == 1;
-        if (h->plan_segs == 2 && segs.size() > 1) {
-            // one launch over everything sizes every block's pass-boundary scratch by the longest subject
-            const size_t worst = (size_t)gc.num_sms * 4 * 128 * (size_t)g.max_len * sizeof(uint2);
-            use_segs = smaxq > 64 && worst > ((size_t)4 << 30);
+    // (the split-aware tail term of variant_cost stays off: with it the model prefers the 3-blocks-per-SM
+    // R25x2 instances for 10 kb queries, whose table speed was measured on single-chunk 150-nt reads --
+    // scripts/split_ab.py: 8 059 vs 8 752 GCUPS with R38x2 at two rounds, 8 362 vs 8 780 on 200 k x 1 kb)
+    int vidx = choose_variant(h, gc, g, p.qlen.data(), p.qlen.size(), p.maxq, &ranked, false);
+    if (vidx < 0) return SW_EINVAL;
+    const double est_ms_all = (double)g.sum_len * (double)p.rows / 6.0e9;
+    const bool one_chunk = j.topk || j.hits || j.may_overflow || !j.wave_q.empty();
+    if (h->pass_split != 0 && !variant_forced(h) && sw_strip_variant(vidx)->G > 1) {
+        // The model asks for more lanes per pair because whole items of a one-lane variant would leave
+        // the last round partly empty.  With the pass split that round costs a fraction of a part, so a
+        // one-lane variant is the faster one as soon as its chains fill the GPU once
+        // (scripts/split_ab.py: 10 kb x 120 000 x 1 kb: R38x1_G4 7 014, band-pipelined 7 340, R32x2_G1 8 390 GCUPS).
+        const int nchunks_est = one_chunk ? 1 : std::max(1, std::min(std::min(nq, 8), (int)(est_ms_all / 50.0)));
+        const uint64_t nql_launch = (uint64_t)std::max(1, nq / nchunks_est);
+        for (int cand : ranked) {
+            const SwStripVariant *cv = sw_strip_variant(cand);
+            if (cv->G != 1) continue;
+            const int npass = (int)((p.maxq + cv->R - 1) / cv->R);
+            const int cp = chunk_passes_for(cand, npass);
+            const uint64_t chains = (uint64_t)pair_blocks(cv, g.npairs) * nql_launch;
+            if ((npass + cp - 1) / cp >= 2 && (double)chains >= 1.05 * (double)gc.num_sms * cv->min_blocks) { vidx = cand; break; }
         }
-        if (segs.empty() || variant_forced(h) || !use_segs) segs.assign(1, Seg{0, g.npairs, g.max_len, g.sum_len});
-        simple = all_strip && segs.size() == 1 && (variant_forced(h) || same_len || strip_q.size() == 1);
-        sticky_ok = same_len;
+    }
+    // large jobs: let the GPU pick among the model's top candidates (decision cached per workload shape)
+    j.base.bnd_cols = g.max_len;
+    if (!j.topk && h->autotune && !variant_forced(h) && est_ms_all >= 400.0 && ranked.size() > 1) {
+        const uint64_t key = tune_signature(h, g, nq, j.bt.out_mode);
+        if (gc.tune_key != key || gc.tune_choice < 0) {
+            int choice = vidx;
+            // the sample launches append nothing: a pair they score is scored again by the real launch
+            SwStripLaunch sample = j.base;
+            if (j.hits) { sample.hits.keys = nullptr; sample.ovf_list = nullptr; sample.ovf_count = nullptr; }
+            SW_TRY(autotune_variant(h, gc, g, sample, ranked, nq, p.same_len, &choice));
+            gc.tune_choice = choice;
+            gc.tune_key = key;
+        }
+        vidx = gc.tune_choice;
+    }
+    // query chunks: a handful of launches so that D2H of finished rows overlaps compute
+    // (each launch has its own tail: aim for >= ~50 ms of work per launch, at ~6 TCUPS)
+    int nchunks = one_chunk ? 1 : std::max(1, std::min(std::min(nq, 8), (int)(est_ms_all / 50.0)));
+    // the device work counter is 32-bit: (pair blocks) x (queries per launch) must stay below 2^31
+    while (nchunks < nq && (uint64_t)(g.npairs / 4 + 1) * (uint64_t)((nq + nchunks - 1) / nchunks) >= (1ull << 31)) nchunks *= 2;
+    nchunks = std::min(nchunks, nq);
+    SwStripLaunch L = j.base;
+    L.vidx = vidx;
+    SW_TRY(strip_setup(h, gc, gc.d_bnd, g.npairs, g.max_len, p.maxq, nq / nchunks, vidx, &L.grid, &L.chunk_passes, &L.bnd_elems));
+    L.superblock = superblock_for(sw_strip_variant(vidx), g.npairs, g.tp_words, L.grid, h->superblock_mb);
+    SW_TRY(plan_pass_split(h, gc, L, g.npairs, g.max_len, p.maxq, (nq + nchunks - 1) / nchunks));
+    if (&gc == &h->gpus[0]) h->last_parts = std::max(1, L.nparts);
+    p.max_grid = L.grid;
+    p.label_v = vidx;
+    p.n_groups = 1;
+    if (h->jit && !j.sc.limit && (est_ms_all >= 2000.0 || h->jit >= 2) && std::strcmp(sw_strip_instance_kind(L), "runtime") == 0) {
+        L.jit_kernel = sw_jit_strip_kernel(sw_strip_variant(vidx), j.sc.goe, j.sc.ge, nullptr, 0);
+        p.jit_used = L.jit_kernel != nullptr;
+    }
+    // (A "tail split" -- the pairs of the last, partly filled round of equal work items on a
+    // side stream with a 2- or 4-lane variant -- was built and measured on 200 k x 1 kb x 10 kb:
+    // 262.9 ms against 261.0 ms without it.  The finer items gain what the slower variant loses.)
+    for (int c = 0; c < nchunks; ++c) {
+        const int a0 = (int)((long long)nq * c / nchunks), a1 = (int)((long long)nq * (c + 1) / nchunks);
+        if (a1 <= a0) continue;
+        Planned pl{L, a0, a1, 0, 0.0};
+        pl.L.q0 = a0; pl.L.nql = a1 - a0; pl.L.qidx = nullptr;
+        p.launches.push_back(pl);
+    }
+    return SW_OK;
+}
 
-        if (simple) {
-            // (the split-aware tail term of variant_cost stays off: with it the model prefers the 3-blocks-per-SM
-            // R25x2 instances for 10 kb queries, whose table speed was measured on single-chunk 150-nt reads --
-            // scripts/split_ab.py: 8 059 vs 8 752 GCUPS with R38x2 at two rounds, 8 362 vs 8 780 on 200 k x 1 kb)
-            int vidx = choose_variant(h, gc, g, sl.data(), sl.size(), smaxq, &ranked, false);
-            if (vidx < 0) return SW_EINVAL;
-            const double est_ms_all = (double)g.sum_len * (double)srows / 6.0e9;
-            if (h->pass_split != 0 && !variant_forced(h) && sw_strip_variant(vidx)->G > 1) {
-                // The model asks for more lanes per pair because whole items of a one-lane variant would leave
-                // the last round partly empty.  With the pass split that round costs a fraction of a part, so a
-                // one-lane variant is the faster one as soon as its chains fill the GPU once
-                // (scripts/split_ab.py: 10 kb x 120 000 x 1 kb: R38x1_G4 7 014, band-pipelined 7 340, R32x2_G1 8 390 GCUPS).
-                const int nchunks_est = (topk || hits || may_overflow || !wave_q.empty()) ? 1 : std::max(1, std::min(std::min(nq, 8), (int)(est_ms_all / 50.0)));
-                const uint64_t nql_launch = (uint64_t)std::max(1, nq / nchunks_est);
-                for (int cand : ranked) {
-                    const SwStripVariant *cv = sw_strip_variant(cand);
-                    if (cv->G != 1) continue;
-                    const int P = cv->R;
-                    const int npass = (int)((smaxq + P - 1) / P);
-                    const int cp = std::max(1, std::min<int>(npass, (int)((48 * 1024) / sw_strip_smem_bytes(cand, 1))));
-                    const uint64_t chains = (uint64_t)((g.npairs + cv->block_threads - 1) / cv->block_threads) * nql_launch;
-                    if ((npass + cp - 1) / cp >= 2 && (double)chains >= 1.05 * (double)gc.num_sms * cv->min_blocks) { vidx = cand; break; }
-                }
-            }
-            // large jobs: let the GPU pick among the model's top candidates (decision cached per workload shape)
-            base.bnd_cols = g.max_len;
-            if (!topk && h->autotune && !variant_forced(h) && est_ms_all >= 400.0 && ranked.size() > 1) {
-                uint64_t key = 1469598103934665603ull;
-                auto log2b = [](uint64_t x) { uint64_t b = 0; while (x >>= 1) ++b; return b; };
-                const uint64_t parts[] = {h->q_max_len, h->q_sum_len, (uint64_t)nq, g.max_len, log2b(g.npairs), log2b(g.sum_len),
-                                          (uint64_t)(uint16_t)h->params.match, (uint64_t)(uint16_t)h->params.mismatch,
-                                          (uint64_t)(uint16_t)h->params.gap_open, (uint64_t)(uint16_t)h->params.gap_extend,
-                                          (uint64_t)h->params.score_width, (uint64_t)g.out_mode};
-                for (uint64_t x : parts) { key ^= x; key *= 1099511628211ull; }
-                if (gc.tune_key != key || gc.tune_choice < 0) {
-                    int choice = vidx;
-                    // the sample launches append nothing: a pair they score is scored again by the real launch
-                    SwStripLaunch sample = base;
-                    if (hits) { sample.hits.keys = nullptr; sample.ovf_list = nullptr; sample.ovf_count = nullptr; }
-                    rc = autotune_variant(h, gc, g, sample, ranked, nq, same_len, &choice);
-                    if (rc != SW_OK) return rc;
-                    gc.tune_choice = choice;
-                    gc.tune_key = key;
-                }
-                vidx = gc.tune_choice;
-            }
-            // query chunks: a handful of launches so that D2H of finished rows overlaps compute
-            // (each launch has its own tail: aim for >= ~50 ms of work per launch, at ~6 TCUPS)
-            int nchunks = std::max(1, std::min(std::min(nq, 8), (int)(est_ms_all / 50.0)));
-            if (topk || hits || may_overflow || !wave_q.empty()) nchunks = 1;
-            // the device work counter is 32-bit: (pair blocks) x (queries per launch) must stay below 2^31
-            while (nchunks < nq && (uint64_t)(g.npairs / 4 + 1) * (uint64_t)((nq + nchunks - 1) / nchunks) >= (1ull << 31)) nchunks *= 2;
-            nchunks = std::min(nchunks, nq);
-            SwStripLaunch L = base;
-            L.vidx = vidx;
-            rc = strip_setup(h, gc, gc.d_bnd, g.npairs, g.max_len, smaxq, nq / nchunks, vidx, &L.grid, &L.chunk_passes, &L.bnd_elems);
-            if (rc != SW_OK) return rc;
-            L.superblock = superblock_for(sw_strip_variant(vidx), g.npairs, g.tp_words, L.grid, h->superblock_mb);
-            rc = plan_pass_split(h, gc, L, g.npairs, g.max_len, smaxq, (nq + nchunks - 1) / nchunks);
-            if (rc != SW_OK) return rc;
-            if (&gc == &h->gpus[0]) h->last_parts = std::max(1, L.nparts);
-            max_grid = L.grid;
-            label_v = vidx;
-            n_groups_total = 1;
-            if (h->jit && !sc.limit && (est_ms_all >= 2000.0 || h->jit >= 2) && std::strcmp(sw_strip_instance_kind(L), "runtime") == 0) {
-                L.jit_kernel = sw_jit_strip_kernel(sw_strip_variant(vidx), sc.goe, sc.ge, nullptr, 0);
-                jit_used = L.jit_kernel != nullptr;
-            }
-            // (A "tail split" -- the pairs of the last, partly filled round of equal work items on a
-            // side stream with a 2- or 4-lane variant -- was built and measured on 200 k x 1 kb x 10 kb:
-            // 262.9 ms against 261.0 ms without it.  The finer items gain what the slower variant loses.)
-            for (int c = 0; c < nchunks; ++c) {
-                const int a0 = (int)((long long)nq * c / nchunks), a1 = (int)((long long)nq * (c + 1) / nchunks);
-                if (a1 <= a0) continue;
-                Planned p{L, a0, a1, 0, 0.0};
-                p.L.q0 = a0; p.L.nql = a1 - a0; p.L.qidx = nullptr;
-                plan.push_back(p);
+// Variant of one (length group, query set) launch of the length-group plan: the highest throughput among
+// the variants with at least gmin lanes per pair whose longest work item takes at most tau seconds, else
+// the least throughput-plus-item cost.  *item_s = the chosen variant's longest work item.
+int pick_group_variant(const GpuCtx &gc, const Seg &sg, const uint32_t *ql, size_t nql, uint32_t maxq, int gmin, double tau,
+                       double *item_s)
+{
+    const int nv = sw_strip_variant_count();
+    if (const char *e = std::getenv("SW_B200_PLAN_FORCE")) {          // A/B measurements: this variant for every group
+        for (int i = 0; i < nv; ++i) if (std::strcmp(sw_strip_variant(i)->name, e) == 0) { *item_s = 1.0; return i; }
+    }
+    int best = -1, best_any = -1;
+    double best_thr = 0, best_any_cost = 0, best_item = 0, best_any_item = 0;
+    const double cols_avg = std::max(1.0, (double)sg.sum_len / (2.0 * std::max<uint32_t>(sg.p1 - sg.p0, 1)));
+    for (int i = 0; i < nv; ++i) {
+        const SwStripVariant *v = sw_strip_variant(i);
+        if (v->U != 4) continue;                                     // experimental instances: by name only
+        const int P = v->R * v->G, vpe = v->G * v->S;
+        double rows = 0;
+        for (size_t k = 0; k < nql; ++k) rows += (double)((ql[k] + P - 1) / P) * P;
+        const double speed = variant_speed_at(gc, v, sg.max_len) * 1e9;
+        const double thr = rows * (double)sg.sum_len * (cols_avg + vpe - 1) / cols_avg / speed;
+        const double qrows = (double)((maxq + P - 1) / P) * P;
+        const int ppb = v->block_threads / v->G;
+        const double item = qrows * ((double)sg.max_len + vpe - 1) * 2.0 * ppb * ((double)gc.num_sms * v->min_blocks) / speed;
+        const double any_cost = thr + item + (v->G < gmin ? 10.0 * thr : 0.0);
+        if (best_any < 0 || any_cost < best_any_cost) { best_any = i; best_any_cost = any_cost; best_any_item = item; }
+        if (v->G < gmin || item > tau) continue;
+        if (best < 0 || thr < best_thr) { best = i; best_thr = thr; best_item = item; }
+    }
+    *item_s = best >= 0 ? best_item : best_any_item;
+    return best >= 0 ? best : best_any;
+}
+
+// General case: every (length group, query group) gets its own launch and variant; launches run on
+// several streams so that the tail of one overlaps the start of the next, longest work items first.
+int plan_length_groups(sw_handle *h, ScoreJob &j, StripPlan &p, const std::vector<Seg> &segs)
+{
+    GpuCtx &gc = j.gc;
+    std::vector<int> &qidx_host = j.g.qidx_host;     // stays alive until this slot is scored again
+    qidx_host.clear();
+    // lanes needed to keep the GPU busy decide the least lanes per pair; the time budget of a
+    // single work item decides when a length group needs more lanes per pair than that
+    const double fill = (double)gc.num_sms * 3 * 128;
+    int gmin = 1;
+    while (gmin < 32 && (double)j.g.npairs * gmin * (double)j.strip_q.size() < 0.6 * fill) gmin *= 2;
+    const double t_total = (double)j.g.sum_len * (double)p.rows / 8.0e12;          // seconds, optimistic
+    const double tau = std::max(h->plan_tau * t_total, 1.0e-3);      // the longest items start first
+    std::map<int, uint64_t> rows_by_variant;
+    for (const Seg &sg : segs) {
+        if (sg.p1 <= sg.p0) continue;
+        // queries of this length group, grouped by the variant that suits them
+        std::map<int, std::vector<int>> by_variant;
+        std::map<int, double> item_of;
+        if (h->plan_qgroups) {
+            for (int q : j.strip_q) {
+                const uint32_t ql = h->q_len[q];
+                double it = 0;
+                const int v = pick_group_variant(gc, sg, &ql, 1, ql, gmin, tau, &it);
+                by_variant[v].push_back(q);
+                item_of[v] = std::max(item_of[v], it);
             }
         } else {
-            // lanes needed to keep the GPU busy decide the least lanes per pair; the time budget of a
-            // single work item decides when a length group needs more lanes per pair than that
-            const double fill = (double)gc.num_sms * 3 * 128;
-            int gmin = 1;
-            while (gmin < 32 && (double)g.npairs * gmin * (double)strip_q.size() < 0.6 * fill) gmin *= 2;
-            const double t_total = (double)g.sum_len * (double)srows / 8.0e12;          // seconds, optimistic
-            const double tau = std::max(h->plan_tau * t_total, 1.0e-3);      // the longest items start first
-            const int nv = sw_strip_variant_count();
-            auto pick = [&](const Seg &sg, const uint32_t *ql, size_t nql, uint32_t maxq, double *item_s) {
-                if (const char *e = std::getenv("SW_B200_PLAN_FORCE")) {          // A/B measurements: this variant for every group
-                    for (int i = 0; i < nv; ++i) if (std::strcmp(sw_strip_variant(i)->name, e) == 0) { *item_s = 1.0; return i; }
-                }
-                int best = -1, best_any = -1;
-                double best_thr = 0, best_any_cost = 0, best_item = 0, best_any_item = 0;
-                const double cols_avg = std::max(1.0, (double)sg.sum_len / (2.0 * std::max<uint32_t>(sg.p1 - sg.p0, 1)));
-                for (int i = 0; i < nv; ++i) {
-                    const SwStripVariant *v = sw_strip_variant(i);
-                    if (v->U != 4) continue;                                     // experimental instances: by name only
-                    const int P = v->R * v->G, vpe = v->G * v->S;
-                    double rows = 0;
-                    for (size_t k = 0; k < nql; ++k) rows += (double)((ql[k] + P - 1) / P) * P;
-                    const double speed = variant_speed_at(gc, v, sg.max_len) * 1e9;
-                    const double thr = rows * (double)sg.sum_len * (cols_avg + vpe - 1) / cols_avg / speed;
-                    const double qrows = (double)((maxq + P - 1) / P) * P;
-                    const int ppb = v->block_threads / v->G;
-                    const double item = qrows * ((double)sg.max_len + vpe - 1) * 2.0 * ppb * ((double)gc.num_sms * v->min_blocks) / speed;
-                    const double any_cost = thr + item + (v->G < gmin ? 10.0 * thr : 0.0);
-                    if (best_any < 0 || any_cost < best_any_cost) { best_any = i; best_any_cost = any_cost; best_any_item = item; }
-                    if (v->G < gmin || item > tau) continue;
-                    if (best < 0 || thr < best_thr) { best = i; best_thr = thr; best_item = item; }
-                }
-                *item_s = best >= 0 ? best_item : best_any_item;
-                return best >= 0 ? best : best_any;
-            };
-            std::map<int, uint64_t> rows_by_variant;
-            for (const Seg &sg : segs) {
-                if (sg.p1 <= sg.p0) continue;
-                // queries of this length group, grouped by the variant that suits them
-                std::map<int, std::vector<int>> by_variant;
-                std::map<int, double> item_of;
-                if (h->plan_qgroups) {
-                    for (int q : strip_q) {
-                        const uint32_t ql = h->q_len[q];
-                        double it = 0;
-                        const int v = pick(sg, &ql, 1, ql, &it);
-                        by_variant[v].push_back(q);
-                        item_of[v] = std::max(item_of[v], it);
-                    }
-                } else {
-                    double it = 0;
-                    const int v = pick(sg, sl.data(), sl.size(), smaxq, &it);
-                    by_variant[v] = strip_q;
-                    item_of[v] = it;
-                }
-                // fold small groups into the largest one of this length group (every launch has a tail)
-                int big = -1;
-                uint64_t big_rows = 0, all_rows = 0;
-                std::map<int, uint64_t> vrows;
-                for (auto &kv : by_variant) {
-                    uint64_t r = 0;
-                    for (int q : kv.second) r += h->q_len[q];
-                    vrows[kv.first] = r;
-                    all_rows += r;
-                    if (r >= big_rows) { big_rows = r; big = kv.first; }
-                }
-                for (auto it = by_variant.begin(); it != by_variant.end();) {
-                    const double ms = (double)sg.sum_len * (double)vrows[it->first] / 8.0e9;
-                    if (it->first != big && (ms < 2.0 || (double)vrows[it->first] < 0.03 * (double)all_rows)) {
-                        std::vector<int> &dst = by_variant[big];
-                        dst.insert(dst.end(), it->second.begin(), it->second.end());
-                        vrows[big] += vrows[it->first];
-                        it = by_variant.erase(it);
-                    } else {
-                        ++it;
-                    }
-                }
-                for (auto &kv : by_variant) {
-                    std::vector<int> &ql = kv.second;
-                    // longest queries first inside a super-block: the longest work items start earliest
-                    std::sort(ql.begin(), ql.end(), [&](int x, int y) { return h->q_len[x] != h->q_len[y] ? h->q_len[x] > h->q_len[y] : x < y; });
-                    uint32_t gmaxq = 0;
-                    for (int q : ql) gmaxq = std::max(gmaxq, h->q_len[q]);
-                    Planned p{base, 0, 0, 0, item_of[kv.first]};
-                    SwStripLaunch &L = p.L;
-                    L.vidx = kv.first;
-                    // this length group's window of the pair list
-                    L.db.pair_subj = db.pair_subj + 2 * (size_t)sg.p0;
-                    L.db.pair_len = db.pair_len + 2 * (size_t)sg.p0;
-                    L.db.tile_woff = db.tile_woff + sg.p0 / 32;
-                    L.db.npairs = sg.p1 - sg.p0;
-                    L.db.max_len = sg.max_len;
-                    L.bnd_cols = sg.max_len;
-                    L.q0 = 0; L.nql = (int)ql.size();
-                    L.qidx = (const int *)(uintptr_t)qidx_host.size();          // offset for now, pointer after the upload
-                    qidx_host.insert(qidx_host.end(), ql.begin(), ql.end());
-                    rows_by_variant[kv.first] += vrows[kv.first] * (sg.sum_len >> 8);
-                    plan.push_back(p);
-                    ++n_groups_total;
-                }
+            double it = 0;
+            const int v = pick_group_variant(gc, sg, p.qlen.data(), p.qlen.size(), p.maxq, gmin, tau, &it);
+            by_variant[v] = j.strip_q;
+            item_of[v] = it;
+        }
+        // fold small groups into the largest one of this length group (every launch has a tail)
+        int big = -1;
+        uint64_t big_rows = 0, all_rows = 0;
+        std::map<int, uint64_t> vrows;
+        for (auto &kv : by_variant) {
+            uint64_t r = 0;
+            for (int q : kv.second) r += h->q_len[q];
+            vrows[kv.first] = r;
+            all_rows += r;
+            if (r >= big_rows) { big_rows = r; big = kv.first; }
+        }
+        for (auto it = by_variant.begin(); it != by_variant.end();) {
+            const double ms = (double)sg.sum_len * (double)vrows[it->first] / 8.0e9;
+            if (it->first != big && (ms < 2.0 || (double)vrows[it->first] < 0.03 * (double)all_rows)) {
+                std::vector<int> &dst = by_variant[big];
+                dst.insert(dst.end(), it->second.begin(), it->second.end());
+                vrows[big] += vrows[it->first];
+                it = by_variant.erase(it);
+            } else {
+                ++it;
             }
-            // longest work items first, round-robin over the streams
-            std::stable_sort(plan.begin(), plan.end(), [](const Planned &x, const Planned &y) { return x.item_s > y.item_s; });
-            const int ns_used = topk ? 1 : h->plan_streams;   // top-k lists are per block index: one kernel at a time
-            for (size_t i = 0; i < plan.size(); ++i) plan[i].stream = (int)(i % ns_used);
-            SW_CUDA(h, gc.d_qidx.reserve(std::max<size_t>(1, qidx_host.size()) * sizeof(int)));
-            for (Planned &p : plan) {
-                SwStripLaunch &L = p.L;
-                const size_t off = (size_t)(uintptr_t)L.qidx;
-                L.qidx = gc.d_qidx.as<int>() + off;
-                uint32_t gmaxq = 0;
-                for (int k = 0; k < L.nql; ++k) gmaxq = std::max(gmaxq, h->q_len[qidx_host[off + k]]);
-                DevBuf &bb = p.stream == 0 ? gc.d_bnd : gc.d_bnd_aux[p.stream - 1];
-                rc = strip_setup(h, gc, bb, L.db.npairs, L.db.max_len, gmaxq, L.nql, L.vidx, &L.grid, &L.chunk_passes, &L.bnd_elems);
-                if (rc != SW_OK) return rc;
-                // more work items than the 32-bit work counter can address: does not happen per length group
-                max_grid = std::max(max_grid, L.grid);
-                if (h->jit >= 2 && !sc.limit && std::strcmp(sw_strip_instance_kind(L), "runtime") == 0) {
-                    L.jit_kernel = sw_jit_strip_kernel(sw_strip_variant(L.vidx), sc.goe, sc.ge, nullptr, 0);
-                    jit_used |= L.jit_kernel != nullptr;
-                }
-            }
-            uint64_t lr = 0;
-            for (auto &kv : rows_by_variant) if (kv.second >= lr) { lr = kv.second; label_v = kv.first; }
-            SW_CUDA(h, cudaMemcpyAsync(gc.d_qidx.p, qidx_host.data(), qidx_host.size() * sizeof(int), cudaMemcpyHostToDevice, gc.st_compute));
+        }
+        for (auto &kv : by_variant) {
+            std::vector<int> &ql = kv.second;
+            // longest queries first inside a super-block: the longest work items start earliest
+            std::sort(ql.begin(), ql.end(), [&](int x, int y) { return h->q_len[x] != h->q_len[y] ? h->q_len[x] > h->q_len[y] : x < y; });
+            Planned pl{j.base, 0, 0, 0, item_of[kv.first]};
+            SwStripLaunch &L = pl.L;
+            L.vidx = kv.first;
+            // this length group's window of the pair list
+            L.db.pair_subj = j.db.pair_subj + 2 * (size_t)sg.p0;
+            L.db.pair_len = j.db.pair_len + 2 * (size_t)sg.p0;
+            L.db.tile_woff = j.db.tile_woff + sg.p0 / 32;
+            L.db.npairs = sg.p1 - sg.p0;
+            L.db.max_len = sg.max_len;
+            L.bnd_cols = sg.max_len;
+            L.q0 = 0; L.nql = (int)ql.size();
+            L.qidx = (const int *)(uintptr_t)qidx_host.size();          // offset for now, pointer after the upload
+            qidx_host.insert(qidx_host.end(), ql.begin(), ql.end());
+            rows_by_variant[kv.first] += vrows[kv.first] * (sg.sum_len >> 8);
+            p.launches.push_back(pl);
+            ++p.n_groups;
         }
     }
-    if (&gc == &h->gpus[0]) {      // one writer: the per-GPU workers run concurrently
-        if (label_v >= 0)
-            std::snprintf(h->last_kernel, sizeof h->last_kernel, "%s%s%s", sw_strip_variant(label_v)->name, jit_used ? "+jit" : "",
-                          n_groups_total > 1 ? "+groups" : "");
-        else
-            std::snprintf(h->last_kernel, sizeof h->last_kernel, "%s", wave_q.empty() ? "generic32" : sw_wave_kernel_name(0));
-        if (!wave_q.empty() && label_v >= 0) {
-            uint64_t wrows = 0;
-            for (int q : wave_q) wrows += h->q_len[q];
-            if (2 * wrows > h->q_sum_len) std::snprintf(h->last_kernel, sizeof h->last_kernel, "%s+groups", sw_wave_kernel_name(0));
+    // longest work items first, round-robin over the streams
+    std::stable_sort(p.launches.begin(), p.launches.end(), [](const Planned &x, const Planned &y) { return x.item_s > y.item_s; });
+    const int ns_used = j.topk ? 1 : h->plan_streams;   // top-k lists are per block index: one kernel at a time
+    for (size_t i = 0; i < p.launches.size(); ++i) p.launches[i].stream = (int)(i % ns_used);
+    SW_CUDA(h, gc.d_qidx.reserve(std::max<size_t>(1, qidx_host.size()) * sizeof(int)));
+    for (Planned &pl : p.launches) {
+        SwStripLaunch &L = pl.L;
+        const size_t off = (size_t)(uintptr_t)L.qidx;
+        L.qidx = gc.d_qidx.as<int>() + off;
+        uint32_t gmaxq = 0;
+        for (int k = 0; k < L.nql; ++k) gmaxq = std::max(gmaxq, h->q_len[qidx_host[off + k]]);
+        DevBuf &bb = pl.stream == 0 ? gc.d_bnd : gc.d_bnd_aux[pl.stream - 1];
+        SW_TRY(strip_setup(h, gc, bb, L.db.npairs, L.db.max_len, gmaxq, L.nql, L.vidx, &L.grid, &L.chunk_passes, &L.bnd_elems));
+        // more work items than the 32-bit work counter can address: does not happen per length group
+        p.max_grid = std::max(p.max_grid, L.grid);
+        if (h->jit >= 2 && !j.sc.limit && std::strcmp(sw_strip_instance_kind(L), "runtime") == 0) {
+            L.jit_kernel = sw_jit_strip_kernel(sw_strip_variant(L.vidx), j.sc.goe, j.sc.ge, nullptr, 0);
+            p.jit_used |= L.jit_kernel != nullptr;
         }
     }
-    const bool have_strip = !plan.empty();
+    uint64_t lr = 0;
+    for (auto &kv : rows_by_variant) if (kv.second >= lr) { lr = kv.second; p.label_v = kv.first; }
+    SW_CUDA(h, cudaMemcpyAsync(gc.d_qidx.p, qidx_host.data(), qidx_host.size() * sizeof(int), cudaMemcpyHostToDevice, gc.st_compute));
+    return SW_OK;
+}
 
-    const bool use32 = !have_strip && wave_q.empty();        // forced 32-bit scorer
-    if (topk) {
-        if (!have_strip && wave_q.empty()) return SW_EINVAL;  // the 32-bit scorer has no top-k epilogue
-        if (!wave_q.empty()) max_grid = std::max(max_grid, 1);      // list 0 also takes the rows of the band-pipelined queries
-        const size_t bytes = (size_t)max_grid * nq * g.topk_k * sizeof(unsigned long long);
+// Launch plan of the strip queries: one launch (query chunks) or one per (length group, query group).
+int plan_strip(sw_handle *h, ScoreJob &j, StripPlan &p)
+{
+    const Slot &g = j.g;
+    for (int q : j.strip_q) { p.qlen.push_back(h->q_len[q]); p.maxq = std::max(p.maxq, h->q_len[q]); p.rows += h->q_len[q]; }
+    p.same_len = std::all_of(p.qlen.begin(), p.qlen.end(), [&](uint32_t x) { return x == p.qlen[0]; });
+    std::vector<Seg> segs = g.segs;
+    bool use_segs = h->plan_segs == 1;
+    if (h->plan_segs == 2 && segs.size() > 1) {
+        // one launch over everything sizes every block's pass-boundary scratch by the longest subject
+        const size_t worst = (size_t)j.gc.num_sms * 4 * 128 * (size_t)g.max_len * sizeof(uint2);
+        use_segs = p.maxq > 64 && worst > ((size_t)4 << 30);
+    }
+    if (segs.empty() || variant_forced(h) || !use_segs) segs.assign(1, Seg{0, g.npairs, g.max_len, g.sum_len});
+    p.simple = (int)j.strip_q.size() == j.nq && segs.size() == 1 && (variant_forced(h) || p.same_len || j.strip_q.size() == 1);
+    return p.simple ? plan_one_launch(h, j, p) : plan_length_groups(h, j, p, segs);
+}
+
+// Band-pipelined instance for a query of qlen rows.  Pair-bands of 256 rows in its launch: many ->
+// throughput-bound (512-row bands, four pairs per block); fewer -> one pair per block, four columns per
+// step; a handful -> two columns per step; many pairs of long subjects -> 512-row bands with two
+// columns per step (measured crossovers, DESIGN.md section 5)
+int wave_instance(const Slot &g, uint32_t qlen)
+{
+    const size_t warps256 = (size_t)g.npairs * ((qlen + 255) / 256);
+    const double mean_len = (double)g.sum_len / (2.0 * std::max<uint32_t>(g.npairs, 1));
+    int wi = warps256 < 1200 ? 2 : warps256 < 15000 ? 1 : mean_len >= 1000.0 ? 3 : 0;
+    if (const char *e = std::getenv("SW_B200_WAVE_INSTANCE")) {       // A/B measurements
+        const int w = std::atoi(e);
+        if (w >= 0 && w < sw_wave_instance_count() && w < 16) wi = w;
+    }
+    return wi;
+}
+
+// last_kernel of a regular scoring (written by GPU 0 only: the per-GPU workers run concurrently).
+void set_kernel_label(sw_handle *h, const ScoreJob &j, const StripPlan &p)
+{
+    uint64_t wrows = 0;
+    for (int q : j.wave_q) wrows += h->q_len[q];
+    if (p.label_v >= 0 && 2 * wrows > h->q_sum_len)      // most rows on the band-pipelined kernel
+        std::snprintf(h->last_kernel, sizeof h->last_kernel, "%s+groups", sw_wave_kernel_name(0));
+    else if (p.label_v >= 0)
+        std::snprintf(h->last_kernel, sizeof h->last_kernel, "%s%s%s", sw_strip_variant(p.label_v)->name, p.jit_used ? "+jit" : "",
+                      p.n_groups > 1 ? "+groups" : "");
+    else if (!j.wave_q.empty())        // the instance of the last band-pipelined launch
+        std::snprintf(h->last_kernel, sizeof h->last_kernel, "%s", sw_wave_kernel_name(wave_instance(j.g, h->q_len[j.wave_q.back()])));
+    else
+        std::snprintf(h->last_kernel, sizeof h->last_kernel, "generic32");
+}
+
+// The plan's strip launches; side streams start from the compute stream and are joined into it at the end.
+int enqueue_strip(sw_handle *h, ScoreJob &j, StripPlan &p)
+{
+    GpuCtx &gc = j.gc;
+    const bool chunk_events = p.simple && p.launches.size() > 1 && !j.may_overflow && !j.topk && !j.hits;
+    bool forked[kStreams] = {false, false, false, false};
+    for (Planned &pl : p.launches) {
+        SwStripLaunch &L = pl.L;
+        cudaStream_t st = gc.st_compute;
+        if (pl.stream > 0) {
+            st = gc.st_aux[pl.stream - 1];
+            if (!forked[pl.stream]) {
+                // the side streams start after everything queued on the compute stream so far
+                // (output memset, query lists, an earlier batch's kernels)
+                if (!forked[0]) { SW_CUDA(h, cudaEventRecord(gc.ev_fork, gc.st_compute)); forked[0] = true; }
+                SW_CUDA(h, cudaStreamWaitEvent(st, gc.ev_fork, 0));
+                forked[pl.stream] = true;
+            }
+        }
+        L.bnd = (pl.stream == 0 ? gc.d_bnd : gc.d_bnd_aux[pl.stream - 1]).as<uint2>();
+        SW_CUDA(h, assign_counters(gc, L, st, L.nparts > 1 ? 0 : h->sticky, p.simple && p.same_len, j.g.tp_words));
+        if (L.nparts > 1) {
+            const size_t chains = (size_t)pair_blocks(sw_strip_variant(L.vidx), L.db.npairs) * (size_t)L.nql;
+            SW_CUDA(h, cudaMemsetAsync(L.part_done, 0, chains * sizeof(unsigned), st));
+        }
+        if (j.topk) { L.topk_keys = gc.d_topk_keys.as<unsigned long long>(); L.topk_k = j.bt.topk_k; L.topk_nq = j.nq; }
+        SW_CUDA(h, sw_launch_strip(st, L));
+        h->launches++;
+        if (chunk_events) {
+            SW_TRY(push_chunk(h, gc, j.g, pl.q0, pl.q1));
+        }
+    }
+    for (int k = 1; k < kStreams; ++k) {
+        if (!forked[k]) continue;
+        SW_CUDA(h, cudaEventRecord(gc.ev_join[k - 1], gc.st_aux[k - 1]));
+        SW_CUDA(h, cudaStreamWaitEvent(gc.st_compute, gc.ev_join[k - 1], 0));
+    }
+    return SW_OK;
+}
+
+// Band-pipelined launches, one per long query (top-k / hits: into a scratch row per query, filtered from there).
+int enqueue_wave(sw_handle *h, ScoreJob &j)
+{
+    GpuCtx &gc = j.gc; const Slot &g = j.g;
+    const size_t n = j.n;
+    const uint32_t cols_stride = ((g.max_len + 31u) & ~31u) + 32u;    // + slack for the batched boundary stores (kWaveSlack)
+    // tagged 16-byte boundary elements; zeroed once (tag 0 is never used), later launches
+    // are told apart by the epoch in the tag
+    const size_t bnd_bytes = (size_t)g.npairs * 2 * cols_stride * 16;
+    if (gc.d_wave_bnd.cap < bnd_bytes || !gc.d_wave_bnd.p) {
+        SW_CUDA(h, grow_shared(gc, gc.d_wave_bnd, bnd_bytes));
+        SW_CUDA(h, cudaMemsetAsync(gc.d_wave_bnd.p, 0, gc.d_wave_bnd.cap, gc.st_compute));
+    }
+    // state words: best [2 * npairs] | done [npairs]
+    const size_t n_state = 3 * (size_t)g.npairs;
+    SW_CUDA(h, gc.d_wave_state.reserve(n_state * sizeof(unsigned)));
+    int wave_row = -1;
+    for (int q : j.wave_q) {
+        ++wave_row;
+        SwWaveLaunch W;
+        W.instance = wave_instance(g, h->q_len[q]);
+        if (!gc.wave_bps[W.instance]) SW_CUDA(h, sw_wave_occupancy(W.instance, &gc.wave_bps[W.instance]));
+        if (gc.wave_bps[W.instance] < 1) return SW_ECUDA;
+        const int rows = sw_wave_rows_per_band(W.instance);
+        W.db = j.db; W.q = j.dq; W.query = q; W.sc = j.sc;
+        W.npass = (int)((h->q_len[q] + rows - 1) / rows);
+        W.out = g.d_out.p; W.out_stride = n; W.out_mode = j.bt.out_mode;
+        if (j.topk || j.hits) { W.out = gc.d_wave_rows.p; W.out_mode = SW_OUT_I32; W.out_row = wave_row; }
+        W.bnd = gc.d_wave_bnd.p; W.cols_stride = cols_stride;
+        W.bnd_elems = (size_t)g.npairs * 2 * cols_stride; W.out_elems = (j.topk || j.hits) ? j.wave_q.size() * n : (size_t)j.nq * n;
+        gc.wave_epoch = (gc.wave_epoch % 0xFFFFEu) + 1u;            // 1 .. 2^20 - 2
+        if (gc.wave_epoch == 1u && gc.counter_next > 0) {
+            // the epoch wrapped (or first use): stale tags must not match again
+            SW_CUDA(h, cudaMemsetAsync(gc.d_wave_bnd.p, 0, gc.d_wave_bnd.cap, gc.st_compute));
+        }
+        W.epoch = gc.wave_epoch;
+        W.best = (int *)gc.d_wave_state.as<unsigned>();
+        W.done = gc.d_wave_state.as<unsigned>() + 2 * (size_t)g.npairs;
+        W.counter = next_counter(gc);
+        const size_t ppb = (size_t)sw_wave_pairs_per_block(W.instance);
+        const size_t items = (size_t)W.npass * ((g.npairs + ppb - 1) / ppb);
+        W.grid = (int)std::min<size_t>(items, (size_t)gc.num_sms * gc.wave_bps[W.instance]);
+        W.ovf_count = j.base.ovf_count; W.ovf_list = j.base.ovf_list; W.ovf_cap = j.base.ovf_cap;
+        W.dev_err = gc.d_err.as<unsigned>();
+        SW_CUDA(h, cudaMemsetAsync(gc.d_wave_state.p, 0, n_state * sizeof(unsigned), gc.st_compute));
+        SW_CUDA(h, cudaMemsetAsync(W.counter, 0, sizeof(unsigned), gc.st_compute));
+        SW_CUDA(h, sw_launch_wave(gc.st_compute, W));
+        h->launches++;
+        if (!j.topk && !j.hits) continue;
+        const int32_t *row = (const int32_t *)gc.d_wave_rows.p + (size_t)wave_row * n;
+        if (j.topk)         // the row's k best scores become list 0 of this query (pairs flagged for the 32-bit
+                            // scorer keep the sentinel here and reach the merge through the overflow list)
+            SW_CUDA(h, sw_launch_topk_row(gc.st_compute, row, (uint32_t)n, q, j.bt.topk_k, gc.d_topk_keys.as<unsigned long long>()));
+        else                // the row's entries >= min_score join the list (flagged pairs come from the overflow list)
+            SW_CUDA(h, sw_launch_hits_row(gc.st_compute, row, (uint32_t)n, q, j.hl));
+        h->launches++;
+    }
+    return SW_OK;
+}
+
+// Scratch of the launches, zeroed where they need it: top-k key lists, score rows of the band-pipelined queries
+// (top-k / hits), and the 32-bit scorer's (force32, or the overflow fix-up of the few listed pairs) with its launch.
+int reserve_scratch(sw_handle *h, const ScoreJob &j, StripPlan &p, bool use32, SwScore32Launch &s32)
+{
+    GpuCtx &gc = j.gc;
+    if (j.topk) {
+        if (!j.wave_q.empty()) p.max_grid = std::max(p.max_grid, 1);      // list 0 also takes the rows of the band-pipelined queries
+        const size_t bytes = (size_t)p.max_grid * j.nq * j.bt.topk_k * sizeof(unsigned long long);
         SW_CUDA(h, gc.d_topk_keys.reserve(bytes));
         SW_CUDA(h, cudaMemsetAsync(gc.d_topk_keys.p, 0, bytes, gc.st_compute));
     }
-
-    if (hits && use32) return SW_EINVAL;                      // (rejected at submit: the 32-bit scorer has no hit list)
-    if ((topk || hits) && !wave_q.empty()) {
-        const size_t rb = wave_q.size() * (size_t)n * sizeof(int32_t);
+    if ((j.topk || j.hits) && !j.wave_q.empty()) {
+        const size_t rb = j.wave_q.size() * j.n * sizeof(int32_t);
         SW_CUDA(h, gc.d_wave_rows.reserve(rb));
         SW_CUDA(h, cudaMemsetAsync(gc.d_wave_rows.p, 0xFF, rb, gc.st_compute));    // -1 = not scored here
     }
-
-    // 32-bit scratch (force32, or the overflow fix-up of the few listed pairs)
-    const uint32_t max_cols = std::max<uint32_t>(1, std::min<uint32_t>(h->q_max_len, g.max_len));
+    const uint32_t max_cols = std::max<uint32_t>(1, std::min<uint32_t>(h->q_max_len, j.g.max_len));
     int threads32 = 0;
-    if (use32 || may_overflow) {
+    if (use32 || j.may_overflow) {
         const size_t budget = (size_t)1 << 30;
         size_t t = budget / ((size_t)2 * max_cols * sizeof(int32_t));
         t = std::min<size_t>(t, use32 ? (size_t)gc.num_sms * 2 * 128 : 4096);
@@ -1243,202 +1350,148 @@ int score_gpu(sw_handle *h, GpuCtx &gc, Slot &g)
         threads32 = (int)t;
         SW_CUDA(h, gc.d_scratch32.reserve((size_t)2 * max_cols * threads32 * sizeof(int32_t)));
     }
-    SwScore32Launch s32;
-    s32.db = db; s32.q = dq; s32.sc = sc; s32.out = (topk || hits) ? nullptr : g.d_out.p; s32.out_stride = n; s32.out_mode = g.out_mode;
-    s32.scratch = gc.d_scratch32.as<int32_t>(); s32.max_cols = max_cols; s32.threads_total = threads32;
+    s32.db = j.db; s32.q = j.dq; s32.sc = j.sc; s32.out = (j.topk || j.hits) ? nullptr : j.g.d_out.p; s32.out_stride = j.n;
+    s32.out_mode = j.bt.out_mode; s32.scratch = gc.d_scratch32.as<int32_t>(); s32.max_cols = max_cols; s32.threads_total = threads32;
+    return SW_OK;
+}
 
-    size_t nev = 0;
-    if (!use32) {
-        const bool chunk_events = simple && plan.size() > 1 && !may_overflow && !topk && !hits;
-        bool forked[kStreams] = {false, false, false, false};
-        for (size_t i = 0; i < plan.size(); ++i) {
-            Planned &p = plan[i];
-            cudaStream_t st = gc.st_compute;
-            if (p.stream > 0) {
-                st = gc.st_aux[p.stream - 1];
-                if (!forked[p.stream]) {
-                    // the side streams start after everything queued on the compute stream so far
-                    // (output memset, query lists, an earlier batch's kernels)
-                    if (!forked[0]) { SW_CUDA(h, cudaEventRecord(gc.ev_fork, gc.st_compute)); forked[0] = true; }
-                    SW_CUDA(h, cudaStreamWaitEvent(st, gc.ev_fork, 0));
-                    forked[p.stream] = true;
-                }
-            }
-            p.L.bnd = (p.stream == 0 ? gc.d_bnd : gc.d_bnd_aux[p.stream - 1]).as<uint2>();
-            SW_CUDA(h, assign_counters(gc, p.L, st, p.L.nparts > 1 ? 0 : h->sticky, simple && sticky_ok, g.tp_words));
-            if (p.L.nparts > 1) {
-                const SwStripVariant *pv = sw_strip_variant(p.L.vidx);
-                const size_t chains = (size_t)((p.L.db.npairs + pv->block_threads / pv->G - 1) / (pv->block_threads / pv->G)) * (size_t)p.L.nql;
-                SW_CUDA(h, cudaMemsetAsync(p.L.part_done, 0, chains * sizeof(unsigned), st));
-            }
-            if (topk) { p.L.topk_keys = gc.d_topk_keys.as<unsigned long long>(); p.L.topk_k = g.topk_k; p.L.topk_nq = nq; }
-            SW_CUDA(h, sw_launch_strip(st, p.L));
-            h->launches++;
-            if (chunk_events) {
-                QueryChunk qc{p.q0, p.q1, pool_event(h, g, nev++, &rc)};
-                if (rc != SW_OK) return rc;
-                SW_CUDA(h, cudaEventRecord(qc.done, gc.st_compute));
-                g.chunks.push_back(qc);
-            }
+// Exact scores of the pairs on the overflow list: long entries on the band-pipelined 32-bit scorer, the
+// rest on the 32-bit scorer; in hits mode the list's entries >= min_score then join the hit list.
+int enqueue_overflow(sw_handle *h, ScoreJob &j, SwScore32Launch &s32)
+{
+    GpuCtx &gc = j.gc; const Slot &g = j.g;
+    s32.mode = 2; s32.list_count = g.d_ovf_count.as<unsigned>(); s32.list = g.d_ovf_list.as<uint2>();
+    s32.list_cap = kOvfCap; s32.list_score = g.d_ovf_score.as<int32_t>();
+    if (h->wave32) {
+        // long entries (with the default scoring every entry is >= 6 400 x 6 400 nt) are scored
+        // by bands on many warps; the launch is list-driven, so nothing is read back here
+        SwWave32Launch W;
+        W.db = j.db; W.q = j.dq; W.sc = j.sc;
+        W.list_count = s32.list_count; W.list = s32.list; W.list_cap = kOvfCap; W.list_score = s32.list_score;
+        W.out = s32.out; W.out_stride = j.n; W.out_elems = (size_t)j.nq * j.n; W.out_mode = j.bt.out_mode;
+        W.cols_stride = ((g.max_len + 31u) & ~31u) + 32u;
+        const size_t per_slot = (size_t)2 * W.cols_stride * 16;
+        W.nslots = (uint32_t)std::min<size_t>(64, std::max<size_t>(2, ((size_t)64 << 20) / per_slot));
+        W.bnd_elems = (size_t)W.nslots * 2 * W.cols_stride;
+        bool fresh = false;
+        if (gc.d_wave32_bnd.cap < W.bnd_elems * 16 || !gc.d_wave32_bnd.p) {
+            SW_CUDA(h, grow_shared(gc, gc.d_wave32_bnd, W.bnd_elems * 16));
+            fresh = true;
         }
-        for (int k = 1; k < kStreams; ++k) {
-            if (!forked[k]) continue;
-            SW_CUDA(h, cudaEventRecord(gc.ev_join[k - 1], gc.st_aux[k - 1]));
-            SW_CUDA(h, cudaStreamWaitEvent(gc.st_compute, gc.ev_join[k - 1], 0));
-        }
-        // ---- band-pipelined launches, one per long query ----------------------------------------
-        if (!wave_q.empty()) {
-            const uint32_t cols_stride = ((g.max_len + 31u) & ~31u) + 32u;    // + slack for the batched boundary stores (kWaveSlack)
-            uint32_t wmaxq = 0;
-            for (int q : wave_q) wmaxq = std::max(wmaxq, h->q_len[q]);
-            (void)wmaxq;
-            {
-                // tagged 16-byte boundary elements; zeroed once (tag 0 is never used), later launches
-                // are told apart by the epoch in the tag
-                const size_t bytes = (size_t)g.npairs * 2 * cols_stride * 16;
-                if (gc.d_wave_bnd.cap < bytes || !gc.d_wave_bnd.p) {
-                    SW_CUDA(h, cudaStreamSynchronize(gc.st_compute));
-                    SW_CUDA(h, gc.d_wave_bnd.reserve(bytes));
-                    SW_CUDA(h, cudaMemsetAsync(gc.d_wave_bnd.p, 0, gc.d_wave_bnd.cap, gc.st_compute));
-                }
-            }
-            // state words: best [2 * npairs] | done [npairs]
-            const size_t n_state = 3 * (size_t)g.npairs;
-            SW_CUDA(h, gc.d_wave_state.reserve(n_state * sizeof(unsigned)));
-            int wave_row = -1;
-            for (int q : wave_q) {
-                ++wave_row;
-                SwWaveLaunch W;
-                // pair-bands of 256 rows in this launch: many -> throughput-bound (512-row bands,
-                // four pairs per block); fewer -> one pair per block, four columns per step; a
-                // handful -> two columns per step; many pairs of long subjects -> 512-row bands with two
-                // columns per step (measured crossovers, DESIGN.md section 5)
-                const size_t warps256 = (size_t)g.npairs * ((h->q_len[q] + 255) / 256);
-                const double mean_len = (double)g.sum_len / (2.0 * std::max<uint32_t>(g.npairs, 1));
-                W.instance = warps256 < 1200 ? 2 : warps256 < 15000 ? 1 : mean_len >= 1000.0 ? 3 : 0;
-                if (const char *e = std::getenv("SW_B200_WAVE_INSTANCE")) {       // A/B measurements
-                    const int wi = std::atoi(e);
-                    if (wi >= 0 && wi < sw_wave_instance_count() && wi < 16) W.instance = wi;
-                }
-                if (!gc.wave_bps[W.instance]) SW_CUDA(h, sw_wave_occupancy(W.instance, &gc.wave_bps[W.instance]));
-                if (gc.wave_bps[W.instance] < 1) return SW_ECUDA;
-                const int rows = sw_wave_rows_per_band(W.instance);
-                W.db = db; W.q = dq; W.query = q; W.sc = sc;
-                W.npass = (int)((h->q_len[q] + rows - 1) / rows);
-                W.out = g.d_out.p; W.out_stride = n; W.out_mode = g.out_mode;
-                if (topk || hits) { W.out = gc.d_wave_rows.p; W.out_mode = SW_OUT_I32; W.out_row = wave_row; }
-                W.bnd = gc.d_wave_bnd.p; W.cols_stride = cols_stride;
-                W.bnd_elems = (size_t)g.npairs * 2 * cols_stride; W.out_elems = (topk || hits) ? wave_q.size() * (size_t)n : (size_t)nq * n;
-                gc.wave_epoch = (gc.wave_epoch % 0xFFFFEu) + 1u;            // 1 .. 2^20 - 2
-                if (gc.wave_epoch == 1u && gc.counter_next > 0) {
-                    // the epoch wrapped (or first use): stale tags must not match again
-                    SW_CUDA(h, cudaMemsetAsync(gc.d_wave_bnd.p, 0, gc.d_wave_bnd.cap, gc.st_compute));
-                }
-                W.epoch = gc.wave_epoch;
-                W.best = (int *)gc.d_wave_state.as<unsigned>();
-                W.done = gc.d_wave_state.as<unsigned>() + 2 * (size_t)g.npairs;
-                W.counter = next_counter(gc);
-                const size_t ppb = (size_t)sw_wave_pairs_per_block(W.instance);
-                const size_t items = (size_t)W.npass * ((g.npairs + ppb - 1) / ppb);
-                W.grid = (int)std::min<size_t>(items, (size_t)gc.num_sms * gc.wave_bps[W.instance]);
-                W.ovf_count = base.ovf_count; W.ovf_list = base.ovf_list; W.ovf_cap = base.ovf_cap;
-                W.dev_err = gc.d_err.as<unsigned>();
-                SW_CUDA(h, cudaMemsetAsync(gc.d_wave_state.p, 0, n_state * sizeof(unsigned), gc.st_compute));
-                SW_CUDA(h, cudaMemsetAsync(W.counter, 0, sizeof(unsigned), gc.st_compute));
-                SW_CUDA(h, sw_launch_wave(gc.st_compute, W));
-                h->launches++;
-                if (topk) {
-                    // the row's k best scores become list 0 of this query (pairs flagged for the 32-bit
-                    // scorer keep the sentinel here and reach the merge through the overflow list)
-                    SW_CUDA(h, sw_launch_topk_row(gc.st_compute, (const int32_t *)gc.d_wave_rows.p + (size_t)wave_row * n, (uint32_t)n, q,
-                                                  g.topk_k, gc.d_topk_keys.as<unsigned long long>()));
-                    h->launches++;
-                }
-                if (hits) {
-                    // the row's entries >= min_score join the list (flagged pairs come from the overflow list)
-                    SW_CUDA(h, sw_launch_hits_row(gc.st_compute, (const int32_t *)gc.d_wave_rows.p + (size_t)wave_row * n, (uint32_t)n, q, hl));
-                    h->launches++;
-                }
-                if (&gc == &h->gpus[0] && label_v < 0)
-                    std::snprintf(h->last_kernel, sizeof h->last_kernel, "%s", sw_wave_kernel_name(W.instance));
-            }
-        }
-        if (may_overflow) {
-            s32.mode = 2; s32.list_count = g.d_ovf_count.as<unsigned>(); s32.list = g.d_ovf_list.as<uint2>();
-            s32.list_cap = kOvfCap; s32.list_score = g.d_ovf_score.as<int32_t>();
-            if (h->wave32) {
-                // long entries (with the default scoring every entry is >= 6 400 x 6 400 nt) are scored
-                // by bands on many warps; the launch is list-driven, so nothing is read back here
-                SwWave32Launch W;
-                W.db = db; W.q = dq; W.sc = sc;
-                W.list_count = s32.list_count; W.list = s32.list; W.list_cap = kOvfCap; W.list_score = s32.list_score;
-                W.out = s32.out; W.out_stride = n; W.out_elems = (size_t)nq * n; W.out_mode = g.out_mode;
-                W.cols_stride = ((g.max_len + 31u) & ~31u) + 32u;
-                const size_t per_slot = (size_t)2 * W.cols_stride * 16;
-                W.nslots = (uint32_t)std::min<size_t>(64, std::max<size_t>(2, ((size_t)64 << 20) / per_slot));
-                W.bnd_elems = (size_t)W.nslots * 2 * W.cols_stride;
-                bool fresh = false;
-                if (gc.d_wave32_bnd.cap < W.bnd_elems * 16 || !gc.d_wave32_bnd.p) {
-                    SW_CUDA(h, cudaStreamSynchronize(gc.st_compute));
-                    SW_CUDA(h, gc.d_wave32_bnd.reserve(W.bnd_elems * 16));
-                    fresh = true;
-                }
-                const size_t state_bytes = (size_t)3 * SW_WAVE32_MAX_ENTRIES * sizeof(unsigned);
-                SW_CUDA(h, gc.d_wave32_state.reserve(state_bytes));
-                W.state = gc.d_wave32_state.as<unsigned>();
-                W.maxb = (h->q_max_len + SW_WAVE32_ROWS - 1) / SW_WAVE32_ROWS;
-                W.min_cells = h->wave32_min_cells;
-                if (!gc.wave32_bps) SW_CUDA(h, sw_wave32_occupancy(&gc.wave32_bps));
-                if (gc.wave32_bps < 1) return SW_ECUDA;
-                // one warp per scheduler: a larger grid lets the first (few hundred) claiming blocks pile
-                // up on a few SMs (measured: 16 blocks per SM = 2.3x slower for one 100 kb entry)
-                W.grid = gc.num_sms * std::min(gc.wave32_bps, 4);
-                W.dev_err = gc.d_err.as<unsigned>();
-                // 4 096 entries per launch (12 tag bits); a launch that finds no entry costs one
-                // atomic per block
-                W.entry_limit = kWave32Parts * SW_WAVE32_MAX_ENTRIES;
-                for (unsigned part = 0; part < kWave32Parts; ++part) {
-                    gc.wave32_epoch = gc.wave32_epoch % 255u + 1u;
-                    if (fresh || gc.wave32_epoch == 1u)      // stale tags must never match
-                        SW_CUDA(h, cudaMemsetAsync(gc.d_wave32_bnd.p, 0, gc.d_wave32_bnd.cap, gc.st_compute));
-                    fresh = false;
-                    W.bnd = gc.d_wave32_bnd.p; W.epoch = gc.wave32_epoch;
-                    W.entry_base = part * SW_WAVE32_MAX_ENTRIES;
-                    SW_CUDA(h, cudaMemsetAsync(gc.d_wave32_state.p, 0, state_bytes, gc.st_compute));
-                    W.counter = next_counter(gc);
-                    SW_CUDA(h, cudaMemsetAsync(W.counter, 0, sizeof(unsigned), gc.st_compute));
-                    SW_CUDA(h, sw_launch_wave32(gc.st_compute, W));
-                    h->launches++;
-                }
-                s32.wave32_min_cells = W.min_cells; s32.wave32_limit = W.entry_limit;
-            }
-            SW_CUDA(h, sw_launch_score32(gc.st_compute, s32));
-            h->launches++;
-            if (hits) {
-                SW_CUDA(h, sw_launch_hits_ovf(gc.st_compute, s32.list_count, s32.list, s32.list_score, kOvfCap, hl));
-                h->launches++;
-            }
-        }
-        if (topk) {
-            SW_CUDA(h, sw_launch_topk_merge(gc.st_compute, gc.d_topk_keys.as<unsigned long long>(), max_grid, nq, g.topk_k,
-                                            may_overflow ? g.d_ovf_count.as<unsigned>() : nullptr, g.d_ovf_list.as<uint2>(),
-                                            g.d_ovf_score.as<int32_t>(), kOvfCap, g.d_topk_out.as<unsigned long long>()));
+        const size_t state_bytes = (size_t)3 * SW_WAVE32_MAX_ENTRIES * sizeof(unsigned);
+        SW_CUDA(h, gc.d_wave32_state.reserve(state_bytes));
+        W.state = gc.d_wave32_state.as<unsigned>();
+        W.maxb = (h->q_max_len + SW_WAVE32_ROWS - 1) / SW_WAVE32_ROWS;
+        W.min_cells = h->wave32_min_cells;
+        if (!gc.wave32_bps) SW_CUDA(h, sw_wave32_occupancy(&gc.wave32_bps));
+        if (gc.wave32_bps < 1) return SW_ECUDA;
+        // one warp per scheduler: a larger grid lets the first (few hundred) claiming blocks pile
+        // up on a few SMs (measured: 16 blocks per SM = 2.3x slower for one 100 kb entry)
+        W.grid = gc.num_sms * std::min(gc.wave32_bps, 4);
+        W.dev_err = gc.d_err.as<unsigned>();
+        // 4 096 entries per launch (12 tag bits); a launch that finds no entry costs one
+        // atomic per block
+        W.entry_limit = kWave32Parts * SW_WAVE32_MAX_ENTRIES;
+        for (unsigned part = 0; part < kWave32Parts; ++part) {
+            gc.wave32_epoch = gc.wave32_epoch % 255u + 1u;
+            if (fresh || gc.wave32_epoch == 1u)      // stale tags must never match
+                SW_CUDA(h, cudaMemsetAsync(gc.d_wave32_bnd.p, 0, gc.d_wave32_bnd.cap, gc.st_compute));
+            fresh = false;
+            W.bnd = gc.d_wave32_bnd.p; W.epoch = gc.wave32_epoch;
+            W.entry_base = part * SW_WAVE32_MAX_ENTRIES;
+            SW_CUDA(h, cudaMemsetAsync(gc.d_wave32_state.p, 0, state_bytes, gc.st_compute));
+            W.counter = next_counter(gc);
+            SW_CUDA(h, cudaMemsetAsync(W.counter, 0, sizeof(unsigned), gc.st_compute));
+            SW_CUDA(h, sw_launch_wave32(gc.st_compute, W));
             h->launches++;
         }
-    } else {
-        s32.mode = 0; s32.q0 = 0; s32.q1 = nq;
-        SW_CUDA(h, sw_launch_score32(gc.st_compute, s32));
+        s32.wave32_min_cells = W.min_cells; s32.wave32_limit = W.entry_limit;
+    }
+    SW_CUDA(h, sw_launch_score32(gc.st_compute, s32));
+    h->launches++;
+    if (j.hits) {
+        SW_CUDA(h, sw_launch_hits_ovf(gc.st_compute, s32.list_count, s32.list, s32.list_score, kOvfCap, j.hl));
         h->launches++;
     }
-    if (g.chunks.empty()) {
-        QueryChunk qc{0, nq, pool_event(h, g, nev++, &rc)};
-        if (rc != SW_OK) return rc;
-        SW_CUDA(h, cudaEventRecord(qc.done, gc.st_compute));
-        g.chunks.push_back(qc);
-    }
-    SW_CUDA(h, cudaEventRecord(g.ev_stop, gc.st_compute));
-    g.ev_stop_deferred = false;
     return SW_OK;
+}
+
+// End of a scoring on the compute stream: one chunk event for all queries unless the query chunks
+// recorded their own, then ev_stop.
+int finish_scoring(sw_handle *h, ScoreJob &j)
+{
+    if (j.g.chunks.empty()) {
+        SW_TRY(push_chunk(h, j.gc, j.g, 0, j.nq));
+    }
+    SW_CUDA(h, cudaEventRecord(j.g.ev_stop, j.gc.st_compute));
+    j.g.ev_stop_deferred = false;
+    return SW_OK;
+}
+
+// Scores the batch in slot g against the queries on one GPU: outputs, query routing, launch plan,
+// last_kernel, then the launches.
+int score_gpu(sw_handle *h, GpuCtx &gc, Slot &g, const Batch &bt)
+{
+    if (&gc == &h->gpus[0]) h->last_parts = 1;
+    SW_CUDA(h, cudaSetDevice(gc.dev));
+    ScoreJob j{gc, g, bt, bt.nq, g.s1 - g.s0, bt.out_mode == SW_OUT_TOPK, bt.out_mode == SW_OUT_HITS};
+    g.chunks.clear();
+    g.scored = true;
+    g.ovf_used = false;
+    if (j.n == 0 || j.nq == 0) return SW_OK;
+    SW_TRY(reserve_outputs(h, j));
+    SW_CUDA(h, cudaEventRecord(g.ev_start, gc.st_compute));
+    if (g.npairs == 0) return finish_scoring(h, j);
+
+    j.sc = scoring_of(h);
+    j.db = dev_db(g);
+    j.dq = dev_queries(h, gc);
+    // Value range: the packed 16-bit kernel is always used; when match * min(m, n) could exceed
+    // the 16-bit range it flags the (rare) pairs whose running maximum got near 32767: they go to
+    // the overflow list and the 32-bit kernel recomputes exactly those.
+    const uint64_t smax = (uint64_t)j.sc.match * std::min<uint64_t>(h->q_max_len, g.max_len);
+    j.may_overflow = !j.sc.limit && (smax + (uint64_t)j.sc.match >= 32000ull);
+    SW_CUDA(h, gc.d_counters.reserve(kMaxCounters * sizeof(unsigned)));
+    route_queries(h, gc, g, j.wave_q, j.strip_q);
+
+    SwStripLaunch &base = j.base;
+    base.db = j.db; base.q = j.dq; base.sc = j.sc;
+    base.out = (j.topk || j.hits) ? nullptr : g.d_out.p; base.out_stride = j.n; base.out_elems = j.hits ? bt.hits_max : (size_t)j.nq * j.n;
+    base.out_mode = bt.out_mode;
+    base.hits = j.hl;
+    base.dev_err = gc.d_err.as<unsigned>();
+    if (j.may_overflow) {
+        SW_CUDA(h, g.d_ovf_count.reserve(sizeof(unsigned)));
+        SW_CUDA(h, g.d_ovf_list.reserve((size_t)kOvfCap * sizeof(uint2)));
+        SW_CUDA(h, g.d_ovf_score.reserve((size_t)kOvfCap * sizeof(int32_t)));
+        SW_CUDA(h, cudaMemsetAsync(g.d_ovf_count.p, 0, sizeof(unsigned), gc.st_compute));
+        base.ovf_count = g.d_ovf_count.as<unsigned>(); base.ovf_list = g.d_ovf_list.as<uint2>(); base.ovf_cap = kOvfCap;
+        g.ovf_used = true;
+    }
+    StripPlan p;
+    if (!h->force32 && !j.strip_q.empty()) SW_TRY(plan_strip(h, j, p));
+    if (&gc == &h->gpus[0]) set_kernel_label(h, j, p);
+
+    const bool use32 = p.launches.empty() && j.wave_q.empty();        // forced 32-bit scorer
+    if (use32 && (j.topk || j.hits)) return SW_EINVAL;   // it has no top-k epilogue and no hit list (hits: refused at submit)
+    SwScore32Launch s32;
+    SW_TRY(reserve_scratch(h, j, p, use32, s32));
+    if (use32) {
+        s32.mode = 0; s32.q0 = 0; s32.q1 = j.nq;
+        SW_CUDA(h, sw_launch_score32(gc.st_compute, s32));
+        h->launches++;
+        return finish_scoring(h, j);
+    }
+    SW_TRY(enqueue_strip(h, j, p));
+    if (!j.wave_q.empty()) SW_TRY(enqueue_wave(h, j));
+    if (j.may_overflow) SW_TRY(enqueue_overflow(h, j, s32));
+    if (j.topk) {
+        SW_CUDA(h, sw_launch_topk_merge(gc.st_compute, gc.d_topk_keys.as<unsigned long long>(), p.max_grid, j.nq, bt.topk_k,
+                                        j.may_overflow ? g.d_ovf_count.as<unsigned>() : nullptr, g.d_ovf_list.as<uint2>(),
+                                        g.d_ovf_score.as<int32_t>(), kOvfCap, g.d_topk_out.as<unsigned long long>()));
+        h->launches++;
+    }
+    return finish_scoring(h, j);
 }
 
 // waits for an event with a deadline; forever = no deadline
@@ -1495,6 +1548,161 @@ constexpr int32_t kSmallSentinel = INT32_MIN;
 // what a fetch delivers
 enum FetchKind { FETCH_I32, FETCH_I16, FETCH_TOPK };
 
+// Waits, until t_end (forever: no deadline), for the last chunk event of slot si on every GPU that scored a part of it.
+int wait_slot(sw_handle *h, int si, const std::chrono::steady_clock::time_point &t_end, bool forever)
+{
+    for (auto &g : h->gpus) {
+        const Slot &b = g.slot[si];
+        if (!b.scored || b.chunks.empty()) continue;
+        SW_CUDA(h, cudaSetDevice(g.dev));
+        SW_TRY(wait_event(h, b.chunks.back().done, t_end, forever));
+    }
+    return SW_OK;
+}
+
+// Drains every GPU's copy stream; longest and shortest kernel time (ev_start .. ev_stop) of slot si over the
+// GPUs that scored a part of it.
+int slot_kernel_ms(sw_handle *h, int si, double *ms_max, double *ms_min)
+{
+    *ms_max = 0.0; *ms_min = 1e300;
+    for (auto &g : h->gpus) {
+        const Slot &b = g.slot[si];
+        SW_CUDA(h, cudaSetDevice(g.dev));
+        SW_CUDA(h, cudaStreamSynchronize(g.st_copy));
+        if (!b.scored || b.chunks.empty()) continue;
+        SW_CUDA(h, cudaEventSynchronize(b.ev_stop));
+        float ms = 0.f;
+        SW_CUDA(h, cudaEventElapsedTime(&ms, b.ev_start, b.ev_stop));
+        *ms_max = std::max(*ms_max, (double)ms);
+        *ms_min = std::min(*ms_min, (double)ms);
+    }
+    return SW_OK;
+}
+
+// Small (latency) path: the scores are already in mapped host memory.
+int fetch_small(sw_handle *h, int si, void *scores, const std::chrono::steady_clock::time_point &t_fetch0,
+                const std::chrono::steady_clock::time_point &t_end, bool forever)
+{
+    const Batch &bt = h->batch[si];
+    const size_t nq = (size_t)bt.nq;
+    GpuCtx &g = h->gpus[0];
+    Slot &b = g.slot[si];
+    // Completion is read from mapped host memory.  Default: every result word replaces the
+    // sentinel the host wrote before the launch (4-byte stores arrive whole), so the kernel needs
+    // no system-scope fence and no flag -- its fence.sys alone was a quarter of the warp time of
+    // the config-2 kernel -- and the host sees the last score one PCIe write after it was stored.
+    // Otherwise: the flag the kernel's last block writes after its fence.
+    volatile unsigned *flag = (volatile unsigned *)b.h_small_flag.p;
+    const volatile int32_t *res = (const volatile int32_t *)b.h_small_out.p;
+    const size_t nres = nq * bt.ns;
+    size_t seen = 0;                                           // results [0, seen) have arrived
+    unsigned spins = 0;
+    auto complete = [&]() -> bool {
+        if (b.small_by_flag) return *flag == b.small_seq;
+        while (seen < nres && res[seen] != kSmallSentinel) ++seen;
+        return seen == nres;
+    };
+    while (!complete()) {
+        if ((++spins & 0x3FF) == 0) {
+            if (!forever && std::chrono::steady_clock::now() >= t_end) return SW_ETIMEOUT;
+            cudaError_t qe = cudaStreamQuery(g.st_compute);          // a failed launch would never finish the buffer
+            if (qe != cudaSuccess && qe != cudaErrorNotReady) { h->last_cuda.store((int)qe); return SW_ECUDA; }
+            if (qe == cudaSuccess && !complete()) { h->last_cuda.store((int)cudaErrorUnknown); return SW_ECUDA; }
+        }
+    }
+    std::atomic_thread_fence(std::memory_order_acquire);
+    const auto tr3 = std::chrono::steady_clock::now();
+    std::memcpy(scores, b.h_small_out.p, nq * bt.ns * sizeof(int32_t));
+    if (h->trace_small) {
+        h->tr_wait += std::chrono::duration<double, std::micro>(tr3 - t_fetch0).count();
+        h->tr_copy += std::chrono::duration<double, std::micro>(std::chrono::steady_clock::now() - tr3).count();
+    }
+    float ms = 0.f;
+    if (b.small_timed) {
+        SW_CUDA(h, cudaEventSynchronize(b.ev_stop));
+        SW_CUDA(h, cudaEventElapsedTime(&ms, b.ev_start, b.ev_stop));
+    }
+    finish_timing(h, si, t_fetch0, std::chrono::steady_clock::now(), ms, ms);
+#ifdef SW_BOUNDS_CHECK
+    if (device_error_bits(h)) return SW_EDEVICE;
+#endif
+    return SW_OK;
+}
+
+// Scores that left the 16-bit range (rare): list length check, rescan of an int32 matrix whose list
+// overflowed, side list of sw_fetch_overflow for int16.
+int fetch_overflow_list(sw_handle *h, int si, FetchKind kind, void *scores)
+{
+    Batch &bt = h->batch[si];
+    const size_t nq = (size_t)bt.nq;
+    const size_t esz = kind == FETCH_I16 ? sizeof(int16_t) : sizeof(int32_t);
+    for (auto &g : h->gpus) {
+        Slot &b = g.slot[si];
+        if (!b.ovf_used || b.s1 == b.s0) continue;
+        SW_CUDA(h, cudaSetDevice(g.dev));
+        unsigned cnt = 0;
+        SW_CUDA(h, cudaMemcpy(&cnt, b.d_ovf_count.p, sizeof cnt, cudaMemcpyDeviceToHost));
+        if (cnt == 0) continue;
+        const size_t n = b.s1 - b.s0;
+        if (cnt > kOvfCap) {
+            if (kind != FETCH_I32) return SW_ERANGE;
+            // more flagged pairs than the list holds: rescan the matrix for sentinels (32-bit matrix only)
+            SwScore32Launch s32;
+            s32.db = dev_db(b); s32.q = dev_queries(h, g); s32.sc = scoring_of(h); s32.out = b.d_out.p; s32.out_stride = n;
+            s32.out_mode = SW_OUT_I32; s32.scratch = g.d_scratch32.as<int32_t>();
+            s32.max_cols = std::max<uint32_t>(1, std::min<uint32_t>(h->q_max_len, b.max_len));
+            s32.threads_total = (int)(g.d_scratch32.cap / ((size_t)2 * s32.max_cols * sizeof(int32_t)) / 128 * 128);
+            s32.mode = 1; s32.q0 = 0; s32.q1 = (int)nq;
+            SW_CUDA(h, sw_launch_score32(g.st_compute, s32));
+            h->launches++;
+            SW_CUDA(h, cudaStreamSynchronize(g.st_compute));
+            SW_CUDA(h, cudaMemcpy2D((char *)scores + b.s0 * esz, bt.ns * esz, b.d_out.p, n * esz, n * esz, nq, cudaMemcpyDeviceToHost));
+            continue;
+        }
+        if (kind == FETCH_I16) {
+            SW_CUDA(h, b.h_ovf.reserve((size_t)cnt * (sizeof(uint2) + sizeof(int32_t))));
+            uint2 *hl = (uint2 *)b.h_ovf.p;
+            int32_t *hs = (int32_t *)(hl + cnt);
+            SW_CUDA(h, cudaMemcpy(hl, b.d_ovf_list.p, (size_t)cnt * sizeof(uint2), cudaMemcpyDeviceToHost));
+            SW_CUDA(h, cudaMemcpy(hs, b.d_ovf_score.p, (size_t)cnt * sizeof(int32_t), cudaMemcpyDeviceToHost));
+            for (unsigned i = 0; i < cnt; ++i) {
+                if (hs[i] <= 32767) continue;
+                bt.ovf_index.push_back((uint64_t)hl[i].x * bt.ns + b.s0 + hl[i].y);
+                bt.ovf_score.push_back(hs[i]);
+            }
+        }
+    }
+    return SW_OK;
+}
+
+// Top-k: merges the per-GPU lists (and zero-length subjects, which score 0) on the host.
+void merge_topk(sw_handle *h, int si, int32_t *os, uint64_t *index)
+{
+    const Batch &bt = h->batch[si];
+    const int K = bt.topk_k;
+    std::vector<std::pair<int64_t, uint64_t>> cand;      // (-score, index): ascending sort = best first
+    for (size_t q = 0; q < (size_t)bt.nq; ++q) {
+        cand.clear();
+        for (auto &g : h->gpus) {
+            Slot &b = g.slot[si];
+            if (b.s1 == b.s0) continue;
+            if (!b.chunks.empty() && b.h_topk.p && b.npairs) {
+                const unsigned long long *keys = (const unsigned long long *)b.h_topk.p + q * K;
+                for (int j = 0; j < K; ++j) {
+                    if (keys[j] == 0) continue;
+                    cand.emplace_back(-(int64_t)(keys[j] >> 32), b.s0 + (uint64_t)(uint32_t)~(uint32_t)(keys[j] & 0xFFFFFFFFu));
+                }
+            }
+            for (uint32_t e : b.empties) cand.emplace_back(0, b.s0 + e);     // zero-length subjects score 0
+        }
+        std::sort(cand.begin(), cand.end());
+        for (int j = 0; j < K; ++j) {
+            if ((size_t)j < cand.size()) { os[q * K + j] = (int32_t)(-cand[j].first); index[q * K + j] = cand[j].second; }
+            else { os[q * K + j] = -1; index[q * K + j] = ~0ull; }
+        }
+    }
+}
+
 int fetch_slot(sw_handle *h, int si, FetchKind kind, void *scores, uint64_t *index, size_t cap, int timeout_ms)
 {
     Batch &bt = h->batch[si];
@@ -1502,67 +1710,13 @@ int fetch_slot(sw_handle *h, int si, FetchKind kind, void *scores, uint64_t *ind
     const bool forever = timeout_ms < 0;
     const auto t_fetch0 = std::chrono::steady_clock::now();
     const auto t_end = t_fetch0 + std::chrono::milliseconds(forever ? 0 : timeout_ms);
-    if (bt.hits_min > 0) return SW_ESTATE;                  // a hits batch has no matrix / top-k lists
-    if (kind == FETCH_TOPK) {
-        if (bt.topk_k <= 0) return SW_ESTATE;
-        if (cap < nq * (size_t)bt.topk_k) return SW_ECAPACITY;
-    } else {
-        if (bt.topk_k > 0) return SW_ESTATE;
-        if ((kind == FETCH_I16) != (bt.out_mode == SW_OUT_I16)) return SW_ESTATE;
-        if (cap < nq * bt.ns) return SW_ECAPACITY;
-    }
-
-    // ---- small (latency) path: scores are already in mapped host memory ----------------------
-    if (bt.small) {
-        GpuCtx &g = h->gpus[0];
-        Slot &b = g.slot[si];
-        // Completion is read from mapped host memory.  Default: every result word replaces the
-        // sentinel the host wrote before the launch (4-byte stores arrive whole), so the kernel needs
-        // no system-scope fence and no flag -- its fence.sys alone was a quarter of the warp time of
-        // the config-2 kernel -- and the host sees the last score one PCIe write after it was stored.
-        // Otherwise: the flag the kernel's last block writes after its fence.
-        volatile unsigned *flag = (volatile unsigned *)b.h_small_flag.p;
-        const volatile int32_t *res = (const volatile int32_t *)b.h_small_out.p;
-        const size_t nres = nq * bt.ns;
-        size_t seen = 0;                                           // results [0, seen) have arrived
-        unsigned spins = 0;
-        auto complete = [&]() -> bool {
-            if (b.small_by_flag) return *flag == b.small_seq;
-            while (seen < nres && res[seen] != kSmallSentinel) ++seen;
-            return seen == nres;
-        };
-        while (!complete()) {
-            if ((++spins & 0x3FF) == 0) {
-                if (!forever && std::chrono::steady_clock::now() >= t_end) return SW_ETIMEOUT;
-                cudaError_t qe = cudaStreamQuery(g.st_compute);          // a failed launch would never finish the buffer
-                if (qe != cudaSuccess && qe != cudaErrorNotReady) { h->last_cuda.store((int)qe); return SW_ECUDA; }
-                if (qe == cudaSuccess && !complete()) { h->last_cuda.store((int)cudaErrorUnknown); return SW_ECUDA; }
-            }
-        }
-        std::atomic_thread_fence(std::memory_order_acquire);
-        const auto tr3 = std::chrono::steady_clock::now();
-        std::memcpy(scores, b.h_small_out.p, nq * bt.ns * sizeof(int32_t));
-        if (h->trace_small) {
-            h->tr_wait += std::chrono::duration<double, std::micro>(tr3 - t_fetch0).count();
-            h->tr_copy += std::chrono::duration<double, std::micro>(std::chrono::steady_clock::now() - tr3).count();
-        }
-        float ms = 0.f;
-        if (b.small_timed) {
-            SW_CUDA(h, cudaEventSynchronize(b.ev_stop));
-            SW_CUDA(h, cudaEventElapsedTime(&ms, b.ev_start, b.ev_stop));
-        }
-        finish_timing(h, si, t_fetch0, std::chrono::steady_clock::now(), ms, ms);
-#ifdef SW_BOUNDS_CHECK
-        if (device_error_bits(h)) return SW_EDEVICE;
-#endif
-        return SW_OK;
-    }
+    // (a hits batch has no matrix / top-k lists)
+    if (bt.out_mode != (kind == FETCH_TOPK ? SW_OUT_TOPK : kind == FETCH_I16 ? SW_OUT_I16 : SW_OUT_I32)) return SW_ESTATE;
+    if (cap < nq * (kind == FETCH_TOPK ? (size_t)bt.topk_k : bt.ns)) return SW_ECAPACITY;
+    if (bt.small) return fetch_small(h, si, scores, t_fetch0, t_end, forever);
 
     const size_t esz = kind == FETCH_I16 ? sizeof(int16_t) : sizeof(int32_t);
-    bool any_ovf = false;
-    for (auto &g : h->gpus) any_ovf |= g.slot[si].ovf_used && g.slot[si].scored && g.slot[si].s1 > g.slot[si].s0;
     bt.ovf_index.clear(); bt.ovf_score.clear();
-
     if (kind != FETCH_TOPK) {
         size_t maxchunks = 0;
         for (auto &g : h->gpus) maxchunks = std::max(maxchunks, g.slot[si].chunks.size());
@@ -1586,98 +1740,21 @@ int fetch_slot(sw_handle *h, int si, FetchKind kind, void *scores, uint64_t *ind
             }
         }
     } else {
+        SW_TRY(wait_slot(h, si, t_end, forever));
         for (auto &g : h->gpus) {
             Slot &b = g.slot[si];
-            if (b.s1 == b.s0 || nq == 0 || b.chunks.empty()) continue;
+            if (!b.scored || b.chunks.empty()) continue;
             SW_CUDA(h, cudaSetDevice(g.dev));
-            int rc = wait_event(h, b.chunks.back().done, t_end, forever);
-            if (rc != SW_OK) return rc;
             const size_t bytes = nq * (size_t)bt.topk_k * sizeof(unsigned long long);
             SW_CUDA(h, b.h_topk.reserve(bytes));
             SW_CUDA(h, cudaMemcpyAsync(b.h_topk.p, b.d_topk_out.p, bytes, cudaMemcpyDeviceToHost, g.st_copy));
         }
     }
     const auto t_fetch1 = std::chrono::steady_clock::now();
-    double ms_max = 0.0, ms_min = 1e300;
-    for (auto &g : h->gpus) {
-        Slot &b = g.slot[si];
-        SW_CUDA(h, cudaSetDevice(g.dev));
-        SW_CUDA(h, cudaStreamSynchronize(g.st_copy));
-        if (b.scored && (b.s1 > b.s0) && nq) {
-            SW_CUDA(h, cudaEventSynchronize(b.ev_stop));
-            float ms = 0.f;
-            SW_CUDA(h, cudaEventElapsedTime(&ms, b.ev_start, b.ev_stop));
-            ms_max = std::max(ms_max, (double)ms);
-            ms_min = std::min(ms_min, (double)ms);
-        }
-    }
-
-    // ---- scores that left the 16-bit range (rare): list length check, side list for int16 -----
-    if (any_ovf) {
-        for (auto &g : h->gpus) {
-            Slot &b = g.slot[si];
-            if (!b.ovf_used || b.s1 == b.s0) continue;
-            SW_CUDA(h, cudaSetDevice(g.dev));
-            unsigned cnt = 0;
-            SW_CUDA(h, cudaMemcpy(&cnt, b.d_ovf_count.p, sizeof cnt, cudaMemcpyDeviceToHost));
-            if (cnt == 0) continue;
-            const size_t n = b.s1 - b.s0;
-            if (cnt > kOvfCap) {
-                if (kind != FETCH_I32) return SW_ERANGE;
-                // more flagged pairs than the list holds: rescan the matrix for sentinels (32-bit matrix only)
-                SwScore32Launch s32;
-                s32.db = dev_db(b); s32.q = dev_queries(h, g); s32.sc = scoring_of(h); s32.out = b.d_out.p; s32.out_stride = n;
-                s32.out_mode = SW_OUT_I32; s32.scratch = g.d_scratch32.as<int32_t>();
-                s32.max_cols = std::max<uint32_t>(1, std::min<uint32_t>(h->q_max_len, b.max_len));
-                s32.threads_total = (int)(g.d_scratch32.cap / ((size_t)2 * s32.max_cols * sizeof(int32_t)) / 128 * 128);
-                s32.mode = 1; s32.q0 = 0; s32.q1 = (int)nq;
-                SW_CUDA(h, sw_launch_score32(g.st_compute, s32));
-                h->launches++;
-                SW_CUDA(h, cudaStreamSynchronize(g.st_compute));
-                SW_CUDA(h, cudaMemcpy2D((char *)scores + b.s0 * esz, bt.ns * esz, b.d_out.p, n * esz, n * esz, nq, cudaMemcpyDeviceToHost));
-                continue;
-            }
-            if (kind == FETCH_I16) {
-                SW_CUDA(h, b.h_ovf.reserve((size_t)cnt * (sizeof(uint2) + sizeof(int32_t))));
-                uint2 *hl = (uint2 *)b.h_ovf.p;
-                int32_t *hs = (int32_t *)(hl + cnt);
-                SW_CUDA(h, cudaMemcpy(hl, b.d_ovf_list.p, (size_t)cnt * sizeof(uint2), cudaMemcpyDeviceToHost));
-                SW_CUDA(h, cudaMemcpy(hs, b.d_ovf_score.p, (size_t)cnt * sizeof(int32_t), cudaMemcpyDeviceToHost));
-                for (unsigned i = 0; i < cnt; ++i) {
-                    if (hs[i] <= 32767) continue;
-                    bt.ovf_index.push_back((uint64_t)hl[i].x * bt.ns + b.s0 + hl[i].y);
-                    bt.ovf_score.push_back(hs[i]);
-                }
-            }
-        }
-    }
-
-    // ---- top-k: merge the per-GPU lists on the host -------------------------------------------
-    if (kind == FETCH_TOPK) {
-        const int K = bt.topk_k;
-        int32_t *os = (int32_t *)scores;
-        std::vector<std::pair<int64_t, uint64_t>> cand;      // (-score, index): ascending sort = best first
-        for (size_t q = 0; q < nq; ++q) {
-            cand.clear();
-            for (auto &g : h->gpus) {
-                Slot &b = g.slot[si];
-                if (b.s1 == b.s0) continue;
-                if (!b.chunks.empty() && b.h_topk.p && b.npairs) {
-                    const unsigned long long *keys = (const unsigned long long *)b.h_topk.p + q * K;
-                    for (int j = 0; j < K; ++j) {
-                        if (keys[j] == 0) continue;
-                        cand.emplace_back(-(int64_t)(keys[j] >> 32), b.s0 + (uint64_t)(uint32_t)~(uint32_t)(keys[j] & 0xFFFFFFFFu));
-                    }
-                }
-                for (uint32_t e : b.empties) cand.emplace_back(0, b.s0 + e);     // zero-length subjects score 0
-            }
-            std::sort(cand.begin(), cand.end());
-            for (int j = 0; j < K; ++j) {
-                if ((size_t)j < cand.size()) { os[q * K + j] = (int32_t)(-cand[j].first); index[q * K + j] = cand[j].second; }
-                else { os[q * K + j] = -1; index[q * K + j] = ~0ull; }
-            }
-        }
-    }
+    double ms_max = 0.0, ms_min = 0.0;
+    SW_TRY(slot_kernel_ms(h, si, &ms_max, &ms_min));
+    SW_TRY(fetch_overflow_list(h, si, kind, scores));
+    if (kind == FETCH_TOPK) merge_topk(h, si, (int32_t *)scores, index);
     finish_timing(h, si, t_fetch0, t_fetch1, ms_max, ms_min);
     if (device_error_bits(h)) return SW_EDEVICE;
     return SW_OK;
@@ -1690,21 +1767,20 @@ int fetch_slot(sw_handle *h, int si, FetchKind kind, void *scores, uint64_t *ind
 int fetch_hits_slot(sw_handle *h, int si, uint32_t *row, uint64_t *index, int32_t *score, size_t cap, size_t *count, int timeout_ms)
 {
     Batch &bt = h->batch[si];
-    if (bt.hits_min <= 0) return SW_ESTATE;
+    if (bt.out_mode != SW_OUT_HITS) return SW_ESTATE;
     const bool forever = timeout_ms < 0;
     const auto t_fetch0 = std::chrono::steady_clock::now();
     const auto t_end = t_fetch0 + std::chrono::milliseconds(forever ? 0 : timeout_ms);
     if (!bt.hits_staged) {
         const size_t ng = h->gpus.size();
+        SW_TRY(wait_slot(h, si, t_end, forever));
         std::vector<unsigned long long> cnt(ng, 0);
         bool too_many = false;
         for (size_t gi = 0; gi < ng; ++gi) {
             GpuCtx &g = h->gpus[gi];
             Slot &b = g.slot[si];
-            if (b.s1 == b.s0 || bt.nq == 0 || b.chunks.empty()) continue;
+            if (!b.scored || b.chunks.empty()) continue;
             SW_CUDA(h, cudaSetDevice(g.dev));
-            int rc = wait_event(h, b.chunks.back().done, t_end, forever);
-            if (rc != SW_OK) return rc;
             SW_CUDA(h, cudaMemcpy(&cnt[gi], b.d_hits_count.p, sizeof(unsigned long long), cudaMemcpyDeviceToHost));
             too_many |= cnt[gi] > bt.hits_max;
             if (b.ovf_used) {
@@ -1728,10 +1804,8 @@ int fetch_hits_slot(sw_handle *h, int si, uint32_t *row, uint64_t *index, int32_
             const int end_bit = std::max(1, b.hits_shift + row_bits);          // only the key bits in use
             // sized for max_hits (a count never exceeds it here): a buffer that grows would be freed, and cudaFree
             // waits for the whole device -- the next batch's kernels included
-            if (g.d_hits_key2.cap < bt.hits_max * sizeof(unsigned long long) || g.d_hits_score2.cap < bt.hits_max * sizeof(int32_t)) {
-                SW_CUDA(h, g.d_hits_key2.reserve(bt.hits_max * sizeof(unsigned long long)));
-                SW_CUDA(h, g.d_hits_score2.reserve(bt.hits_max * sizeof(int32_t)));
-            }
+            SW_CUDA(h, g.d_hits_key2.reserve(bt.hits_max * sizeof(unsigned long long)));
+            SW_CUDA(h, g.d_hits_score2.reserve(bt.hits_max * sizeof(int32_t)));
             size_t tmp = 0;
             SW_CUDA(h, cub::DeviceRadixSort::SortPairs(nullptr, tmp, b.d_hits_key.as<unsigned long long>(), g.d_hits_key2.as<unsigned long long>(),
                                                       b.d_hits_score.as<int32_t>(), g.d_hits_score2.as<int32_t>(), (int)bt.hits_max, 0, 64, g.st_copy));
@@ -1745,22 +1819,9 @@ int fetch_hits_slot(sw_handle *h, int si, uint32_t *row, uint64_t *index, int32_
             SW_CUDA(h, cudaMemcpyAsync((unsigned long long *)b.h_hits.p + c, g.d_hits_score2.p, (size_t)c * sizeof(int32_t),
                                        cudaMemcpyDeviceToHost, g.st_copy));
         }
-        double ms_max = 0.0, ms_min = 1e300;
-        size_t total = 0;
-        for (size_t gi = 0; gi < ng; ++gi) {
-            GpuCtx &g = h->gpus[gi];
-            Slot &b = g.slot[si];
-            SW_CUDA(h, cudaSetDevice(g.dev));
-            SW_CUDA(h, cudaStreamSynchronize(g.st_copy));
-            total += cnt[gi];
-            if (b.scored && b.s1 > b.s0 && bt.nq) {
-                SW_CUDA(h, cudaEventSynchronize(b.ev_stop));
-                float ms = 0.f;
-                SW_CUDA(h, cudaEventElapsedTime(&ms, b.ev_start, b.ev_stop));
-                ms_max = std::max(ms_max, (double)ms);
-                ms_min = std::min(ms_min, (double)ms);
-            }
-        }
+        double ms_max = 0.0, ms_min = 0.0;
+        SW_TRY(slot_kernel_ms(h, si, &ms_max, &ms_min));
+        const size_t total = *count;
         bt.hits_row.resize(total); bt.hits_index.resize(total); bt.hits_score.resize(total);
         std::vector<size_t> cur(ng, 0);
         size_t o = 0;
@@ -1831,6 +1892,14 @@ int load_batch(sw_handle *h, int si, const uint8_t *packed, const uint32_t *len,
     return SW_OK;
 }
 
+// The output of a scoring submitted now: top-k and hit list replace the matrix.
+void take_output_settings(const sw_handle *h, Batch &bt)
+{
+    bt.out_mode = h->topk_k > 0 ? SW_OUT_TOPK : h->hits_min > 0 ? SW_OUT_HITS : h->out_mode;
+    bt.topk_k = h->topk_k;
+    bt.hits_min = h->hits_min; bt.hits_max = h->hits_max; bt.hits_staged = false;
+}
+
 int score_batch_slot(sw_handle *h, int si)
 {
     const auto t_enq0 = std::chrono::steady_clock::now();
@@ -1839,19 +1908,17 @@ int score_batch_slot(sw_handle *h, int si)
     for (auto &g : h->gpus) db_len += g.slot[si].sum_len;
     bt.cells = db_len * h->q_sum_len;
     bt.nq = (int)h->q_len.size();
-    bt.out_mode = h->out_mode;
-    bt.topk_k = h->topk_k;
-    bt.hits_min = h->hits_min; bt.hits_max = h->hits_max; bt.hits_staged = false;
+    take_output_settings(h, bt);
     h->last_cells = bt.cells;
     const size_t ng = h->gpus.size();
     std::vector<int> rcs(ng, SW_OK);
     if (ng == 1) {
-        rcs[0] = score_gpu(h, h->gpus[0], h->gpus[0].slot[si]);
+        rcs[0] = score_gpu(h, h->gpus[0], h->gpus[0].slot[si], bt);
     } else {
         // one host worker per GPU: launch plans, allocations and (first call) autotune run concurrently
         std::vector<std::thread> workers;
         for (size_t gi = 0; gi < ng; ++gi)
-            workers.emplace_back([&, gi]() { rcs[gi] = score_gpu(h, h->gpus[gi], h->gpus[gi].slot[si]); });
+            workers.emplace_back([&, gi]() { rcs[gi] = score_gpu(h, h->gpus[gi], h->gpus[gi].slot[si], bt); });
         for (auto &w : workers) w.join();
     }
     for (int rc : rcs) {
@@ -1932,11 +1999,12 @@ int small_submit(sw_handle *h, int si, const uint8_t *packed, const uint32_t *le
     bt.ns = ns; bt.loaded = true; bt.scored = true; bt.small = true;
     bt.have_ids = ids != nullptr;
     if (ids) bt.ids.assign(ids, ids + ns); else bt.ids.clear();
-    bt.nq = nq; bt.out_mode = SW_OUT_I32; bt.topk_k = 0; bt.hits_min = 0; bt.hits_staged = false;
+    bt.nq = nq;
+    take_output_settings(h, bt);                     // the int32 matrix (checked above)
     bt.cells = sum * h->q_sum_len;
     h->last_cells = bt.cells;
     for (auto &gg : h->gpus) { gg.slot[si].s0 = 0; gg.slot[si].s1 = 0; gg.slot[si].chunks.clear(); gg.slot[si].ovf_used = false; }
-    g.s0 = 0; g.s1 = ns; g.is_small = true; g.max_len = maxlen; g.sum_len = sum; g.out_mode = SW_OUT_I32; g.topk_k = 0;
+    g.s0 = 0; g.s1 = ns; g.is_small = true; g.max_len = maxlen; g.sum_len = sum;
 
     // ---- staging layout: [pair descriptors (32 bytes each) | raw bases]
     const size_t ntiles = (np_max + 31) / 32;
@@ -1997,13 +2065,13 @@ int small_submit(sw_handle *h, int si, const uint8_t *packed, const uint32_t *le
     L.dev_err = gc.d_err.as<unsigned>();
     const int P = v->R * v->G;
     const int need_passes = (int)((h->q_max_len + P - 1) / P);
-    const size_t pass_bytes = sw_strip_smem_bytes(vidx, 1);
-    L.chunk_passes = std::max(1, std::min(need_passes, std::max<int>(1, (int)((48 * 1024) / pass_bytes))));
-    const int ppb = v->block_threads / v->G;
-    const size_t items = ((np + ppb - 1) / ppb) * (size_t)nq;
+    L.chunk_passes = chunk_passes_for(vidx, need_passes);
+    // (not strip_setup: a static schedule on at most 4 blocks per SM, with no occupancy query on this path)
+    const size_t items = (size_t)pair_blocks(v, np) * (size_t)nq;
     L.grid = (int)std::min<size_t>(std::max<size_t>(items, 1), (size_t)gc.num_sms * 4);
     if (need_passes > 1) {
-        const size_t per_block = (size_t)maxlen * ppb * sizeof(uint2);
+        const size_t per_block = (size_t)maxlen * (v->block_threads / v->G) * sizeof(uint2);
+        // (no drain, unlike grow_shared: no driver calls to spare here, and the cudaFree of a smaller buffer waits for the device)
         SW_CUDA(h, gc.d_bnd.reserve((size_t)L.grid * per_block));
         L.bnd_elems = (size_t)L.grid * per_block / sizeof(uint2);
     }
@@ -2127,8 +2195,7 @@ int sw_init(sw_handle_t **out, const sw_params_t *p, const int *gpu_ids, int n_g
     *out = nullptr;
     sw_params_t prm;
     if (p) prm = *p; else sw_default_params(&prm);
-    int rc = validate_params(&prm);
-    if (rc != SW_OK) return rc;
+    SW_TRY(validate_params(&prm));
     int ndev = 0;
     if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev <= 0) { cudaGetLastError(); return SW_ENODEV; }
     std::vector<int> ids;
@@ -2295,8 +2362,7 @@ int sw_set_queries(sw_handle_t *h, const uint8_t *packed, const uint32_t *len, c
     }
     h->q_packed.resize(h->q_packed.size() + 16, 0);
     for (auto &g : h->gpus) {
-        int rc = upload_queries(h, g);
-        if (rc != SW_OK) return rc;
+        SW_TRY(upload_queries(h, g));
     }
     for (Batch &bt : h->batch) bt.scored = false;
     return SW_OK;
@@ -2341,18 +2407,9 @@ int sw_wait(sw_handle_t *h, int timeout_ms)
     if (!h) return SW_EINVAL;
     const bool forever = timeout_ms < 0;
     const auto t_end = std::chrono::steady_clock::now() + std::chrono::milliseconds(forever ? 0 : timeout_ms);
-    double ms_max = 0.0;
-    for (auto &g : h->gpus) {
-        Slot &b = g.slot[0];
-        if (!b.scored || b.chunks.empty()) continue;
-        SW_CUDA(h, cudaSetDevice(g.dev));
-        int rc = wait_event(h, b.chunks.back().done, t_end, forever);
-        if (rc != SW_OK) return rc;
-        SW_CUDA(h, cudaEventSynchronize(b.ev_stop));
-        float ms = 0.f;
-        SW_CUDA(h, cudaEventElapsedTime(&ms, b.ev_start, b.ev_stop));
-        ms_max = std::max(ms_max, (double)ms);
-    }
+    SW_TRY(wait_slot(h, 0, t_end, forever));
+    double ms_max = 0.0, ms_min = 0.0;
+    SW_TRY(slot_kernel_ms(h, 0, &ms_max, &ms_min));     // (the copy streams are idle between calls)
     h->last_ms = ms_max;
     h->last_cells = h->batch[0].cells;
     return SW_OK;
@@ -2375,13 +2432,10 @@ int sw_score_batch(sw_handle_t *h, const uint8_t *packed, const uint32_t *len, c
     // take the slot that is not in flight; this replaces whatever sw_load_db left there
     const int si = (h->n_inflight == 1) ? (1 - h->fifo[0]) : 0;
     bool taken = false;
-    int rc = small_submit(h, si, packed, len, off, ids, ns, &taken);
-    if (rc != SW_OK) return rc;
+    SW_TRY(small_submit(h, si, packed, len, off, ids, ns, &taken));
     if (!taken) {
-        rc = load_batch(h, si, packed, len, off, ids, ns);
-        if (rc != SW_OK) return rc;
-        rc = score_batch_slot(h, si);
-        if (rc != SW_OK) return rc;
+        SW_TRY(load_batch(h, si, packed, len, off, ids, ns));
+        SW_TRY(score_batch_slot(h, si));
     }
     h->fifo[h->n_inflight++] = si;
     return SW_OK;
@@ -2591,7 +2645,6 @@ int sw_set_small_batch_timing(sw_handle_t *h, int enable)
 int sw_set_arith(sw_handle_t *h, int arith)
 {
     if (!h || arith < -1 || arith > 0) return SW_EINVAL;     /* only packed s16 is compiled in */
-    h->force_arith = arith;
     return SW_OK;
 }
 
