@@ -151,8 +151,8 @@ int sw_fetch_best(sw_handle_t *h, int32_t *best_score, uint64_t *best_index, int
 
 /* ---- output path ------------------------------------------------------------
  * The bank returns a 12-bit score per (ID) slot (ScoreBank_v2.v:39-41); the result buffer the
- * reference planned (CAPI_template/ResBuffer.v:11-22) has ports only.  Four shapes here (the fourth, the hit
- * list of sw_set_hits, is described below):
+ * reference planned (CAPI_template/ResBuffer.v:11-22) has ports only.  Five shapes here (the fourth and fifth, the
+ * hit list of sw_set_hits and the per-subject best of sw_set_subject_best, are described below):
  *   SW_OUTPUT_I32   int32 matrix [rows][ns]                     (default; sw_fetch / sw_fetch_db)
  *   SW_OUTPUT_I16   int16 matrix [rows][ns]: half the HBM and half the D2H bytes.  A score above
  *                   32767 is stored as -1 in the matrix and returned exactly by sw_fetch_overflow
@@ -201,6 +201,29 @@ int sw_fetch_db_topk(sw_handle_t *h, int32_t *scores, uint64_t *index, size_t ca
 int sw_set_hits(sw_handle_t *h, int32_t min_score, size_t max_hits);
 int sw_fetch_hits(sw_handle_t *h, uint32_t *row, uint64_t *index, int32_t *score, size_t cap, size_t *count, int timeout_ms);
 int sw_fetch_db_hits(sw_handle_t *h, uint32_t *row, uint64_t *index, int32_t *score, size_t cap, size_t *count);
+
+/* Per-subject best: for every subject, which query row it matches best and by how much it beats the next one, in
+ * place of a matrix (12 bytes per subject instead of 2 or 4 per pair).  enable != 0 turns it on, 0 turns it off
+ * (back to matrices).  With rows = sw_query_rows(h), for every subject s of the batch:
+ *   best_score[s]   = the largest score over all rows: max over column s of the int32 matrix, exact above 32767 too;
+ *   best_row[s]     = the LOWEST row reaching best_score[s] (row nq + i = reverse complement of query i with
+ *                     sw_set_strands(h, 1));
+ *   second_score[s] = the largest score over all rows other than best_row[s]: equal to best_score[s] when two rows
+ *                     tie, -1 when rows == 1.
+ *   A zero-length subject gives (0, 0, 0), or (0, 0, -1) with one row.  All three arrays are in input order (index =
+ *   input index within the batch; ids via sw_fetch_ids).  The result is the same for every kernel, work order, pass
+ *   split, GPU count and streaming order.  The int16 / int32 output setting is ignored while the mode is on.
+ *   Setting: like the other modes, only while no batch is in flight (SW_EAGAIN), and scored batches become stale.
+ *   It excludes top-k and hits (SW_EINVAL either way round).  Submitting with the forced 32-bit scorer
+ *   (sw_set_kernel_choice force32) is SW_EINVAL; nothing is enqueued then.
+ *   Fetching: cap = entries each array holds; cap < ns: SW_ECAPACITY, nothing written, the batch stays fetchable.
+ *   second_score may be NULL.  More scores beyond 16 bits than the side list holds: SW_ERANGE, the batch is
+ *   consumed.  Fetching a subject-best batch with a matrix / top-k / hits / best-hit call, or a batch of another mode
+ *   with these two, is SW_ESTATE. */
+int sw_set_subject_best(sw_handle_t *h, int enable);
+int sw_fetch_subject_best(sw_handle_t *h, int32_t *best_score, uint32_t *best_row, int32_t *second_score, size_t cap,
+                          int timeout_ms);
+int sw_fetch_db_subject_best(sw_handle_t *h, int32_t *best_score, uint32_t *best_row, int32_t *second_score, size_t cap);
 
 /* ---- introspection --------------------------------------------------------- */
 const char *sw_strerror(int code);

@@ -12,6 +12,7 @@ capi_sample_aligner/software-C,C++/src/main_test.c:290-528):
     Engine.score_batch(...)                          <- stream of type-10 records
     Engine.fetch(timeout_ms)                         <- (IDs, results, vld) + WED poll, result-2048
     Engine.fetch_hits(timeout_ms)                    <- the same stream filtered on results >= min_score
+    Engine.fetch_subject_best(timeout_ms)            <- per ID: the best query row, its score and the runner-up
 """
 import ctypes as C
 import os
@@ -107,6 +108,9 @@ def load_library():
     L.sw_set_hits.argtypes = [vp, C.c_int32, sz]
     L.sw_fetch_hits.argtypes = [vp, vp, vp, vp, sz, C.POINTER(sz), i32]
     L.sw_fetch_db_hits.argtypes = [vp, vp, vp, vp, sz, C.POINTER(sz)]
+    L.sw_set_subject_best.argtypes = [vp, i32]
+    L.sw_fetch_subject_best.argtypes = [vp, vp, vp, vp, sz, i32]
+    L.sw_fetch_db_subject_best.argtypes = [vp, vp, vp, vp, sz]
     L.sw_device_error_bits.argtypes = [vp]
     L.sw_device_error_bits.restype = C.c_uint
     L.sw_is_check_build.restype = i32
@@ -158,6 +162,7 @@ class Engine:
         self.out_mode = SW_OUTPUT_I32
         self.topk = 0
         self.hits = 0        # min_score of the hit-list mode (0 = off)
+        self.subject_best = False
         self._ids_ns = 0     # subjects of the batch sw_fetch_ids refers to (last loaded / fetched)
 
     # -- plumbing ---------------------------------------------------------------------
@@ -289,6 +294,34 @@ class Engine:
         rc, row, idx, sc = self._hits(lambda r, i, s, cap, cnt: self.lib.sw_fetch_db_hits(self.h, r, i, s, cap, cnt))
         self._check(rc)
         return row, idx, sc
+
+    def set_subject_best(self, enable=True):
+        """True: instead of a matrix, per subject its best row, best score and runner-up score
+        (fetch_subject_best / fetch_db_subject_best).  False = back to matrices."""
+        self._check(self.lib.sw_set_subject_best(self.h, int(bool(enable))))
+        self.subject_best = bool(enable)
+
+    @staticmethod
+    def _subject_best_arrays(ns):
+        return np.empty(ns, dtype=np.int32), np.empty(ns, dtype=np.uint32), np.empty(ns, dtype=np.int32)
+
+    def fetch_subject_best(self, timeout_ms=-1):
+        """(best_score int32[ns], best_row uint32[ns], second_score int32[ns]) of the oldest batch in flight:
+        per subject (input order) the column maximum of its int32 matrix, the lowest row reaching it, and the
+        largest score of the other rows (-1 with one row)."""
+        ns = self._batch_ns[0] if self._batch_ns else self.ns
+        bs, br, sec = self._subject_best_arrays(ns)
+        rc = self.lib.sw_fetch_subject_best(self.h, _ptr(bs), _ptr(br), _ptr(sec), ns, timeout_ms)
+        if self._batch_ns and rc in (SW_OK, SW_ERANGE):          # SW_ERANGE consumes the batch too
+            self._ids_ns = self._batch_ns.pop(0)
+        self._check(rc)
+        return bs, br, sec
+
+    def fetch_db_subject_best(self):
+        """fetch_subject_best for the resident database (after score_db)."""
+        bs, br, sec = self._subject_best_arrays(self.ns)
+        self._check(self.lib.sw_fetch_db_subject_best(self.h, _ptr(bs), _ptr(br), _ptr(sec), self.ns))
+        return bs, br, sec
 
     def set_jit(self, mode):
         self._check(self.lib.sw_set_jit(self.h, mode))

@@ -120,9 +120,10 @@ struct Slot {
     DevBuf d_raw, d_off, d_len, d_pair_subj, d_pair_len, d_tile_woff, d_tp, d_out;
     DevBuf d_ovf_count, d_ovf_list, d_ovf_score, d_topk_out;
     DevBuf d_hits_key, d_hits_score, d_hits_count;   // hit list of the last scoring (reserved at the first one in hits mode)
+    DevBuf d_sbest_key, d_sbest_second;              // per-subject best of the last scoring (subject-best mode)
     uint32_t npairs = 0, max_len = 0;
     uint64_t sum_len = 0, tp_words = 0;
-    PinnedBuf h_stage_a, h_stage_b, h_stage_c, h_stage_d, h_topk, h_ovf, h_hits;
+    PinnedBuf h_stage_a, h_stage_b, h_stage_c, h_stage_d, h_topk, h_ovf, h_hits, h_sbest;
     cudaEvent_t ev_start = nullptr, ev_stop = nullptr, ev_upload = nullptr;
     std::vector<cudaEvent_t> ev_pool;  // chunk-done events, created once
     std::vector<QueryChunk> chunks;
@@ -160,7 +161,7 @@ struct GpuCtx {
     DevBuf d_wave_bnd, d_wave_state;  // band-pipelined kernel: boundary rows; progress / best / done words
     int wave_bps[16] = {0};           // resident blocks per SM of its instances (0 = not asked yet)
     DevBuf d_wave32_bnd, d_wave32_state;   // 32-bit band-pipelined scorer of the overflow list
-    DevBuf d_wave_rows;               // top-k / hits mode: one scratch score row per band-pipelined query
+    DevBuf d_wave_rows;               // top-k / hits / subject-best mode: one scratch score row per band-pipelined query
     DevBuf d_hits_key2, d_hits_score2, d_sort_tmp;   // fetch of a hit list: radix-sort output and temp storage (copy stream)
     uint32_t wave32_epoch = 0;        // 8-bit tag field: 1 .. 255, boundary rows zeroed when it restarts
     int wave32_bps = 0;
@@ -179,7 +180,7 @@ struct Batch {
     int nq = 0;                       // query rows the scores of this batch have
     bool loaded = false, scored = false, small = false;
     // output of the scoring, fixed at submit: SW_OUT_I32 / I16 / TOPK (topk_k lists) / HITS (scores >= hits_min,
-    // at most hits_max per GPU)
+    // at most hits_max per GPU) / SBEST (per subject: best score, its row, runner-up score)
     int out_mode = SW_OUT_I32, topk_k = 0;
     int32_t hits_min = 0;
     size_t hits_max = 0;
@@ -215,6 +216,7 @@ struct sw_handle {
     int topk_k = 0;                   // > 0: fused top-k instead of a matrix
     int32_t hits_min = 0;             // > 0: hit list (scores >= hits_min) instead of a matrix
     size_t hits_max = 0;              // entries of each GPU's hit list
+    bool sbest = false;               // per-subject best instead of a matrix
     bool small_path = true;
     bool small_timing = true;         // record CUDA events around the latency path's kernel (sw_last_kernel_ms)
     int jit = 1;                      // run-time specialisation of gap penalties: 0 off, 1 large jobs, 2 always
@@ -296,7 +298,7 @@ std::vector<DevBuf *> all_devbufs(GpuCtx &g)
     for (Slot &b : g.slot) {
         DevBuf *bufs[] = {&b.d_raw, &b.d_off, &b.d_len, &b.d_pair_subj, &b.d_pair_len, &b.d_tile_woff, &b.d_tp, &b.d_out,
                           &b.d_ovf_count, &b.d_ovf_list, &b.d_ovf_score, &b.d_topk_out, &b.d_small_in, &b.d_small_done,
-                          &b.d_hits_key, &b.d_hits_score, &b.d_hits_count};
+                          &b.d_hits_key, &b.d_hits_score, &b.d_hits_count, &b.d_sbest_key, &b.d_sbest_second};
         v.insert(v.end(), std::begin(bufs), std::end(bufs));
     }
     return v;
@@ -310,7 +312,7 @@ void free_gpu(GpuCtx &g)
         for (cudaEvent_t e : b.ev_pool) cudaEventDestroy(e);
         b.ev_pool.clear();
         b.chunks.clear();
-        PinnedBuf *pins[] = {&b.h_stage_a, &b.h_stage_b, &b.h_stage_c, &b.h_stage_d, &b.h_topk, &b.h_ovf, &b.h_hits, &b.h_small_in, &b.h_small_out,
+        PinnedBuf *pins[] = {&b.h_stage_a, &b.h_stage_b, &b.h_stage_c, &b.h_stage_d, &b.h_topk, &b.h_ovf, &b.h_hits, &b.h_sbest, &b.h_small_in, &b.h_small_out,
                              &b.h_small_flag};
         for (PinnedBuf *p : pins) p->release();
         if (b.ev_start) cudaEventDestroy(b.ev_start);
@@ -860,8 +862,8 @@ int push_chunk(sw_handle *h, GpuCtx &gc, Slot &g, int q0, int q1)
 struct ScoreJob {
     GpuCtx &gc; Slot &g; const Batch &bt;   // bt: the output settings
     int nq = 0; size_t n = 0;               // n: subjects of the shard
-    bool topk = false, hits = false, may_overflow = false;
-    SwScoring sc{}; SwDevDb db{}; SwDevQueries dq{}; SwHitList hl{};
+    bool topk = false, hits = false, sbest = false, may_overflow = false;
+    SwScoring sc{}; SwDevDb db{}; SwDevQueries dq{}; SwHitList hl{}; SwSubjectBest sb{};
     std::vector<int> wave_q, strip_q;       // queries of the band-pipelined kernel / of the strip kernel
     SwStripLaunch base;                     // what every strip launch of the scoring has in common
 };
@@ -878,11 +880,20 @@ struct StripPlan {
     size_t n_groups = 0;              // launches of the length-group plan
 };
 
-// Output buffers of a scoring, zeroed on the compute stream: the matrix, the top-k lists or the hit list.
+// Output buffers of a scoring, zeroed on the compute stream: the matrix, the top-k lists, the hit list or the
+// per-subject best.
 int reserve_outputs(sw_handle *h, ScoreJob &j)
 {
     GpuCtx &gc = j.gc; Slot &g = j.g;
-    if (j.hits) {
+    if (j.sbest) {
+        // key 0 = a phantom row scoring 0 (scores are >= 0); with one row the runner-up is -1 and never updated
+        SW_CUDA(h, g.d_sbest_key.reserve(j.n * sizeof(unsigned long long)));
+        SW_CUDA(h, g.d_sbest_second.reserve(j.n * sizeof(int32_t)));
+        SW_CUDA(h, cudaMemsetAsync(g.d_sbest_key.p, 0, j.n * sizeof(unsigned long long), gc.st_compute));
+        SW_CUDA(h, cudaMemsetAsync(g.d_sbest_second.p, j.nq == 1 ? 0xFF : 0, j.n * sizeof(int32_t), gc.st_compute));
+        j.sb.key = g.d_sbest_key.as<unsigned long long>();
+        j.sb.second = j.nq > 1 ? g.d_sbest_second.as<int32_t>() : nullptr;
+    } else if (j.hits) {
         // hit list: keys row << hits_shift | shard-local subject (the fetch sorts them: row-major order)
         int sb = 0;
         while ((1ull << sb) < (uint64_t)j.n) ++sb;
@@ -973,7 +984,7 @@ int plan_one_launch(sw_handle *h, ScoreJob &j, StripPlan &p)
     int vidx = choose_variant(h, gc, g, p.qlen.data(), p.qlen.size(), p.maxq, &ranked, false);
     if (vidx < 0) return SW_EINVAL;
     const double est_ms_all = (double)g.sum_len * (double)p.rows / 6.0e9;
-    const bool one_chunk = j.topk || j.hits || j.may_overflow || !j.wave_q.empty();
+    const bool one_chunk = j.topk || j.hits || j.sbest || j.may_overflow || !j.wave_q.empty();
     if (h->pass_split != 0 && !variant_forced(h) && sw_strip_variant(vidx)->G > 1) {
         // The model asks for more lanes per pair because whole items of a one-lane variant would leave
         // the last round partly empty.  With the pass split that round costs a fraction of a part, so a
@@ -998,7 +1009,7 @@ int plan_one_launch(sw_handle *h, ScoreJob &j, StripPlan &p)
             int choice = vidx;
             // the sample launches append nothing: a pair they score is scored again by the real launch
             SwStripLaunch sample = j.base;
-            if (j.hits) { sample.hits.keys = nullptr; sample.ovf_list = nullptr; sample.ovf_count = nullptr; }
+            if (j.hits || j.sbest) { sample.hits.keys = nullptr; sample.sbest.key = nullptr; sample.ovf_list = nullptr; sample.ovf_count = nullptr; }
             SW_TRY(autotune_variant(h, gc, g, sample, ranked, nq, p.same_len, &choice));
             gc.tune_choice = choice;
             gc.tune_key = key;
@@ -1228,7 +1239,7 @@ void set_kernel_label(sw_handle *h, const ScoreJob &j, const StripPlan &p)
 int enqueue_strip(sw_handle *h, ScoreJob &j, StripPlan &p)
 {
     GpuCtx &gc = j.gc;
-    const bool chunk_events = p.simple && p.launches.size() > 1 && !j.may_overflow && !j.topk && !j.hits;
+    const bool chunk_events = p.simple && p.launches.size() > 1 && !j.may_overflow && !j.topk && !j.hits && !j.sbest;
     bool forked[kStreams] = {false, false, false, false};
     for (Planned &pl : p.launches) {
         SwStripLaunch &L = pl.L;
@@ -1264,7 +1275,8 @@ int enqueue_strip(sw_handle *h, ScoreJob &j, StripPlan &p)
     return SW_OK;
 }
 
-// Band-pipelined launches, one per long query (top-k / hits: into a scratch row per query, filtered from there).
+// Band-pipelined launches, one per long query (top-k / hits / subject best: into a scratch row per query, reduced
+// from there).
 int enqueue_wave(sw_handle *h, ScoreJob &j)
 {
     GpuCtx &gc = j.gc; const Slot &g = j.g;
@@ -1291,9 +1303,10 @@ int enqueue_wave(sw_handle *h, ScoreJob &j)
         W.db = j.db; W.q = j.dq; W.query = q; W.sc = j.sc;
         W.npass = (int)((h->q_len[q] + rows - 1) / rows);
         W.out = g.d_out.p; W.out_stride = n; W.out_mode = j.bt.out_mode;
-        if (j.topk || j.hits) { W.out = gc.d_wave_rows.p; W.out_mode = SW_OUT_I32; W.out_row = wave_row; }
+        const bool scratch_row = j.topk || j.hits || j.sbest;
+        if (scratch_row) { W.out = gc.d_wave_rows.p; W.out_mode = SW_OUT_I32; W.out_row = wave_row; }
         W.bnd = gc.d_wave_bnd.p; W.cols_stride = cols_stride;
-        W.bnd_elems = (size_t)g.npairs * 2 * cols_stride; W.out_elems = (j.topk || j.hits) ? j.wave_q.size() * n : (size_t)j.nq * n;
+        W.bnd_elems = (size_t)g.npairs * 2 * cols_stride; W.out_elems = scratch_row ? j.wave_q.size() * n : (size_t)j.nq * n;
         gc.wave_epoch = (gc.wave_epoch % 0xFFFFEu) + 1u;            // 1 .. 2^20 - 2
         if (gc.wave_epoch == 1u && gc.counter_next > 0) {
             // the epoch wrapped (or first use): stale tags must not match again
@@ -1312,20 +1325,22 @@ int enqueue_wave(sw_handle *h, ScoreJob &j)
         SW_CUDA(h, cudaMemsetAsync(W.counter, 0, sizeof(unsigned), gc.st_compute));
         SW_CUDA(h, sw_launch_wave(gc.st_compute, W));
         h->launches++;
-        if (!j.topk && !j.hits) continue;
+        if (!scratch_row) continue;
         const int32_t *row = (const int32_t *)gc.d_wave_rows.p + (size_t)wave_row * n;
         if (j.topk)         // the row's k best scores become list 0 of this query (pairs flagged for the 32-bit
                             // scorer keep the sentinel here and reach the merge through the overflow list)
             SW_CUDA(h, sw_launch_topk_row(gc.st_compute, row, (uint32_t)n, q, j.bt.topk_k, gc.d_topk_keys.as<unsigned long long>()));
-        else                // the row's entries >= min_score join the list (flagged pairs come from the overflow list)
+        else if (j.hits)    // the row's entries >= min_score join the list (flagged pairs come from the overflow list)
             SW_CUDA(h, sw_launch_hits_row(gc.st_compute, row, (uint32_t)n, q, j.hl));
+        else                // the row's scores update the per-subject best (flagged pairs: from the overflow list)
+            SW_CUDA(h, sw_launch_sbest_row(gc.st_compute, row, (uint32_t)n, q, j.sb));
         h->launches++;
     }
     return SW_OK;
 }
 
 // Scratch of the launches, zeroed where they need it: top-k key lists, score rows of the band-pipelined queries
-// (top-k / hits), and the 32-bit scorer's (force32, or the overflow fix-up of the few listed pairs) with its launch.
+// (top-k / hits / subject best), and the 32-bit scorer's (force32, or the overflow fix-up of the few listed pairs) with its launch.
 int reserve_scratch(sw_handle *h, const ScoreJob &j, StripPlan &p, bool use32, SwScore32Launch &s32)
 {
     GpuCtx &gc = j.gc;
@@ -1335,7 +1350,7 @@ int reserve_scratch(sw_handle *h, const ScoreJob &j, StripPlan &p, bool use32, S
         SW_CUDA(h, gc.d_topk_keys.reserve(bytes));
         SW_CUDA(h, cudaMemsetAsync(gc.d_topk_keys.p, 0, bytes, gc.st_compute));
     }
-    if ((j.topk || j.hits) && !j.wave_q.empty()) {
+    if ((j.topk || j.hits || j.sbest) && !j.wave_q.empty()) {
         const size_t rb = j.wave_q.size() * j.n * sizeof(int32_t);
         SW_CUDA(h, gc.d_wave_rows.reserve(rb));
         SW_CUDA(h, cudaMemsetAsync(gc.d_wave_rows.p, 0xFF, rb, gc.st_compute));    // -1 = not scored here
@@ -1350,13 +1365,14 @@ int reserve_scratch(sw_handle *h, const ScoreJob &j, StripPlan &p, bool use32, S
         threads32 = (int)t;
         SW_CUDA(h, gc.d_scratch32.reserve((size_t)2 * max_cols * threads32 * sizeof(int32_t)));
     }
-    s32.db = j.db; s32.q = j.dq; s32.sc = j.sc; s32.out = (j.topk || j.hits) ? nullptr : j.g.d_out.p; s32.out_stride = j.n;
+    s32.db = j.db; s32.q = j.dq; s32.sc = j.sc; s32.out = (j.topk || j.hits || j.sbest) ? nullptr : j.g.d_out.p; s32.out_stride = j.n;
     s32.out_mode = j.bt.out_mode; s32.scratch = gc.d_scratch32.as<int32_t>(); s32.max_cols = max_cols; s32.threads_total = threads32;
     return SW_OK;
 }
 
 // Exact scores of the pairs on the overflow list: long entries on the band-pipelined 32-bit scorer, the
-// rest on the 32-bit scorer; in hits mode the list's entries >= min_score then join the hit list.
+// rest on the 32-bit scorer; in hits mode the list's entries >= min_score then join the hit list, in subject-best
+// mode the list's exact scores update the per-subject best.
 int enqueue_overflow(sw_handle *h, ScoreJob &j, SwScore32Launch &s32)
 {
     GpuCtx &gc = j.gc; const Slot &g = j.g;
@@ -1413,6 +1429,10 @@ int enqueue_overflow(sw_handle *h, ScoreJob &j, SwScore32Launch &s32)
         SW_CUDA(h, sw_launch_hits_ovf(gc.st_compute, s32.list_count, s32.list, s32.list_score, kOvfCap, j.hl));
         h->launches++;
     }
+    if (j.sbest) {
+        SW_CUDA(h, sw_launch_sbest_ovf(gc.st_compute, s32.list_count, s32.list, s32.list_score, kOvfCap, j.sb));
+        h->launches++;
+    }
     return SW_OK;
 }
 
@@ -1434,7 +1454,7 @@ int score_gpu(sw_handle *h, GpuCtx &gc, Slot &g, const Batch &bt)
 {
     if (&gc == &h->gpus[0]) h->last_parts = 1;
     SW_CUDA(h, cudaSetDevice(gc.dev));
-    ScoreJob j{gc, g, bt, bt.nq, g.s1 - g.s0, bt.out_mode == SW_OUT_TOPK, bt.out_mode == SW_OUT_HITS};
+    ScoreJob j{gc, g, bt, bt.nq, g.s1 - g.s0, bt.out_mode == SW_OUT_TOPK, bt.out_mode == SW_OUT_HITS, bt.out_mode == SW_OUT_SBEST};
     g.chunks.clear();
     g.scored = true;
     g.ovf_used = false;
@@ -1456,9 +1476,11 @@ int score_gpu(sw_handle *h, GpuCtx &gc, Slot &g, const Batch &bt)
 
     SwStripLaunch &base = j.base;
     base.db = j.db; base.q = j.dq; base.sc = j.sc;
-    base.out = (j.topk || j.hits) ? nullptr : g.d_out.p; base.out_stride = j.n; base.out_elems = j.hits ? bt.hits_max : (size_t)j.nq * j.n;
+    base.out = (j.topk || j.hits || j.sbest) ? nullptr : g.d_out.p; base.out_stride = j.n;
+    base.out_elems = j.hits ? bt.hits_max : j.sbest ? j.n : (size_t)j.nq * j.n;
     base.out_mode = bt.out_mode;
     base.hits = j.hl;
+    base.sbest = j.sb;
     base.dev_err = gc.d_err.as<unsigned>();
     if (j.may_overflow) {
         SW_CUDA(h, g.d_ovf_count.reserve(sizeof(unsigned)));
@@ -1473,7 +1495,8 @@ int score_gpu(sw_handle *h, GpuCtx &gc, Slot &g, const Batch &bt)
     if (&gc == &h->gpus[0]) set_kernel_label(h, j, p);
 
     const bool use32 = p.launches.empty() && j.wave_q.empty();        // forced 32-bit scorer
-    if (use32 && (j.topk || j.hits)) return SW_EINVAL;   // it has no top-k epilogue and no hit list (hits: refused at submit)
+    // it has no top-k epilogue, no hit list and no per-subject best (hits / subject best: refused at submit)
+    if (use32 && (j.topk || j.hits || j.sbest)) return SW_EINVAL;
     SwScore32Launch s32;
     SW_TRY(reserve_scratch(h, j, p, use32, s32));
     if (use32) {
@@ -1710,7 +1733,7 @@ int fetch_slot(sw_handle *h, int si, FetchKind kind, void *scores, uint64_t *ind
     const bool forever = timeout_ms < 0;
     const auto t_fetch0 = std::chrono::steady_clock::now();
     const auto t_end = t_fetch0 + std::chrono::milliseconds(forever ? 0 : timeout_ms);
-    // (a hits batch has no matrix / top-k lists)
+    // (a hits / subject-best batch has no matrix / top-k lists)
     if (bt.out_mode != (kind == FETCH_TOPK ? SW_OUT_TOPK : kind == FETCH_I16 ? SW_OUT_I16 : SW_OUT_I32)) return SW_ESTATE;
     if (cap < nq * (kind == FETCH_TOPK ? (size_t)bt.topk_k : bt.ns)) return SW_ECAPACITY;
     if (bt.small) return fetch_small(h, si, scores, t_fetch0, t_end, forever);
@@ -1854,6 +1877,59 @@ int fetch_hits_slot(sw_handle *h, int si, uint32_t *row, uint64_t *index, int32_
     return SW_OK;
 }
 
+// Per-subject best of a batch: wait for every GPU's kernels, check the overflow side list, copy each GPU's key and
+// runner-up arrays to pinned staging on its copy stream (the next batch's kernels keep running), then decode them
+// into the caller's arrays.  Shards are disjoint input ranges: each GPU's subjects go to offset s0, no merge.
+int fetch_sbest_slot(sw_handle *h, int si, int32_t *best_score, uint32_t *best_row, int32_t *second_score, size_t cap,
+                     int timeout_ms)
+{
+    Batch &bt = h->batch[si];
+    if (bt.out_mode != SW_OUT_SBEST) return SW_ESTATE;
+    if (cap < bt.ns) return SW_ECAPACITY;
+    const bool forever = timeout_ms < 0;
+    const auto t_fetch0 = std::chrono::steady_clock::now();
+    const auto t_end = t_fetch0 + std::chrono::milliseconds(forever ? 0 : timeout_ms);
+    SW_TRY(wait_slot(h, si, t_end, forever));
+    for (auto &g : h->gpus) {
+        Slot &b = g.slot[si];
+        if (!b.scored || b.chunks.empty() || !b.ovf_used) continue;
+        SW_CUDA(h, cudaSetDevice(g.dev));
+        unsigned novf = 0;
+        SW_CUDA(h, cudaMemcpy(&novf, b.d_ovf_count.p, sizeof novf, cudaMemcpyDeviceToHost));
+        if (novf > kOvfCap) return SW_ERANGE;       // pairs beyond the list never updated their subjects
+    }
+    for (auto &g : h->gpus) {
+        Slot &b = g.slot[si];
+        const size_t n = b.s1 - b.s0;
+        if (!b.scored || b.chunks.empty()) continue;
+        SW_CUDA(h, cudaSetDevice(g.dev));
+        SW_CUDA(h, b.h_sbest.reserve(n * (sizeof(unsigned long long) + sizeof(int32_t))));
+        SW_CUDA(h, cudaMemcpyAsync(b.h_sbest.p, b.d_sbest_key.p, n * sizeof(unsigned long long), cudaMemcpyDeviceToHost, g.st_copy));
+        if (second_score)
+            SW_CUDA(h, cudaMemcpyAsync((unsigned long long *)b.h_sbest.p + n, b.d_sbest_second.p, n * sizeof(int32_t),
+                                       cudaMemcpyDeviceToHost, g.st_copy));
+    }
+    const auto t_fetch1 = std::chrono::steady_clock::now();
+    double ms_max = 0.0, ms_min = 0.0;
+    SW_TRY(slot_kernel_ms(h, si, &ms_max, &ms_min));
+    for (auto &g : h->gpus) {
+        const Slot &b = g.slot[si];
+        const size_t n = b.s1 - b.s0;
+        if (!b.scored || b.chunks.empty()) continue;
+        const unsigned long long *key = (const unsigned long long *)b.h_sbest.p;
+        for (size_t i = 0; i < n; ++i) {
+            // key 0 (never updated: a zero-length subject) is the phantom row 0 scoring 0
+            best_score[b.s0 + i] = (int32_t)(key[i] >> 32);
+            best_row[b.s0 + i] = key[i] ? 0xFFFFFFFFu - (uint32_t)key[i] : 0u;
+        }
+        if (second_score) std::memcpy(second_score + b.s0, key + n, n * sizeof(int32_t));
+    }
+    bt.ovf_index.clear(); bt.ovf_score.clear();          // sw_fetch_overflow: nothing for a subject-best batch
+    finish_timing(h, si, t_fetch0, t_fetch1, ms_max, ms_min);
+    if (device_error_bits(h)) return SW_EDEVICE;
+    return SW_OK;
+}
+
 int load_batch(sw_handle *h, int si, const uint8_t *packed, const uint32_t *len, const uint64_t *off,
                const uint64_t *ids, size_t ns)
 {
@@ -1892,10 +1968,10 @@ int load_batch(sw_handle *h, int si, const uint8_t *packed, const uint32_t *len,
     return SW_OK;
 }
 
-// The output of a scoring submitted now: top-k and hit list replace the matrix.
+// The output of a scoring submitted now: top-k, hit list and per-subject best replace the matrix.
 void take_output_settings(const sw_handle *h, Batch &bt)
 {
-    bt.out_mode = h->topk_k > 0 ? SW_OUT_TOPK : h->hits_min > 0 ? SW_OUT_HITS : h->out_mode;
+    bt.out_mode = h->topk_k > 0 ? SW_OUT_TOPK : h->hits_min > 0 ? SW_OUT_HITS : h->sbest ? SW_OUT_SBEST : h->out_mode;
     bt.topk_k = h->topk_k;
     bt.hits_min = h->hits_min; bt.hits_max = h->hits_max; bt.hits_staged = false;
 }
@@ -1964,8 +2040,8 @@ int small_submit(sw_handle *h, int si, const uint8_t *packed, const uint32_t *le
     *taken = false;
     const int nq = (int)h->q_len.size();
     if (!h->small_path || ns == 0 || nq == 0 || ns > 8192 || (size_t)nq * ns > (1u << 20)) return SW_OK;
-    // (hits mode: the completion protocol below reads a fixed number of result words, a list has no such end)
-    if (h->topk_k > 0 || h->hits_min > 0 || h->out_mode != SW_OUT_I32 || h->params.score_width != 0) return SW_OK;
+    // (hits / subject-best mode: the completion protocol below reads a fixed number of int32 result words)
+    if (h->topk_k > 0 || h->hits_min > 0 || h->sbest || h->out_mode != SW_OUT_I32 || h->params.score_width != 0) return SW_OK;
     uint64_t bmin = ~0ull, bmax = 0, sum = 0;
     uint32_t maxlen = 0;
     size_t n_empty = 0;
@@ -2116,8 +2192,9 @@ int fetch_db_common(sw_handle_t *h, FetchKind kind, void *scores, uint64_t *inde
     return fetch_slot(h, 0, kind, scores, index, cap, -1);
 }
 
-// hits mode with the forced 32-bit scorer: refused before anything is enqueued (that scorer has no hit list)
-bool hits_need_strip(const sw_handle *h) { return h->hits_min > 0 && h->force32; }
+// hits / subject-best mode with the forced 32-bit scorer: refused before anything is enqueued (that scorer has no
+// hit list and no per-subject best)
+bool mode_needs_strip(const sw_handle *h) { return (h->hits_min > 0 || h->sbest) && h->force32; }
 
 int fetch_common(sw_handle_t *h, FetchKind kind, void *scores, uint64_t *index, size_t cap, int timeout_ms)
 {
@@ -2290,7 +2367,7 @@ int sw_set_output(sw_handle_t *h, int mode)
 
 int sw_set_topk(sw_handle_t *h, int k)
 {
-    if (!h || k < 0 || k > SW_MAX_TOPK || (k > 0 && h->hits_min > 0)) return SW_EINVAL;
+    if (!h || k < 0 || k > SW_MAX_TOPK || (k > 0 && (h->hits_min > 0 || h->sbest))) return SW_EINVAL;
     if (h->n_inflight) return SW_EAGAIN;
     h->topk_k = k;
     for (Batch &bt : h->batch) bt.scored = false;
@@ -2301,7 +2378,7 @@ int sw_set_hits(sw_handle_t *h, int32_t min_score, size_t max_hits)
 {
     // (the device counter is 32-bit and counts past the list's end; the radix sort takes an int count)
     if (!h || min_score < 0 || (min_score > 0 && (max_hits == 0 || max_hits > 0x7FFFFFFFu))) return SW_EINVAL;
-    if (min_score > 0 && h->topk_k > 0) return SW_EINVAL;
+    if (min_score > 0 && (h->topk_k > 0 || h->sbest)) return SW_EINVAL;
     if (h->n_inflight) return SW_EAGAIN;
     h->hits_min = min_score;
     h->hits_max = min_score > 0 ? max_hits : 0;
@@ -2324,6 +2401,31 @@ int sw_fetch_db_hits(sw_handle_t *h, uint32_t *row, uint64_t *index, int32_t *sc
     if (h->n_inflight) return SW_EAGAIN;
     if (!h->batch[0].loaded || !h->batch[0].scored) return SW_ESTATE;
     return fetch_hits_slot(h, 0, row, index, score, cap, count, -1);
+}
+
+int sw_set_subject_best(sw_handle_t *h, int enable)
+{
+    if (!h || (enable && (h->topk_k > 0 || h->hits_min > 0))) return SW_EINVAL;
+    if (h->n_inflight) return SW_EAGAIN;
+    h->sbest = enable != 0;
+    for (Batch &bt : h->batch) bt.scored = false;
+    return SW_OK;
+}
+
+int sw_fetch_subject_best(sw_handle_t *h, int32_t *best_score, uint32_t *best_row, int32_t *second_score, size_t cap,
+                          int timeout_ms)
+{
+    if (!h || !best_score || !best_row) return SW_EINVAL;
+    if (h->n_inflight == 0) return SW_ESTATE;
+    return pop_fifo(h, fetch_sbest_slot(h, h->fifo[0], best_score, best_row, second_score, cap, timeout_ms));
+}
+
+int sw_fetch_db_subject_best(sw_handle_t *h, int32_t *best_score, uint32_t *best_row, int32_t *second_score, size_t cap)
+{
+    if (!h || !best_score || !best_row) return SW_EINVAL;
+    if (h->n_inflight) return SW_EAGAIN;
+    if (!h->batch[0].loaded || !h->batch[0].scored) return SW_ESTATE;
+    return fetch_sbest_slot(h, 0, best_score, best_row, second_score, cap, -1);
 }
 
 int sw_set_queries(sw_handle_t *h, const uint8_t *packed, const uint32_t *len, const uint64_t *off, int nq)
@@ -2398,7 +2500,7 @@ int sw_score_db(sw_handle_t *h)
     if (!h) return SW_EINVAL;
     if (h->n_inflight) return SW_EAGAIN;
     if (!h->batch[0].loaded || h->batch[0].small) return SW_ESTATE;
-    if (hits_need_strip(h)) return SW_EINVAL;
+    if (mode_needs_strip(h)) return SW_EINVAL;
     return score_batch_slot(h, 0);
 }
 
@@ -2428,7 +2530,7 @@ int sw_score_batch(sw_handle_t *h, const uint8_t *packed, const uint32_t *len, c
 {
     if (!h || (ns > 0 && (!packed || !len || !off))) return SW_EINVAL;
     if (h->n_inflight >= 2) return SW_EAGAIN;          // both buffers busy: the bank's `full`
-    if (hits_need_strip(h)) return SW_EINVAL;
+    if (mode_needs_strip(h)) return SW_EINVAL;
     // take the slot that is not in flight; this replaces whatever sw_load_db left there
     const int si = (h->n_inflight == 1) ? (1 - h->fifo[0]) : 0;
     bool taken = false;

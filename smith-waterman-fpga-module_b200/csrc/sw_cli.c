@@ -4,12 +4,14 @@
  *
  *   sw_b200_cli -q query.fa -l library.fa [-t seconds] [-o out.txt] [-R score.txt]
  *               [-m match] [-x mismatch] [-g gap_open] [-e gap_extend] [-w score_width] [-G ngpus]
- *               [-T min_score]
+ *               [-T min_score] [-B]
  *
  * Without -o / -R it prints, like main_test, "result: %d, biased: %d" for every pair
  * (biased = score + 2048, the RTL's ZERO offset).  -T scores in hit-list mode (sw_set_hits) and prints
  * those lines only for the pairs scoring at least min_score; -o / -R list every subject, so they do
- * not combine with it.
+ * not combine with it.  -B scores in subject-best mode (sw_set_subject_best) and prints one line per
+ * subject, "<subject> best <query> result: %d, second: %d" (second = -1 with one query); it combines
+ * with none of -o / -R / -T.
  */
 #include "../../include/sw_b200.h"
 
@@ -21,25 +23,25 @@ static void usage(const char *n)
 {
     fprintf(stderr, "Usage: %s -q <query.fa> -l <library.fa> [-t timeout_s] [-o out.txt] [-R score.txt]\n"
                     "          [-m match] [-x mismatch] [-g gap_open] [-e gap_extend] [-w score_width] [-G ngpus]\n"
-                    "          [-T min_score]\n", n);
+                    "          [-T min_score] [-B]\n", n);
 }
 
 int main(int argc, char **argv)
 {
     const char *qf = NULL, *lf = NULL, *of = NULL, *rf = NULL;
-    int timeout_s = 10, ngpus = 1, opt, rc, i, min_score = 0;
+    int timeout_s = 10, ngpus = 1, opt, rc, i, min_score = 0, subject_best = 0;
     sw_params_t p;
     sw_handle_t *h = NULL;
     sw_seqset_t *q = NULL, *db = NULL;
-    int32_t *scores = NULL, *hscore = NULL;
-    uint32_t *hrow = NULL;
+    int32_t *scores = NULL, *hscore = NULL, *bscore = NULL, *bsecond = NULL;
+    uint32_t *hrow = NULL, *brow = NULL;
     uint64_t *hindex = NULL;
     size_t nhits = 0;
     int gpu_ids[64];
     static struct option lo[] = {{"timeout", required_argument, 0, 't'}, {"query", required_argument, 0, 'q'},
                                  {"library", required_argument, 0, 'l'}, {"help", no_argument, 0, 'h'}, {0, 0, 0, 0}};
     sw_default_params(&p);
-    while ((opt = getopt_long(argc, argv, "ht:q:l:o:R:m:x:g:e:w:G:T:", lo, NULL)) >= 0) {
+    while ((opt = getopt_long(argc, argv, "ht:q:l:o:R:m:x:g:e:w:G:T:B", lo, NULL)) >= 0) {
         switch (opt) {
             case 'q': qf = optarg; break;
             case 'l': lf = optarg; break;
@@ -53,6 +55,7 @@ int main(int argc, char **argv)
             case 'w': p.score_width = atoi(optarg); break;
             case 'G': ngpus = atoi(optarg); break;
             case 'T': min_score = atoi(optarg); break;
+            case 'B': subject_best = 1; break;
             case 'h': usage(argv[0]); return 0;
             default: usage(argv[0]); return -1;
         }
@@ -60,6 +63,11 @@ int main(int argc, char **argv)
     if (!qf || !lf) { printf("Input files missing\n"); usage(argv[0]); return -1; }
     if (min_score < 0 || (min_score > 0 && (of || rf))) {
         printf("-T takes a score >= 1 and prints hits only: it does not combine with -o / -R\n");
+        usage(argv[0]);
+        return -1;
+    }
+    if (subject_best && (of || rf || min_score > 0)) {
+        printf("-B prints each subject's best query only: it does not combine with -o / -R / -T\n");
         usage(argv[0]);
         return -1;
     }
@@ -75,6 +83,7 @@ int main(int argc, char **argv)
         if (max_hits > ((size_t)1 << 26)) max_hits = (size_t)1 << 26;
         if ((rc = sw_set_hits(h, min_score, max_hits ? max_hits : 1)) != SW_OK) goto fail;
     }
+    if (subject_best && (rc = sw_set_subject_best(h, 1)) != SW_OK) goto fail;
     if ((rc = sw_set_queries(h, q->packed, q->len, q->off, (int)q->n)) != SW_OK) goto fail;
     if ((rc = sw_score_batch(h, db->packed, db->len, db->off, NULL, db->n)) != SW_OK) goto fail;
     if (min_score > 0) {
@@ -91,6 +100,17 @@ int main(int argc, char **argv)
             printf("%s x %s result: %d, biased: %d(0x%04x)\n", q->name[hrow[i]], db->name[hindex[i]],
                    (int)hscore[i], (int)hscore[i] + 2048, (unsigned)(hscore[i] + 2048));
         free(hrow); free(hindex); free(hscore); sw_destroy(h); sw_seqset_free(q); sw_seqset_free(db);
+        return 0;
+    }
+    if (subject_best) {
+        bscore = (int32_t *)malloc((db->n + 1) * sizeof *bscore);
+        bsecond = (int32_t *)malloc((db->n + 1) * sizeof *bsecond);
+        brow = (uint32_t *)malloc((db->n + 1) * sizeof *brow);
+        if (!bscore || !bsecond || !brow) { rc = SW_ENOMEM; goto fail; }
+        if ((rc = sw_fetch_subject_best(h, bscore, brow, bsecond, db->n, timeout_s * 1000)) != SW_OK) goto fail;
+        for (i = 0; (size_t)i < db->n; ++i)
+            printf("%s best %s result: %d, second: %d\n", db->name[i], q->name[brow[i]], (int)bscore[i], (int)bsecond[i]);
+        free(bscore); free(bsecond); free(brow); sw_destroy(h); sw_seqset_free(q); sw_seqset_free(db);
         return 0;
     }
     scores = (int32_t *)calloc(q->n * db->n + 1, sizeof(int32_t));
@@ -125,6 +145,6 @@ fail:
     printf("error: %s", sw_strerror(rc));
     if (rc == SW_ECUDA) printf(" [%s]", sw_last_cuda_error_string(h));
     printf("\n");
-    free(scores); free(hrow); free(hindex); free(hscore); sw_destroy(h); sw_seqset_free(q); sw_seqset_free(db);
+    free(scores); free(hrow); free(hindex); free(hscore); free(bscore); free(bsecond); free(brow); sw_destroy(h); sw_seqset_free(q); sw_seqset_free(db);
     return -1;
 }

@@ -340,6 +340,7 @@ cudaError_t sw_launch_strip(cudaStream_t st, const SwStripLaunch &L)
     a.topk_keys = L.topk_keys; a.topk_k = L.topk_k; a.topk_nq = L.topk_nq;
     a.hits = L.hits.keys; a.hits_score = L.hits.score; a.hits_count = L.hits.count; a.hits_cap = L.hits.cap;
     a.min_score = L.hits.min_score; a.hits_shift = L.hits.shift;
+    a.sbest_key = L.sbest.key; a.sbest_second = L.sbest.second;
     a.dev_err = L.dev_err;
     a.done_count = L.done_count; a.done_flag = L.done_flag; a.done_seq = L.done_seq;
 #ifdef SW_BOUNDS_CHECK
@@ -347,6 +348,7 @@ cudaError_t sw_launch_strip(cudaStream_t st, const SwStripLaunch &L)
 #endif
     if (L.out_mode == SW_OUT_TOPK && (L.topk_k < 1 || L.topk_k > kMaxTopK || !L.topk_keys)) return cudaErrorInvalidValue;
     if (L.out_mode == SW_OUT_HITS && (L.direct || (L.hits.keys && (!L.hits.score || !L.hits.count)))) return cudaErrorInvalidValue;
+    if (L.out_mode == SW_OUT_SBEST && L.direct) return cudaErrorInvalidValue;
     const size_t smem = sw_strip_smem_bytes(L.vidx, L.chunk_passes);
     if (L.jit_kernel && !L.direct && !sc.limit) {
         void *params[] = {&a};
@@ -591,6 +593,42 @@ cudaError_t sw_launch_hits_ovf(cudaStream_t st, const unsigned *ovf_count, const
 {
     if (!hl.keys) return cudaSuccess;
     hits_ovf_kernel<<<std::max<unsigned>(1, std::min<unsigned>((ovf_cap + 255) / 256, 256)), 256, 0, st>>>(ovf_count, ovf_list, ovf_score, ovf_cap, hl);
+    return cudaGetLastError();
+}
+
+namespace {
+// per-subject best updates of one materialised score row (the band-pipelined kernel's) / of the overflow list
+__global__ void __launch_bounds__(256) sbest_row_kernel(const int32_t *row, uint32_t n, int q, const SwSubjectBest sb)
+{
+    const uint32_t stride = gridDim.x * blockDim.x;
+    for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) {
+        const int32_t v = row[i];
+        if (v >= 0) sbest_update(sb.key, sb.second, i, q, v);                // < 0: not scored here / sentinel
+    }
+}
+
+__global__ void __launch_bounds__(256) sbest_ovf_kernel(const unsigned *ovf_count, const uint2 *ovf_list, const int32_t *ovf_score,
+                                                        unsigned ovf_cap, const SwSubjectBest sb)
+{
+    const unsigned c = *ovf_count, n = c < ovf_cap ? c : ovf_cap;
+    for (unsigned i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x)
+        sbest_update(sb.key, sb.second, ovf_list[i].y, (int)ovf_list[i].x, ovf_score[i]);
+}
+}  // namespace
+
+cudaError_t sw_launch_sbest_row(cudaStream_t st, const int32_t *row, uint32_t n, int q, const SwSubjectBest &sb)
+{
+    if (n == 0 || !sb.key) return cudaSuccess;
+    const uint32_t grid = std::min<uint32_t>((n + 255) / 256, 1024);
+    sbest_row_kernel<<<grid, 256, 0, st>>>(row, n, q, sb);
+    return cudaGetLastError();
+}
+
+cudaError_t sw_launch_sbest_ovf(cudaStream_t st, const unsigned *ovf_count, const uint2 *ovf_list, const int32_t *ovf_score,
+                                unsigned ovf_cap, const SwSubjectBest &sb)
+{
+    if (!sb.key) return cudaSuccess;
+    sbest_ovf_kernel<<<std::max<unsigned>(1, std::min<unsigned>((ovf_cap + 255) / 256, 256)), 256, 0, st>>>(ovf_count, ovf_list, ovf_score, ovf_cap, sb);
     return cudaGetLastError();
 }
 

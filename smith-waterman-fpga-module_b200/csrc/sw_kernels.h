@@ -14,6 +14,7 @@
 #define SW_OUT_I16  1
 #define SW_OUT_TOPK 2
 #define SW_OUT_HITS 3
+#define SW_OUT_SBEST 4
 #define SW_MAX_TOPK 32
 
 /* Database shard resident in HBM.  Layout (DESIGN.md "data layout"):
@@ -87,6 +88,14 @@ struct SwHitList {
     int min_score = 1, shift = 0;
 };
 
+/* Per-subject best (SW_OUT_SBEST): key[s] = score << 32 | (0xFFFFFFFF - row) of subject s's best row, second[s] = the
+ * best score of its other rows (sbest_update in sw_strip.cuh); both over the shard's subjects.  key == null: update
+ * nothing; second == null: one row only. */
+struct SwSubjectBest {
+    unsigned long long *key = nullptr;
+    int32_t *second = nullptr;
+};
+
 /* One strip-kernel launch: queries qidx[0..nql) (or q0 .. q0+nql-1 when qidx is null) against all
  * pairs of db.  bnd: scratch for pass boundaries, grid * bnd_cols * (block_threads/G) uint2.
  * counter: zeroed device word (work queue) or null for a static schedule.  chunk_passes: passes (of
@@ -122,6 +131,7 @@ struct SwStripLaunch {
     unsigned long long *topk_keys = nullptr;
     int topk_k = 0, topk_nq = 0;
     SwHitList hits{};             /* SW_OUT_HITS; out_elems is then the list's allocated length (bounds-check build) */
+    SwSubjectBest sbest{};        /* SW_OUT_SBEST; out_elems is then the shard's subject count (bounds-check build) */
     unsigned *dev_err = nullptr;
     unsigned *done_count = nullptr, *done_flag = nullptr;   /* latency path: completion flag in mapped host memory */
     unsigned done_seq = 0;
@@ -247,5 +257,12 @@ cudaError_t sw_launch_topk_merge(cudaStream_t st, const unsigned long long *keys
 cudaError_t sw_launch_hits_row(cudaStream_t st, const int32_t *row, uint32_t n, int q, const SwHitList &hl);
 cudaError_t sw_launch_hits_ovf(cudaStream_t st, const unsigned *ovf_count, const uint2 *ovf_list, const int32_t *ovf_score,
                                unsigned ovf_cap, const SwHitList &hl);
+
+/* Per-subject best updates that do not come from the strip epilogue: sbest_row = every entry >= 0 of one
+ * materialised score row of query row q (entries < 0 are skipped: not scored here, or the overflow sentinel) -- the
+ * band-pipelined kernel's rows; sbest_ovf = the overflow-list entries with their exact 32-bit score (ovf_score). */
+cudaError_t sw_launch_sbest_row(cudaStream_t st, const int32_t *row, uint32_t n, int q, const SwSubjectBest &sb);
+cudaError_t sw_launch_sbest_ovf(cudaStream_t st, const unsigned *ovf_count, const uint2 *ovf_list, const int32_t *ovf_score,
+                                unsigned ovf_cap, const SwSubjectBest &sb);
 
 #endif

@@ -54,6 +54,7 @@
 #define SW_OUT_I16  1               /* int16 out[q][subject]                                     */
 #define SW_OUT_TOPK 2               /* no matrix: per-block private top-k lists, merged later    */
 #define SW_OUT_HITS 3               /* no matrix: (row << hits_shift | subject, score) of every score >= min_score */
+#define SW_OUT_SBEST 4              /* no matrix: per subject the best (score, lowest row) and the runner-up score */
 
 /* device-side error word (bit set = which check failed); only written by SW_BOUNDS_CHECK builds
  * and by the wave kernel's spin-wait guard */
@@ -217,6 +218,10 @@ struct StripArgs {
     unsigned long long *hits_count;   // 64-bit: a shard of 10 M subjects x 1 000 rows has 10^10 pairs
     unsigned hits_cap;
     int min_score, hits_shift;
+    // per-subject best (SW_OUT_SBEST, sbest_update): sbest_key[subject] = score << 32 | (0xFFFFFFFF - row) of the
+    // best row so far, sbest_second[subject] = the best score of the other rows, for every pair not on the overflow list
+    unsigned long long *sbest_key;   // null = update nothing (autotune's sample launches)
+    int *sbest_second;               // null = one row only (no runner-up)
 #ifdef SW_BOUNDS_CHECK
     unsigned long long tp_words, bnd_elems, out_elems;
 #endif
@@ -244,6 +249,18 @@ __device__ __forceinline__ bool hits_slots(unsigned long long *count, bool take0
     p0 = base + __popc(b0 & below);
     p1 = base + n0 + __popc(b1 & below);
     return true;
+}
+
+// Per-subject best: the update of one (subject, row) pair.  Keys are score << 32 | (0xFFFFFFFF - row), so the
+// largest key is the best score at its lowest row (key 0 = a phantom row scoring 0).  A key that held the maximum
+// and is displaced reaches `second` through the update that displaced it; any other key reaches it directly.  So
+// `second` ends as the best score of every row but the final best one -- provided each pair arrives exactly once
+// (a pair that arrives twice would set second = best).  second == null: one row, no runner-up.
+__device__ __forceinline__ void sbest_update(unsigned long long *key, int *second, uint32_t s, int row, int score)
+{
+    const unsigned long long k = ((unsigned long long)(uint32_t)score << 32) | (0xFFFFFFFFu - (uint32_t)row);
+    const unsigned long long old = atomicMax(key + s, k);
+    if (second) atomicMax(second + s, k > old ? (int)(old >> 32) : score);
 }
 
 // Column codes: 0..15 = t_lo | t_hi << 2 (both members have a base in this column);
@@ -894,6 +911,19 @@ __global__ void __launch_bounds__(BT, MINB) sw_strip_kernel(const StripArgs a)
                 if (t1 && p1 < a.hits_cap) {
                     SW_CHECK(p1 < a.out_elems, SW_DEVERR_OUT, a);
                     a.hits[p1] = row | subj_hi; a.hits_score[p1] = sc1;
+                }
+            }
+        } else if (a.out_mode == SW_OUT_SBEST) {
+            // flagged pairs are updated from their exact score (sbest_ovf_kernel), never from here; pass-split
+            // parts other than the last left the item above, so each (subject, row) arrives once
+            if (owner && a.sbest_key) {
+                if (!ov0) {
+                    SW_CHECK(subj_lo < a.out_elems, SW_DEVERR_OUT, a);
+                    sbest_update(a.sbest_key, a.sbest_second, subj_lo, eq, sc0);
+                }
+                if (has1 && !ov1) {
+                    SW_CHECK(subj_hi < a.out_elems, SW_DEVERR_OUT, a);
+                    sbest_update(a.sbest_key, a.sbest_second, subj_hi, eq, sc1);
                 }
             }
         } else {
