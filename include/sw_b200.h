@@ -225,6 +225,43 @@ int sw_fetch_subject_best(sw_handle_t *h, int32_t *best_score, uint32_t *best_ro
                           int timeout_ms);
 int sw_fetch_db_subject_best(sw_handle_t *h, int32_t *best_score, uint32_t *best_row, int32_t *second_score, size_t cap);
 
+/* Locate: where the best local alignment of selected (query row, subject) pairs of the resident database begins and
+ * ends, computed on the GPU with two score-only passes per pair (no traceback; DESIGN.md section 5.7).
+ *   Definition.  Take a pair of query row r and subject s.  Let S be its score, which is exactly the int32 matrix
+ *   entry, above 32 767 too.  Use the recurrence of DESIGN section 2 in its explicit form (M, I, G, H), with 1-based
+ *   cells (i, j): i is the query position and j the subject position.
+ *   - End.  Take the cell whose diagonal value M(i, j) equals S and has the smallest j, breaking ties by the
+ *     smallest i.  Then q_end = i and s_end = j.
+ *     - max M == max H for every parameter set validate_params accepts, so this cell always exists.  Gap values
+ *       only ever come from earlier M values plus non-positive penalties.
+ *     - With mismatch <= 0 it is always a matched base pair, also when gap_open + gap_extend == 0.
+ *   - Begin.  Run the same recurrence on reverse(query[0:q_end]) x reverse(subject[0:s_end]) and apply the same rule
+ *     there: the first cell in (column, row) order whose M reaches S.  If that cell is (a, b), then
+ *     q_begin = q_end - a and s_begin = s_end - b.
+ *     - This is the largest s_begin, then the largest q_begin, over the alignments of score S that end at the end
+ *       cell.
+ *     - Because of the end rule, every alignment of score S inside that rectangle ends at the end cell.  So the
+ *       plain local recurrence is exact here: no anchoring or special boundary is needed.
+ *   - Output.  The coordinates are 0-based and half-open, so query[q_begin:q_end] and subject[s_begin:s_end] are
+ *     the aligned stretches.  With mismatch <= 0, query[q_begin] == subject[s_begin] and
+ *     query[q_end-1] == subject[s_end-1].
+ *   - Score 0.  This includes a zero-length query or subject.  The result is (0, 0, 0, 0, 0).
+ *   - Both strands.  When sw_set_strands(h, 1) is on, row nq + i is the reverse complement of query i.  Its q_*
+ *     coordinates are positions in that reverse complement, as it was scored.
+ * Pairs: (row[i], index[i]), index = input index in the database of the last sw_load_db (as sw_fetch_db_hits,
+ * sw_fetch_db_topk and the position in sw_fetch_db_subject_best give it), in any order, repeats allowed.  Blocks
+ * until score[i] and coord[4*i .. 4*i+3] = {q_begin, q_end, s_begin, s_end} are written, in the caller's order.
+ * Each GPU locates the pairs of its own shard; all GPUs run at once.
+ * Errors (nothing is launched): SW_EINVAL for a null handle, null arrays with n > 0, score_width != 0, row >=
+ * sw_query_rows(h) or index >= the database's size; SW_EAGAIN while a batch is in flight; SW_ESTATE when no database
+ * is loaded or sw_score_batch has reused its buffers since the last sw_load_db.  Then n == 0 returns SW_OK.
+ * SW_EDEVICE when sw_device_error_bits is non-zero afterwards.
+ * Other handle state is untouched: the call may follow an unfetched sw_score_db (it queues behind that work), and
+ * the following fetch returns what it would have returned without it; last cells, kernel time and kernel name,
+ * stats, the autotune cache and the output settings keep their values. */
+int sw_locate_db(sw_handle_t *h, const uint32_t *row, const uint64_t *index, size_t n, int32_t *score,
+                 uint32_t *coord /* 4*n: q_begin, q_end, s_begin, s_end */);
+
 /* ---- introspection --------------------------------------------------------- */
 const char *sw_strerror(int code);
 int sw_last_cuda_error(const sw_handle_t *h);          /* cudaError_t as int */

@@ -111,6 +111,7 @@ def load_library():
     L.sw_set_subject_best.argtypes = [vp, i32]
     L.sw_fetch_subject_best.argtypes = [vp, vp, vp, vp, sz, i32]
     L.sw_fetch_db_subject_best.argtypes = [vp, vp, vp, vp, sz]
+    L.sw_locate_db.argtypes = [vp, vp, vp, sz, vp, vp]
     L.sw_device_error_bits.argtypes = [vp]
     L.sw_device_error_bits.restype = C.c_uint
     L.sw_is_check_build.restype = i32
@@ -322,6 +323,19 @@ class Engine:
         bs, br, sec = self._subject_best_arrays(self.ns)
         self._check(self.lib.sw_fetch_db_subject_best(self.h, _ptr(bs), _ptr(br), _ptr(sec), self.ns))
         return bs, br, sec
+
+    def locate_db(self, rows, index):
+        """Where the best local alignment of each (query row, subject) pair of the resident database begins and
+        ends: (score int32[n], coord uint32[n, 4]) with coord = (q_begin, q_end, s_begin, s_end), 0-based and
+        half-open; index = input index in the database of load_db.  The tie rule is in include/sw_b200.h."""
+        rows = np.ascontiguousarray(rows, dtype=np.uint32).reshape(-1)
+        index = np.ascontiguousarray(index, dtype=np.uint64).reshape(-1)
+        if rows.size != index.size:
+            raise ValueError("rows and index differ in length")
+        score = np.empty(rows.size, dtype=np.int32)
+        coord = np.empty((rows.size, 4), dtype=np.uint32)
+        self._check(self.lib.sw_locate_db(self.h, _ptr(rows), _ptr(index), rows.size, _ptr(score), _ptr(coord)))
+        return score, coord
 
     def set_jit(self, mode):
         self._check(self.lib.sw_set_jit(self.h, mode))

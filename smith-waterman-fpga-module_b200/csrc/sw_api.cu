@@ -163,6 +163,8 @@ struct GpuCtx {
     DevBuf d_wave32_bnd, d_wave32_state;   // 32-bit band-pipelined scorer of the overflow list
     DevBuf d_wave_rows;               // top-k / hits / subject-best mode: one scratch score row per band-pipelined query
     DevBuf d_hits_key2, d_hits_score2, d_sort_tmp;   // fetch of a hit list: radix-sort output and temp storage (copy stream)
+    DevBuf d_loc_pair, d_loc_score, d_loc_coord, d_loc_scratch;   // sw_locate_db: pairs, results, (H, G) strip rows
+    PinnedBuf h_loc;                  // sw_locate_db staging: pairs in, scores and coordinates out
     uint32_t wave32_epoch = 0;        // 8-bit tag field: 1 .. 255, boundary rows zeroed when it restarts
     int wave32_bps = 0;
     uint32_t wave_epoch = 0;          // launches so far: the tag of the boundary elements (20 bits)
@@ -179,6 +181,8 @@ struct Batch {
     size_t ns = 0;
     int nq = 0;                       // query rows the scores of this batch have
     bool loaded = false, scored = false, small = false;
+    bool resident = false;            // slot 0 holds the database of the last sw_load_db (no sw_score_batch since)
+    std::vector<uint32_t> lens;       // resident database: subject lengths (sw_locate_db routes and sorts pairs by them)
     // output of the scoring, fixed at submit: SW_OUT_I32 / I16 / TOPK (topk_k lists) / HITS (scores >= hits_min,
     // at most hits_max per GPU) / SBEST (per subject: best score, its row, runner-up score)
     int out_mode = SW_OUT_I32, topk_k = 0;
@@ -294,7 +298,8 @@ std::vector<DevBuf *> all_devbufs(GpuCtx &g)
     std::vector<DevBuf *> v = {&g.d_qpacked, &g.d_qoff, &g.d_qlen, &g.d_qidx, &g.d_bnd, &g.d_counters, &g.d_scratch32,
                                &g.d_best_score, &g.d_best_index, &g.d_topk_keys, &g.d_err, &g.d_wave_bnd, &g.d_wave_state, &g.d_wave32_bnd, &g.d_wave32_state, &g.d_wave_rows,
                                &g.d_bnd_aux[0], &g.d_bnd_aux[1], &g.d_bnd_aux[2], &g.d_part_done, &g.d_part_best,
-                               &g.d_hits_key2, &g.d_hits_score2, &g.d_sort_tmp};
+                               &g.d_hits_key2, &g.d_hits_score2, &g.d_sort_tmp, &g.d_loc_pair, &g.d_loc_score, &g.d_loc_coord,
+                               &g.d_loc_scratch};
     for (Slot &b : g.slot) {
         DevBuf *bufs[] = {&b.d_raw, &b.d_off, &b.d_len, &b.d_pair_subj, &b.d_pair_len, &b.d_tile_woff, &b.d_tp, &b.d_out,
                           &b.d_ovf_count, &b.d_ovf_list, &b.d_ovf_score, &b.d_topk_out, &b.d_small_in, &b.d_small_done,
@@ -319,6 +324,7 @@ void free_gpu(GpuCtx &g)
         if (b.ev_stop) cudaEventDestroy(b.ev_stop);
         if (b.ev_upload) cudaEventDestroy(b.ev_upload);
     }
+    g.h_loc.release();
     for (cudaStream_t st : g.st_aux) if (st) cudaStreamDestroy(st);
     if (g.ev_fork) cudaEventDestroy(g.ev_fork);
     for (cudaEvent_t e : g.ev_join) if (e) cudaEventDestroy(e);
@@ -1935,7 +1941,7 @@ int load_batch(sw_handle *h, int si, const uint8_t *packed, const uint32_t *len,
 {
     const auto t_load0 = std::chrono::steady_clock::now();
     Batch &bt = h->batch[si];
-    bt.ns = ns; bt.loaded = false; bt.scored = false; bt.cells = 0; bt.small = false;
+    bt.ns = ns; bt.loaded = false; bt.scored = false; bt.cells = 0; bt.small = false; bt.resident = false;
     bt.have_ids = ids != nullptr;
     if (ids) bt.ids.assign(ids, ids + ns); else bt.ids.clear();
     const size_t ng = h->gpus.size();
@@ -2203,6 +2209,84 @@ int fetch_common(sw_handle_t *h, FetchKind kind, void *scores, uint64_t *index, 
     return pop_fifo(h, fetch_slot(h, h->fifo[0], kind, scores, index, cap, timeout_ms));
 }
 
+// sw_locate_db: the scratch of one launch, 2 * (longest subject) * threads int32, stays within the 32-bit scorer's
+// budget; the thread count is capped to fit.
+constexpr size_t kLocateScratchBytes = size_t(1) << 30;
+
+// Routes each pair to the GPU whose shard holds its subject (pairs with an empty query or subject score 0 here),
+// sorts every GPU's pairs by descending cells so that the threads of a warp get similar lengths, runs all GPUs at
+// once on their compute streams (behind any scoring still queued there) and scatters the results into the caller's
+// order.  The arguments are validated by sw_locate_db.
+int locate_pairs(sw_handle *h, const uint32_t *row, const uint64_t *index, size_t n, int32_t *score, uint32_t *coord)
+{
+    const Batch &bt = h->batch[0];
+    const size_t ng = h->gpus.size();
+    std::vector<std::vector<std::pair<uint64_t, size_t>>> work(ng);     // (cells, position in the caller's arrays)
+    for (size_t i = 0; i < n; ++i) {
+        const uint64_t cells = (uint64_t)h->q_len[row[i]] * bt.lens[index[i]];
+        if (cells == 0) { score[i] = 0; std::memset(coord + 4 * i, 0, 4 * sizeof(uint32_t)); continue; }
+        size_t gi = 0;
+        while (h->gpus[gi].slot[0].s1 <= index[i]) ++gi;
+        work[gi].emplace_back(cells, i);
+    }
+    const SwScoring sc = scoring_of(h);
+    for (size_t gi = 0; gi < ng; ++gi) {
+        auto &w = work[gi];
+        if (w.empty()) continue;
+        GpuCtx &gc = h->gpus[gi];
+        Slot &g = gc.slot[0];
+        std::sort(w.begin(), w.end(), [](const std::pair<uint64_t, size_t> &a, const std::pair<uint64_t, size_t> &b) {
+            return a.first != b.first ? a.first > b.first : a.second < b.second;
+        });
+        const size_t m = w.size();
+        uint32_t max_cols = 0;
+        for (const auto &p : w) max_cols = std::max(max_cols, bt.lens[index[p.second]]);
+        const size_t fit = kLocateScratchBytes / (2 * sizeof(int32_t) * (size_t)max_cols) / 128 * 128;
+        const size_t threads = std::max<size_t>(128, std::min((m + 127) / 128 * 128, fit));
+        SW_CUDA(h, cudaSetDevice(gc.dev));
+        // staging: [m pairs {row, shard-local subject}][m scores][m coordinate quadruples]
+        SW_CUDA(h, gc.h_loc.reserve(m * (sizeof(uint2) + sizeof(int32_t) + sizeof(uint4))));
+        uint2 *hp = (uint2 *)gc.h_loc.p;
+        for (size_t k = 0; k < m; ++k) hp[k] = make_uint2(row[w[k].second], (uint32_t)(index[w[k].second] - g.s0));
+        SW_CUDA(h, gc.d_loc_pair.reserve(m * sizeof(uint2)));
+        SW_CUDA(h, gc.d_loc_score.reserve(m * sizeof(int32_t)));
+        SW_CUDA(h, gc.d_loc_coord.reserve(m * sizeof(uint4)));
+        SW_CUDA(h, gc.d_loc_scratch.reserve(2 * sizeof(int32_t) * (size_t)max_cols * threads));
+        SW_CUDA(h, cudaMemcpyAsync(gc.d_loc_pair.p, hp, m * sizeof(uint2), cudaMemcpyHostToDevice, gc.st_compute));
+        SwLocateLaunch L;
+        L.db = dev_db(g); L.raw_bytes = g.d_raw.cap;
+        L.q = dev_queries(h, gc); L.q_bytes = gc.d_qpacked.cap;
+        L.sc = sc;
+        L.pairs = gc.d_loc_pair.as<uint2>(); L.npairs = (uint32_t)m;
+        L.score = gc.d_loc_score.as<int32_t>(); L.coord = gc.d_loc_coord.as<uint4>(); L.out_elems = m;
+        L.scratch = gc.d_loc_scratch.as<int32_t>(); L.max_cols = max_cols;
+        L.threads_total = (int)threads;
+        L.dev_err = gc.d_err.as<unsigned>();
+        SW_CUDA(h, sw_launch_locate(gc.st_compute, L));
+        h->launches++;
+        SW_CUDA(h, cudaMemcpyAsync((char *)gc.h_loc.p + m * sizeof(uint2), gc.d_loc_score.p, m * sizeof(int32_t),
+                                   cudaMemcpyDeviceToHost, gc.st_compute));
+        SW_CUDA(h, cudaMemcpyAsync((char *)gc.h_loc.p + m * (sizeof(uint2) + sizeof(int32_t)), gc.d_loc_coord.p,
+                                   m * sizeof(uint4), cudaMemcpyDeviceToHost, gc.st_compute));
+    }
+    for (size_t gi = 0; gi < ng; ++gi) {
+        const auto &w = work[gi];
+        if (w.empty()) continue;
+        GpuCtx &gc = h->gpus[gi];
+        SW_CUDA(h, cudaSetDevice(gc.dev));
+        SW_CUDA(h, cudaStreamSynchronize(gc.st_compute));
+        const size_t m = w.size();
+        const int32_t *hs = (const int32_t *)((const char *)gc.h_loc.p + m * sizeof(uint2));
+        const uint32_t *hc = (const uint32_t *)(hs + m);
+        for (size_t k = 0; k < m; ++k) {
+            score[w[k].second] = hs[k];
+            std::memcpy(coord + 4 * w[k].second, hc + 4 * k, 4 * sizeof(uint32_t));
+        }
+    }
+    if (device_error_bits(h)) return SW_EDEVICE;
+    return SW_OK;
+}
+
 }  // namespace
 
 // ================================================================================================
@@ -2428,6 +2512,20 @@ int sw_fetch_db_subject_best(sw_handle_t *h, int32_t *best_score, uint32_t *best
     return fetch_sbest_slot(h, 0, best_score, best_row, second_score, cap, -1);
 }
 
+int sw_locate_db(sw_handle_t *h, const uint32_t *row, const uint64_t *index, size_t n, int32_t *score, uint32_t *coord)
+{
+    // coordinates of the wrapping 12-bit machine are not defined
+    if (!h || (n > 0 && (!row || !index || !score || !coord)) || h->params.score_width != 0) return SW_EINVAL;
+    if (h->n_inflight) return SW_EAGAIN;
+    const Batch &bt = h->batch[0];
+    if (!bt.loaded || !bt.resident) return SW_ESTATE;
+    const size_t rows = h->q_len.size();
+    for (size_t i = 0; i < n; ++i)
+        if (row[i] >= rows || index[i] >= bt.ns) return SW_EINVAL;
+    if (n == 0) return SW_OK;
+    return locate_pairs(h, row, index, n, score, coord);
+}
+
 int sw_set_queries(sw_handle_t *h, const uint8_t *packed, const uint32_t *len, const uint64_t *off, int nq)
 {
     if (!h || nq < 0 || (nq > 0 && (!packed || !len || !off))) return SW_EINVAL;
@@ -2492,7 +2590,10 @@ int sw_load_db(sw_handle_t *h, const uint8_t *packed, const uint32_t *len, const
 {
     if (!h || (ns > 0 && (!packed || !len || !off))) return SW_EINVAL;
     if (h->n_inflight) return SW_EAGAIN;
-    return load_batch(h, 0, packed, len, off, ids, ns);
+    SW_TRY(load_batch(h, 0, packed, len, off, ids, ns));
+    h->batch[0].lens.assign(len, len + ns);
+    h->batch[0].resident = true;
+    return SW_OK;
 }
 
 int sw_score_db(sw_handle_t *h)
@@ -2533,6 +2634,7 @@ int sw_score_batch(sw_handle_t *h, const uint8_t *packed, const uint32_t *len, c
     if (mode_needs_strip(h)) return SW_EINVAL;
     // take the slot that is not in flight; this replaces whatever sw_load_db left there
     const int si = (h->n_inflight == 1) ? (1 - h->fifo[0]) : 0;
+    h->batch[si].resident = false;
     bool taken = false;
     SW_TRY(small_submit(h, si, packed, len, off, ids, ns, &taken));
     if (!taken) {

@@ -4,14 +4,17 @@
  *
  *   sw_b200_cli -q query.fa -l library.fa [-t seconds] [-o out.txt] [-R score.txt]
  *               [-m match] [-x mismatch] [-g gap_open] [-e gap_extend] [-w score_width] [-G ngpus]
- *               [-T min_score] [-B]
+ *               [-T min_score] [-B] [-L]
  *
  * Without -o / -R it prints, like main_test, "result: %d, biased: %d" for every pair
  * (biased = score + 2048, the RTL's ZERO offset).  -T scores in hit-list mode (sw_set_hits) and prints
  * those lines only for the pairs scoring at least min_score; -o / -R list every subject, so they do
  * not combine with it.  -B scores in subject-best mode (sw_set_subject_best) and prints one line per
  * subject, "<subject> best <query> result: %d, second: %d" (second = -1 with one query); it combines
- * with none of -o / -R / -T.
+ * with none of -o / -R / -T.  -L (with -T or -B only) scores the library as a resident database
+ * (sw_load_db, sw_score_db) and appends to each of those lines where the best alignment of the pair lies
+ * (sw_locate_db), 1-based and inclusive like ssearch36 prints it: " query %u-%u subject %u-%u"
+ * (0-0 for a score of 0).
  */
 #include "../../include/sw_b200.h"
 
@@ -23,25 +26,32 @@ static void usage(const char *n)
 {
     fprintf(stderr, "Usage: %s -q <query.fa> -l <library.fa> [-t timeout_s] [-o out.txt] [-R score.txt]\n"
                     "          [-m match] [-x mismatch] [-g gap_open] [-e gap_extend] [-w score_width] [-G ngpus]\n"
-                    "          [-T min_score] [-B]\n", n);
+                    "          [-T min_score] [-B] [-L]\n", n);
+}
+
+/* " query b-e subject b-e" of a located pair: 1-based, inclusive; 0-0 for a score of 0 */
+static void print_span(int32_t score, const uint32_t *c)
+{
+    if (score > 0) printf(" query %u-%u subject %u-%u", c[0] + 1, c[1], c[2] + 1, c[3]);
+    else printf(" query 0-0 subject 0-0");
 }
 
 int main(int argc, char **argv)
 {
     const char *qf = NULL, *lf = NULL, *of = NULL, *rf = NULL;
-    int timeout_s = 10, ngpus = 1, opt, rc, i, min_score = 0, subject_best = 0;
+    int timeout_s = 10, ngpus = 1, opt, rc, i, min_score = 0, subject_best = 0, locate = 0;
     sw_params_t p;
     sw_handle_t *h = NULL;
     sw_seqset_t *q = NULL, *db = NULL;
-    int32_t *scores = NULL, *hscore = NULL, *bscore = NULL, *bsecond = NULL;
-    uint32_t *hrow = NULL, *brow = NULL;
-    uint64_t *hindex = NULL;
+    int32_t *scores = NULL, *hscore = NULL, *bscore = NULL, *bsecond = NULL, *lscore = NULL;
+    uint32_t *hrow = NULL, *brow = NULL, *lcoord = NULL;
+    uint64_t *hindex = NULL, *bindex = NULL;
     size_t nhits = 0;
     int gpu_ids[64];
     static struct option lo[] = {{"timeout", required_argument, 0, 't'}, {"query", required_argument, 0, 'q'},
                                  {"library", required_argument, 0, 'l'}, {"help", no_argument, 0, 'h'}, {0, 0, 0, 0}};
     sw_default_params(&p);
-    while ((opt = getopt_long(argc, argv, "ht:q:l:o:R:m:x:g:e:w:G:T:B", lo, NULL)) >= 0) {
+    while ((opt = getopt_long(argc, argv, "ht:q:l:o:R:m:x:g:e:w:G:T:BL", lo, NULL)) >= 0) {
         switch (opt) {
             case 'q': qf = optarg; break;
             case 'l': lf = optarg; break;
@@ -56,6 +66,7 @@ int main(int argc, char **argv)
             case 'G': ngpus = atoi(optarg); break;
             case 'T': min_score = atoi(optarg); break;
             case 'B': subject_best = 1; break;
+            case 'L': locate = 1; break;
             case 'h': usage(argv[0]); return 0;
             default: usage(argv[0]); return -1;
         }
@@ -68,6 +79,11 @@ int main(int argc, char **argv)
     }
     if (subject_best && (of || rf || min_score > 0)) {
         printf("-B prints each subject's best query only: it does not combine with -o / -R / -T\n");
+        usage(argv[0]);
+        return -1;
+    }
+    if (locate && min_score <= 0 && !subject_best) {
+        printf("-L locates the pairs -T or -B prints: it needs one of them\n");
         usage(argv[0]);
         return -1;
     }
@@ -85,21 +101,37 @@ int main(int argc, char **argv)
     }
     if (subject_best && (rc = sw_set_subject_best(h, 1)) != SW_OK) goto fail;
     if ((rc = sw_set_queries(h, q->packed, q->len, q->off, (int)q->n)) != SW_OK) goto fail;
-    if ((rc = sw_score_batch(h, db->packed, db->len, db->off, NULL, db->n)) != SW_OK) goto fail;
+    if (locate) {
+        /* sw_locate_db reads the resident database */
+        if ((rc = sw_load_db(h, db->packed, db->len, db->off, NULL, db->n)) != SW_OK) goto fail;
+        if ((rc = sw_score_db(h)) != SW_OK) goto fail;
+        if ((rc = sw_wait(h, timeout_s * 1000)) != SW_OK) goto fail;
+    } else if ((rc = sw_score_batch(h, db->packed, db->len, db->off, NULL, db->n)) != SW_OK) goto fail;
     if (min_score > 0) {
-        rc = sw_fetch_hits(h, NULL, NULL, NULL, 0, &nhits, timeout_s * 1000);       /* size query */
+        /* size query */
+        rc = locate ? sw_fetch_db_hits(h, NULL, NULL, NULL, 0, &nhits) : sw_fetch_hits(h, NULL, NULL, NULL, 0, &nhits, timeout_s * 1000);
         if (rc == SW_ECAPACITY) {
             hrow = (uint32_t *)malloc(nhits * sizeof *hrow);
             hindex = (uint64_t *)malloc(nhits * sizeof *hindex);
             hscore = (int32_t *)malloc(nhits * sizeof *hscore);
             if (!hrow || !hindex || !hscore) { rc = SW_ENOMEM; goto fail; }
-            rc = sw_fetch_hits(h, hrow, hindex, hscore, nhits, &nhits, timeout_s * 1000);
+            rc = locate ? sw_fetch_db_hits(h, hrow, hindex, hscore, nhits, &nhits)
+                        : sw_fetch_hits(h, hrow, hindex, hscore, nhits, &nhits, timeout_s * 1000);
         }
         if (rc != SW_OK) goto fail;
-        for (i = 0; (size_t)i < nhits; ++i)
-            printf("%s x %s result: %d, biased: %d(0x%04x)\n", q->name[hrow[i]], db->name[hindex[i]],
+        if (locate) {
+            lscore = (int32_t *)malloc((nhits + 1) * sizeof *lscore);
+            lcoord = (uint32_t *)malloc((nhits + 1) * 4 * sizeof *lcoord);
+            if (!lscore || !lcoord) { rc = SW_ENOMEM; goto fail; }
+            if ((rc = sw_locate_db(h, hrow, hindex, nhits, lscore, lcoord)) != SW_OK) goto fail;
+        }
+        for (i = 0; (size_t)i < nhits; ++i) {
+            printf("%s x %s result: %d, biased: %d(0x%04x)", q->name[hrow[i]], db->name[hindex[i]],
                    (int)hscore[i], (int)hscore[i] + 2048, (unsigned)(hscore[i] + 2048));
-        free(hrow); free(hindex); free(hscore); sw_destroy(h); sw_seqset_free(q); sw_seqset_free(db);
+            if (locate) print_span(lscore[i], lcoord + 4 * (size_t)i);
+            printf("\n");
+        }
+        free(hrow); free(hindex); free(hscore); free(lscore); free(lcoord); sw_destroy(h); sw_seqset_free(q); sw_seqset_free(db);
         return 0;
     }
     if (subject_best) {
@@ -107,10 +139,23 @@ int main(int argc, char **argv)
         bsecond = (int32_t *)malloc((db->n + 1) * sizeof *bsecond);
         brow = (uint32_t *)malloc((db->n + 1) * sizeof *brow);
         if (!bscore || !bsecond || !brow) { rc = SW_ENOMEM; goto fail; }
-        if ((rc = sw_fetch_subject_best(h, bscore, brow, bsecond, db->n, timeout_s * 1000)) != SW_OK) goto fail;
-        for (i = 0; (size_t)i < db->n; ++i)
-            printf("%s best %s result: %d, second: %d\n", db->name[i], q->name[brow[i]], (int)bscore[i], (int)bsecond[i]);
-        free(bscore); free(bsecond); free(brow); sw_destroy(h); sw_seqset_free(q); sw_seqset_free(db);
+        rc = locate ? sw_fetch_db_subject_best(h, bscore, brow, bsecond, db->n)
+                    : sw_fetch_subject_best(h, bscore, brow, bsecond, db->n, timeout_s * 1000);
+        if (rc != SW_OK) goto fail;
+        if (locate) {
+            bindex = (uint64_t *)malloc((db->n + 1) * sizeof *bindex);
+            lscore = (int32_t *)malloc((db->n + 1) * sizeof *lscore);
+            lcoord = (uint32_t *)malloc((db->n + 1) * 4 * sizeof *lcoord);
+            if (!bindex || !lscore || !lcoord) { rc = SW_ENOMEM; goto fail; }
+            for (i = 0; (size_t)i < db->n; ++i) bindex[i] = (uint64_t)i;
+            if ((rc = sw_locate_db(h, brow, bindex, db->n, lscore, lcoord)) != SW_OK) goto fail;
+        }
+        for (i = 0; (size_t)i < db->n; ++i) {
+            printf("%s best %s result: %d, second: %d", db->name[i], q->name[brow[i]], (int)bscore[i], (int)bsecond[i]);
+            if (locate) print_span(lscore[i], lcoord + 4 * (size_t)i);
+            printf("\n");
+        }
+        free(bscore); free(bsecond); free(brow); free(bindex); free(lscore); free(lcoord); sw_destroy(h); sw_seqset_free(q); sw_seqset_free(db);
         return 0;
     }
     scores = (int32_t *)calloc(q->n * db->n + 1, sizeof(int32_t));
@@ -145,6 +190,7 @@ fail:
     printf("error: %s", sw_strerror(rc));
     if (rc == SW_ECUDA) printf(" [%s]", sw_last_cuda_error_string(h));
     printf("\n");
-    free(scores); free(hrow); free(hindex); free(hscore); free(bscore); free(bsecond); free(brow); sw_destroy(h); sw_seqset_free(q); sw_seqset_free(db);
+    free(scores); free(hrow); free(hindex); free(hscore); free(bscore); free(bsecond); free(brow); free(bindex); free(lscore); free(lcoord);
+    sw_destroy(h); sw_seqset_free(q); sw_seqset_free(db);
     return -1;
 }

@@ -235,6 +235,28 @@ struct SwScore32Launch {
 };
 cudaError_t sw_launch_score32(cudaStream_t st, const SwScore32Launch &L);
 
+/* Begin / end of the best local alignment of selected pairs (sw_locate.cu, sw_locate_db): one thread per entry of
+ * pairs[0 .. npairs) = {query row, shard-local subject}; score[i] = its score, coord[i] = {q_begin, q_end, s_begin,
+ * s_end}.  scratch: 2 * max_cols * threads_total int32, max_cols >= the longest subject of the pairs.  raw_bytes /
+ * q_bytes / out_elems: sizes of db.raw, q.packed and the two result arrays (bounds-check build).  Exact scores only (sc.limit is ignored). */
+struct SwLocateLaunch {
+    SwDevDb db{};
+    size_t raw_bytes = 0;
+    SwDevQueries q{};
+    size_t q_bytes = 0;
+    SwScoring sc{};
+    const uint2 *pairs = nullptr;
+    uint32_t npairs = 0;
+    int32_t *score = nullptr;
+    uint4 *coord = nullptr;
+    size_t out_elems = 0;
+    int32_t *scratch = nullptr;
+    uint32_t max_cols = 0;
+    int threads_total = 0;
+    unsigned *dev_err = nullptr;
+};
+cudaError_t sw_launch_locate(cudaStream_t st, const SwLocateLaunch &L);
+
 cudaError_t sw_launch_build_tp(cudaStream_t st, const SwDevDb &db);
 
 /* Per-query arg-max over subjects of a materialised int32 matrix (first index reaching the max). */
