@@ -262,6 +262,44 @@ int sw_fetch_db_subject_best(sw_handle_t *h, int32_t *best_score, uint32_t *best
 int sw_locate_db(sw_handle_t *h, const uint32_t *row, const uint64_t *index, size_t n, int32_t *score,
                  uint32_t *coord /* 4*n: q_begin, q_end, s_begin, s_end */);
 
+/* Align: how the located alignment of selected pairs aligns, as a CIGAR, traced back on the GPU (DESIGN.md
+ * section 5.8).  Pairs, validation, score and coord are exactly sw_locate_db's for the same pairs.
+ *   Definition.  Let S, qb, qe, sb, se be the located result, with S > 0.  Run the recurrence of DESIGN section 2 in
+ *   its explicit form (M, I, G, H), local with the 0 clamp and locate's boundaries, over query[qb:qe] x
+ *   subject[sb:se], with 1-based rectangle cells (i, j).  Every cell records:
+ *   - h: H came from M if M >= I, else from I (a tie goes to M);
+ *   - u: I came from up, G(i-1, j), if G(i-1, j) >= G(i, j-1), else from the left (a tie goes to up);
+ *   - g: G was an open, M + go + ge, if M + go + ge >= I + ge, else an extend (a tie goes to open).
+ *   The walk starts at (qe-qb, se-sb) in state M.  In M it emits one '=' or 'X' column, stops at (1, 1), and
+ *   otherwise goes to (i-1, j-1) in the state h names there.  In I it follows u: up emits 'I' (a query base against
+ *   a gap), left emits 'D' (a subject base against a gap); at the cell it lands on it takes state M if g says open,
+ *   else stays in I.
+ *   - The walk always ends at (1, 1) in state M.  An earlier start would be an alignment of score S with a larger
+ *     s_begin, or the same s_begin and a larger q_begin, and locate's begin rule excludes both.
+ *   - It consumes exactly query[qb:qe] and subject[sb:se].
+ *   - It scores S under the engine's gap model, the combined I of DESIGN section 2: a maximal run of I / D columns,
+ *     in any mix, costs gap_open + gap_extend * length.  This is not Gotoh: an I run directly next to a D run is
+ *     priced as one gap.
+ *   - With mismatch <= 0 the first and last ops are '='.
+ *   - Walking back from the end it prefers the diagonal, so indels sit as far left as the score allows: a one-base
+ *     indel in a homopolymer run lands on the run's first base.
+ * Encoding: BAM's, one uint32 per maximal run, len << 4 | op with op 1 = 'I', 2 = 'D', 7 = '=', 8 = 'X'.  The query
+ * plays SAM's read and the subject SAM's reference.  Pair i's ops are cigar[cigar_off[i] .. cigar_off[i+1]), with
+ * cigar_off[0] = 0 (n + 1 entries).  Score 0, which includes an empty query or subject, gives no ops.  With both
+ * strands, row nq + i is aligned as it was scored: as the reverse complement of query i.
+ * Capacity: *count = the total number of ops.  If cap < *count the call returns SW_ECAPACITY and writes only
+ * *count; the call keeps no state, so a retry recomputes.  cap = 0 with cigar = NULL is the size query.  A pair needs
+ * at most (qe-qb) + (se-sb) - 1 ops, so cap = sum over the pairs of (row length + subject length) always suffices.
+ * Traceback storage: 4 bits per cell in device memory, 1 GB per GPU unless SW_B200_ALIGN_SCRATCH_MB (read at sw_init)
+ * says otherwise; pairs run in rounds that fit it.  A pair whose rectangle alone needs more (at the default, more than
+ * 2^31 cells, about a 46 kb x 46 kb rectangle) fails the whole call with SW_ERANGE before anything is written.
+ * Errors: sw_locate_db's (nothing is launched), and SW_EINVAL also for a null cigar_off or count with n > 0 or a null
+ * cigar with cap > 0.  With n == 0 it writes cigar_off[0] = 0 and *count = 0 where given.  Other handle state is
+ * untouched, exactly as for sw_locate_db. */
+int sw_align_db(sw_handle_t *h, const uint32_t *row, const uint64_t *index, size_t n, int32_t *score,
+                uint32_t *coord /* 4*n, as sw_locate_db */, uint64_t *cigar_off /* n + 1 */, uint32_t *cigar,
+                size_t cap, size_t *count);
+
 /* ---- introspection --------------------------------------------------------- */
 const char *sw_strerror(int code);
 int sw_last_cuda_error(const sw_handle_t *h);          /* cudaError_t as int */

@@ -112,6 +112,7 @@ def load_library():
     L.sw_fetch_subject_best.argtypes = [vp, vp, vp, vp, sz, i32]
     L.sw_fetch_db_subject_best.argtypes = [vp, vp, vp, vp, sz]
     L.sw_locate_db.argtypes = [vp, vp, vp, sz, vp, vp]
+    L.sw_align_db.argtypes = [vp, vp, vp, sz, vp, vp, vp, vp, sz, vp]
     L.sw_device_error_bits.argtypes = [vp]
     L.sw_device_error_bits.restype = C.c_uint
     L.sw_is_check_build.restype = i32
@@ -165,6 +166,8 @@ class Engine:
         self.hits = 0        # min_score of the hit-list mode (0 = off)
         self.subject_best = False
         self._ids_ns = 0     # subjects of the batch sw_fetch_ids refers to (last loaded / fetched)
+        self._qlen = np.zeros(0, np.uint64)    # query lengths of set_queries (row nq + i has query i's length)
+        self._db_len = np.zeros(0, np.uint64)  # subject lengths of load_db (align_db sizes its CIGAR buffer with both)
 
     # -- plumbing ---------------------------------------------------------------------
     def _check(self, rc):
@@ -208,6 +211,7 @@ class Engine:
         packed, ln, off = self._as_packed(queries)
         self._check(self.lib.sw_set_queries(self.h, _ptr(packed), _ptr(ln), _ptr(off), len(ln)))
         self.nq = int(self.lib.sw_query_rows(self.h))
+        self._qlen = ln.astype(np.uint64)
 
     def score_batch(self, subjects, ids=None):
         packed, ln, off = self._as_packed(subjects)
@@ -337,6 +341,31 @@ class Engine:
         self._check(self.lib.sw_locate_db(self.h, _ptr(rows), _ptr(index), rows.size, _ptr(score), _ptr(coord)))
         return score, coord
 
+    def align_db(self, rows, index):
+        """The CIGAR of each pair's located alignment: (score int32[n], coord uint32[n, 4], cigar_off uint64[n + 1],
+        cigar uint32[...]), with score and coord as locate_db gives them and pair i's BAM-encoded ops (len << 4 | op)
+        in cigar[cigar_off[i]:cigar_off[i + 1]]; cigar_str turns them into text.  The walk's tie rules are in
+        include/sw_b200.h.  One call: the buffer holds sum(row length + subject length), which always suffices."""
+        rows = np.ascontiguousarray(rows, dtype=np.uint32).reshape(-1)
+        index = np.ascontiguousarray(index, dtype=np.uint64).reshape(-1)
+        if rows.size != index.size:
+            raise ValueError("rows and index differ in length")
+        n = rows.size
+        score = np.empty(n, dtype=np.int32)
+        coord = np.empty((n, 4), dtype=np.uint32)
+        cigar_off = np.empty(n + 1, dtype=np.uint64)
+        cap = 0
+        if n and self._qlen.size and self._db_len.size:
+            # out-of-range rows or indices only mis-size the buffer: the library rejects them
+            qlen = self._qlen[rows % self._qlen.size]
+            slen = np.take(self._db_len, index.astype(np.int64), mode="clip")
+            cap = int(qlen.sum(dtype=np.uint64)) + int(slen.sum(dtype=np.uint64))
+        cigar = np.empty(cap, dtype=np.uint32)
+        count = C.c_size_t(0)
+        self._check(self.lib.sw_align_db(self.h, _ptr(rows), _ptr(index), n, _ptr(score), _ptr(coord), _ptr(cigar_off),
+                                         _ptr(cigar) if cap else None, cap, C.byref(count)))
+        return score, coord, cigar_off, cigar[:count.value]
+
     def set_jit(self, mode):
         self._check(self.lib.sw_set_jit(self.h, mode))
 
@@ -391,6 +420,7 @@ class Engine:
         self._check(self.lib.sw_load_db(self.h, _ptr(packed), _ptr(ln), _ptr(off), _ptr(ids_a), len(ln)))
         self.ns = len(ln)
         self._ids_ns = len(ln)
+        self._db_len = ln.astype(np.uint64)
 
     def score_db(self):
         self._check(self.lib.sw_score_db(self.h))
@@ -443,6 +473,17 @@ class Engine:
     @property
     def last_kernel_name(self):
         return self.lib.sw_last_kernel_name(self.h).decode()
+
+
+CIGAR_OPS = "MIDNSHP=X"      # BAM op codes 0 .. 8
+
+
+def cigar_str(ops):
+    """SAM text of BAM-encoded ops (len << 4 | op), e.g. "23=1I24="; "*" for no ops."""
+    ops = np.asarray(ops, dtype=np.uint32).reshape(-1)
+    if ops.size == 0:
+        return "*"
+    return "".join(f"{int(o) >> 4}{CIGAR_OPS[int(o) & 15]}" for o in ops)
 
 
 def kernel_variants():

@@ -165,6 +165,8 @@ struct GpuCtx {
     DevBuf d_hits_key2, d_hits_score2, d_sort_tmp;   // fetch of a hit list: radix-sort output and temp storage (copy stream)
     DevBuf d_loc_pair, d_loc_score, d_loc_coord, d_loc_scratch;   // sw_locate_db: pairs, results, (H, G) strip rows
     PinnedBuf h_loc;                  // sw_locate_db staging: pairs in, scores and coordinates out
+    DevBuf d_aln_off, d_aln_trace, d_aln_ops, d_aln_nops;   // sw_align_db: per-pair offsets, direction bits, ops, op counts
+    PinnedBuf h_aln;                  // sw_align_db staging: offsets in, op counts and ops out
     uint32_t wave32_epoch = 0;        // 8-bit tag field: 1 .. 255, boundary rows zeroed when it restarts
     int wave32_bps = 0;
     uint32_t wave_epoch = 0;          // launches so far: the tag of the boundary elements (20 bits)
@@ -240,6 +242,7 @@ struct sw_handle {
     int sticky = -1;                  // 0 = super-block order; > 0 = sticky order with this drift bound in pair blocks;
                                       // -1 = sticky order, drift bound of about 1 MB of code stream (4 .. 32 pair blocks)
     double superblock_mb = 24.0;      // code-stream bytes of one super-block
+    size_t align_scratch = size_t(1) << 30;   // sw_align_db: direction-bit bytes per GPU and round (SW_B200_ALIGN_SCRATCH_MB)
     int pass_split = -1;              // pass split of long queries with few work items: 0 never, -1 automatic,
                                       // n > 1 = about n parts whenever the query has that many profile chunks (A/B, tests)
     // bookkeeping
@@ -299,7 +302,7 @@ std::vector<DevBuf *> all_devbufs(GpuCtx &g)
                                &g.d_best_score, &g.d_best_index, &g.d_topk_keys, &g.d_err, &g.d_wave_bnd, &g.d_wave_state, &g.d_wave32_bnd, &g.d_wave32_state, &g.d_wave_rows,
                                &g.d_bnd_aux[0], &g.d_bnd_aux[1], &g.d_bnd_aux[2], &g.d_part_done, &g.d_part_best,
                                &g.d_hits_key2, &g.d_hits_score2, &g.d_sort_tmp, &g.d_loc_pair, &g.d_loc_score, &g.d_loc_coord,
-                               &g.d_loc_scratch};
+                               &g.d_loc_scratch, &g.d_aln_off, &g.d_aln_trace, &g.d_aln_ops, &g.d_aln_nops};
     for (Slot &b : g.slot) {
         DevBuf *bufs[] = {&b.d_raw, &b.d_off, &b.d_len, &b.d_pair_subj, &b.d_pair_len, &b.d_tile_woff, &b.d_tp, &b.d_out,
                           &b.d_ovf_count, &b.d_ovf_list, &b.d_ovf_score, &b.d_topk_out, &b.d_small_in, &b.d_small_done,
@@ -325,6 +328,7 @@ void free_gpu(GpuCtx &g)
         if (b.ev_upload) cudaEventDestroy(b.ev_upload);
     }
     g.h_loc.release();
+    g.h_aln.release();
     for (cudaStream_t st : g.st_aux) if (st) cudaStreamDestroy(st);
     if (g.ev_fork) cudaEventDestroy(g.ev_fork);
     for (cudaEvent_t e : g.ev_join) if (e) cudaEventDestroy(e);
@@ -2213,25 +2217,32 @@ int fetch_common(sw_handle_t *h, FetchKind kind, void *scores, uint64_t *index, 
 // budget; the thread count is capped to fit.
 constexpr size_t kLocateScratchBytes = size_t(1) << 30;
 
-// Routes each pair to the GPU whose shard holds its subject (pairs with an empty query or subject score 0 here),
-// sorts every GPU's pairs by descending cells so that the threads of a warp get similar lengths, runs all GPUs at
-// once on their compute streams (behind any scoring still queued there) and scatters the results into the caller's
-// order.  The arguments are validated by sw_locate_db.
-int locate_pairs(sw_handle *h, const uint32_t *row, const uint64_t *index, size_t n, int32_t *score, uint32_t *coord)
+// One GPU's share of a sw_locate_db / sw_align_db call.
+struct LocateWork {
+    std::vector<std::pair<uint64_t, size_t>> w;   // (cells, position in the caller's arrays), descending cells
+    size_t fit = 0;                   // most threads whose (H, G) scratch stays within kLocateScratchBytes
+    SwLocateLaunch L;                 // the locate launch; sw_align_db's launches reuse its pairs, results and scratch
+};
+
+// Routes each pair to the GPU whose shard holds its subject (pairs with an empty query or subject are left out: they
+// score 0), sorts every GPU's pairs by descending cells so that the threads of a warp get similar lengths, and
+// enqueues the locate launch on every GPU at once on its compute stream (behind any scoring still queued there),
+// followed by the copies of its scores and coordinates to h_loc.  The arguments are validated by the caller.
+int enqueue_locate(sw_handle *h, const uint32_t *row, const uint64_t *index, size_t n, std::vector<LocateWork> &work)
 {
     const Batch &bt = h->batch[0];
     const size_t ng = h->gpus.size();
-    std::vector<std::vector<std::pair<uint64_t, size_t>>> work(ng);     // (cells, position in the caller's arrays)
+    work.assign(ng, LocateWork());
     for (size_t i = 0; i < n; ++i) {
         const uint64_t cells = (uint64_t)h->q_len[row[i]] * bt.lens[index[i]];
-        if (cells == 0) { score[i] = 0; std::memset(coord + 4 * i, 0, 4 * sizeof(uint32_t)); continue; }
+        if (cells == 0) continue;
         size_t gi = 0;
         while (h->gpus[gi].slot[0].s1 <= index[i]) ++gi;
-        work[gi].emplace_back(cells, i);
+        work[gi].w.emplace_back(cells, i);
     }
     const SwScoring sc = scoring_of(h);
     for (size_t gi = 0; gi < ng; ++gi) {
-        auto &w = work[gi];
+        auto &w = work[gi].w;
         if (w.empty()) continue;
         GpuCtx &gc = h->gpus[gi];
         Slot &g = gc.slot[0];
@@ -2243,6 +2254,7 @@ int locate_pairs(sw_handle *h, const uint32_t *row, const uint64_t *index, size_
         for (const auto &p : w) max_cols = std::max(max_cols, bt.lens[index[p.second]]);
         const size_t fit = kLocateScratchBytes / (2 * sizeof(int32_t) * (size_t)max_cols) / 128 * 128;
         const size_t threads = std::max<size_t>(128, std::min((m + 127) / 128 * 128, fit));
+        work[gi].fit = std::max<size_t>(128, fit);
         SW_CUDA(h, cudaSetDevice(gc.dev));
         // staging: [m pairs {row, shard-local subject}][m scores][m coordinate quadruples]
         SW_CUDA(h, gc.h_loc.reserve(m * (sizeof(uint2) + sizeof(int32_t) + sizeof(uint4))));
@@ -2253,7 +2265,7 @@ int locate_pairs(sw_handle *h, const uint32_t *row, const uint64_t *index, size_
         SW_CUDA(h, gc.d_loc_coord.reserve(m * sizeof(uint4)));
         SW_CUDA(h, gc.d_loc_scratch.reserve(2 * sizeof(int32_t) * (size_t)max_cols * threads));
         SW_CUDA(h, cudaMemcpyAsync(gc.d_loc_pair.p, hp, m * sizeof(uint2), cudaMemcpyHostToDevice, gc.st_compute));
-        SwLocateLaunch L;
+        SwLocateLaunch &L = work[gi].L;
         L.db = dev_db(g); L.raw_bytes = g.d_raw.cap;
         L.q = dev_queries(h, gc); L.q_bytes = gc.d_qpacked.cap;
         L.sc = sc;
@@ -2269,21 +2281,160 @@ int locate_pairs(sw_handle *h, const uint32_t *row, const uint64_t *index, size_
         SW_CUDA(h, cudaMemcpyAsync((char *)gc.h_loc.p + m * (sizeof(uint2) + sizeof(int32_t)), gc.d_loc_coord.p,
                                    m * sizeof(uint4), cudaMemcpyDeviceToHost, gc.st_compute));
     }
-    for (size_t gi = 0; gi < ng; ++gi) {
-        const auto &w = work[gi];
+    return SW_OK;
+}
+
+// The located scores and coordinates of GPU gi's m pairs in h_loc, in work order (valid once its compute stream is done).
+const int32_t *located_scores(GpuCtx &gc, size_t m) { return (const int32_t *)((const char *)gc.h_loc.p + m * sizeof(uint2)); }
+const uint32_t *located_coords(GpuCtx &gc, size_t m) { return (const uint32_t *)(located_scores(gc, m) + m); }
+
+// sw_locate_db: enqueue_locate, then the results scattered into the caller's order.
+int locate_pairs(sw_handle *h, const uint32_t *row, const uint64_t *index, size_t n, int32_t *score, uint32_t *coord)
+{
+    std::vector<LocateWork> work;
+    SW_TRY(enqueue_locate(h, row, index, n, work));
+    std::memset(score, 0, n * sizeof(int32_t));
+    std::memset(coord, 0, 4 * n * sizeof(uint32_t));
+    for (size_t gi = 0; gi < work.size(); ++gi) {
+        const auto &w = work[gi].w;
         if (w.empty()) continue;
         GpuCtx &gc = h->gpus[gi];
         SW_CUDA(h, cudaSetDevice(gc.dev));
         SW_CUDA(h, cudaStreamSynchronize(gc.st_compute));
         const size_t m = w.size();
-        const int32_t *hs = (const int32_t *)((const char *)gc.h_loc.p + m * sizeof(uint2));
-        const uint32_t *hc = (const uint32_t *)(hs + m);
+        const int32_t *hs = located_scores(gc, m);
+        const uint32_t *hc = located_coords(gc, m);
         for (size_t k = 0; k < m; ++k) {
             score[w[k].second] = hs[k];
             std::memcpy(coord + 4 * w[k].second, hc + 4 * k, 4 * sizeof(uint32_t));
         }
     }
     if (device_error_bits(h)) return SW_EDEVICE;
+    return SW_OK;
+}
+
+// sw_align_db: enqueue_locate; then, per GPU, the coordinates are read back and the pairs split into rounds whose
+// direction bits fit h->align_scratch, one align launch per round; then the ops are scattered into the caller's order
+// and compacted.  Nothing reaches the caller's arrays unless the whole call succeeds (SW_ECAPACITY writes *count).
+int align_pairs(sw_handle *h, const uint32_t *row, const uint64_t *index, size_t n, int32_t *score, uint32_t *coord,
+                uint64_t *cigar_off, uint32_t *cigar, size_t cap, size_t *count)
+{
+    std::vector<LocateWork> work;
+    SW_TRY(enqueue_locate(h, row, index, n, work));
+    const size_t ng = work.size();
+    // per GPU: rounds [k0, k1) of the work order, with their direction words; staging in h_aln:
+    // [m direction offsets][m op-slot offsets] in, then [m op counts][ops] out
+    std::vector<std::vector<std::pair<size_t, uint64_t>>> rounds(ng);   // (k1, words of the round)
+    std::vector<uint64_t> total_ops(ng, 0), offs;
+    bool too_big = false;
+    for (size_t gi = 0; gi < ng; ++gi) {
+        const size_t m = work[gi].w.size();
+        if (m == 0) continue;
+        GpuCtx &gc = h->gpus[gi];
+        SW_CUDA(h, cudaSetDevice(gc.dev));
+        SW_CUDA(h, cudaStreamSynchronize(gc.st_compute));
+        const int32_t *hs = located_scores(gc, m);
+        const uint32_t *hc = located_coords(gc, m);
+        offs.resize(2 * m);
+        uint64_t *toff = offs.data(), *ooff = toff + m;
+        const uint64_t budget = h->align_scratch / sizeof(uint64_t);
+        uint64_t words = 0, ops = 0;
+        for (size_t k = 0; k < m; ++k) {
+            const uint64_t qm = hc[4 * k + 1] - hc[4 * k], sn = hc[4 * k + 3] - hc[4 * k + 2];
+            const uint64_t pw = hs[k] > 0 ? (qm + 15) / 16 * sn : 0;
+            if (pw > budget) too_big = true;
+            if (words + pw > budget) { rounds[gi].emplace_back(k, words); words = 0; }
+            toff[k] = words; ooff[k] = ops;
+            words += pw;
+            ops += hs[k] > 0 ? qm + sn - 1 : 0;
+        }
+        rounds[gi].emplace_back(m, words);
+        total_ops[gi] = ops;
+        SW_CUDA(h, gc.h_aln.reserve(std::max(2 * m * sizeof(uint64_t), (m + ops) * sizeof(uint32_t))));
+        std::memcpy(gc.h_aln.p, offs.data(), 2 * m * sizeof(uint64_t));
+    }
+    if (too_big) return SW_ERANGE;
+    for (size_t gi = 0; gi < ng; ++gi) {
+        const size_t m = work[gi].w.size();
+        if (m == 0) continue;
+        GpuCtx &gc = h->gpus[gi];
+        SW_CUDA(h, cudaSetDevice(gc.dev));
+        uint64_t max_words = 0;
+        for (const auto &r : rounds[gi]) max_words = std::max(max_words, r.second);
+        SW_CUDA(h, gc.d_aln_off.reserve(2 * m * sizeof(uint64_t)));
+        SW_CUDA(h, gc.d_aln_trace.reserve(max_words * sizeof(uint64_t)));
+        SW_CUDA(h, gc.d_aln_ops.reserve(total_ops[gi] * sizeof(uint32_t)));
+        SW_CUDA(h, gc.d_aln_nops.reserve(m * sizeof(uint32_t)));
+        SW_CUDA(h, cudaMemcpyAsync(gc.d_aln_off.p, gc.h_aln.p, 2 * m * sizeof(uint64_t), cudaMemcpyHostToDevice,
+                                   gc.st_compute));
+        SwAlignLaunch A;
+        A.loc = work[gi].L;
+        A.trace_off = gc.d_aln_off.as<uint64_t>(); A.ops_off = A.trace_off + m;
+        A.trace = gc.d_aln_trace.as<uint64_t>(); A.trace_words = max_words;
+        A.ops = gc.d_aln_ops.as<uint32_t>(); A.ops_elems = total_ops[gi];
+        A.nops = gc.d_aln_nops.as<uint32_t>();
+        size_t k0 = 0;
+        for (const auto &r : rounds[gi]) {
+            const size_t k1 = r.first;
+            if (k1 > k0) {
+                A.job0 = (uint32_t)k0; A.job1 = (uint32_t)k1;
+                A.loc.threads_total = (int)std::max<size_t>(128, std::min((k1 - k0 + 127) / 128 * 128, work[gi].fit));
+                SW_CUDA(h, sw_launch_align(gc.st_compute, A));
+                h->launches++;
+            }
+            k0 = k1;
+        }
+        // read back in place of the offsets, after their upload on the same stream: [m op counts][ops]
+        SW_CUDA(h, cudaMemcpyAsync(gc.h_aln.p, gc.d_aln_nops.p, m * sizeof(uint32_t), cudaMemcpyDeviceToHost, gc.st_compute));
+        if (total_ops[gi])
+            SW_CUDA(h, cudaMemcpyAsync((uint32_t *)gc.h_aln.p + m, gc.d_aln_ops.p, total_ops[gi] * sizeof(uint32_t),
+                                       cudaMemcpyDeviceToHost, gc.st_compute));
+    }
+    // every pair's op count, then the total; ops[i] points at pair i's ops in some GPU's staging
+    std::vector<uint32_t> nops(n, 0);
+    std::vector<const uint32_t *> src(n, nullptr);
+    for (size_t gi = 0; gi < ng; ++gi) {
+        const auto &w = work[gi].w;
+        const size_t m = w.size();
+        if (m == 0) continue;
+        GpuCtx &gc = h->gpus[gi];
+        SW_CUDA(h, cudaSetDevice(gc.dev));
+        SW_CUDA(h, cudaStreamSynchronize(gc.st_compute));
+        const int32_t *hs = located_scores(gc, m);
+        const uint32_t *hc = located_coords(gc, m);
+        const uint32_t *hn = (const uint32_t *)gc.h_aln.p, *hops = hn + m;
+        uint64_t off = 0;                              // op slots in work order, as planned
+        for (size_t k = 0; k < m; ++k) {
+            if (hs[k] <= 0) continue;
+            const uint64_t slot = (uint64_t)(hc[4 * k + 1] - hc[4 * k]) + (hc[4 * k + 3] - hc[4 * k + 2]) - 1;
+            nops[w[k].second] = (uint32_t)std::min<uint64_t>(hn[k], slot);
+            src[w[k].second] = hops + off;
+            off += slot;
+        }
+    }
+    if (device_error_bits(h)) return SW_EDEVICE;
+    size_t total = 0;
+    for (size_t i = 0; i < n; ++i) total += nops[i];
+    *count = total;
+    if (cap < total) return SW_ECAPACITY;
+    std::memset(score, 0, n * sizeof(int32_t));
+    std::memset(coord, 0, 4 * n * sizeof(uint32_t));
+    for (size_t gi = 0; gi < ng; ++gi) {
+        const auto &w = work[gi].w;
+        const size_t m = w.size();
+        if (m == 0) continue;
+        const int32_t *hs = located_scores(h->gpus[gi], m);
+        const uint32_t *hc = located_coords(h->gpus[gi], m);
+        for (size_t k = 0; k < m; ++k) {
+            score[w[k].second] = hs[k];
+            std::memcpy(coord + 4 * w[k].second, hc + 4 * k, 4 * sizeof(uint32_t));
+        }
+    }
+    cigar_off[0] = 0;
+    for (size_t i = 0; i < n; ++i) {
+        if (nops[i]) std::memcpy(cigar + cigar_off[i], src[i], nops[i] * sizeof(uint32_t));
+        cigar_off[i + 1] = cigar_off[i] + nops[i];
+    }
     return SW_OK;
 }
 
@@ -2382,6 +2533,8 @@ int sw_init(sw_handle_t **out, const sw_params_t *p, const int *gpu_ids, int n_g
     if (const char *e = std::getenv("SW_B200_STICKY")) h->sticky = std::atoi(e);
     if (const char *e = std::getenv("SW_B200_PASS_SPLIT")) h->pass_split = std::atoi(e);
     if (const char *e = std::getenv("SW_B200_SUPERBLOCK_MB")) h->superblock_mb = std::max(0.01, std::atof(e));
+    if (const char *e = std::getenv("SW_B200_ALIGN_SCRATCH_MB"))
+        h->align_scratch = std::max<size_t>(sizeof(uint64_t), (size_t)(std::atof(e) * 1048576.0));
     h->gpus.resize(ids.size());
     for (size_t i = 0; i < ids.size(); ++i) {
         GpuCtx &g = h->gpus[i];
@@ -2524,6 +2677,27 @@ int sw_locate_db(sw_handle_t *h, const uint32_t *row, const uint64_t *index, siz
         if (row[i] >= rows || index[i] >= bt.ns) return SW_EINVAL;
     if (n == 0) return SW_OK;
     return locate_pairs(h, row, index, n, score, coord);
+}
+
+int sw_align_db(sw_handle_t *h, const uint32_t *row, const uint64_t *index, size_t n, int32_t *score, uint32_t *coord,
+                uint64_t *cigar_off, uint32_t *cigar, size_t cap, size_t *count)
+{
+    // as sw_locate_db, plus the CIGAR arrays: cigar may be NULL only for the size query (cap == 0)
+    if (!h || (n > 0 && (!row || !index || !score || !coord || !cigar_off || !count)) || (cap > 0 && !cigar) ||
+        h->params.score_width != 0)
+        return SW_EINVAL;
+    if (h->n_inflight) return SW_EAGAIN;
+    const Batch &bt = h->batch[0];
+    if (!bt.loaded || !bt.resident) return SW_ESTATE;
+    const size_t rows = h->q_len.size();
+    for (size_t i = 0; i < n; ++i)
+        if (row[i] >= rows || index[i] >= bt.ns) return SW_EINVAL;
+    if (n == 0) {
+        if (cigar_off) cigar_off[0] = 0;
+        if (count) *count = 0;
+        return SW_OK;
+    }
+    return align_pairs(h, row, index, n, score, coord, cigar_off, cigar, cap, count);
 }
 
 int sw_set_queries(sw_handle_t *h, const uint8_t *packed, const uint32_t *len, const uint64_t *off, int nq)

@@ -4,7 +4,7 @@
  *
  *   sw_b200_cli -q query.fa -l library.fa [-t seconds] [-o out.txt] [-R score.txt]
  *               [-m match] [-x mismatch] [-g gap_open] [-e gap_extend] [-w score_width] [-G ngpus]
- *               [-T min_score] [-B] [-L]
+ *               [-T min_score] [-B] [-L] [-A]
  *
  * Without -o / -R it prints, like main_test, "result: %d, biased: %d" for every pair
  * (biased = score + 2048, the RTL's ZERO offset).  -T scores in hit-list mode (sw_set_hits) and prints
@@ -14,7 +14,8 @@
  * with none of -o / -R / -T.  -L (with -T or -B only) scores the library as a resident database
  * (sw_load_db, sw_score_db) and appends to each of those lines where the best alignment of the pair lies
  * (sw_locate_db), 1-based and inclusive like ssearch36 prints it: " query %u-%u subject %u-%u"
- * (0-0 for a score of 0).
+ * (0-0 for a score of 0).  -A (with -T or -B only; implies -L) also appends how it aligns (sw_align_db):
+ * " cigar <CIGAR>" in SAM's text with the query as the read, "*" for a score of 0.
  */
 #include "../../include/sw_b200.h"
 
@@ -26,7 +27,7 @@ static void usage(const char *n)
 {
     fprintf(stderr, "Usage: %s -q <query.fa> -l <library.fa> [-t timeout_s] [-o out.txt] [-R score.txt]\n"
                     "          [-m match] [-x mismatch] [-g gap_open] [-e gap_extend] [-w score_width] [-G ngpus]\n"
-                    "          [-T min_score] [-B] [-L]\n", n);
+                    "          [-T min_score] [-B] [-L] [-A]\n", n);
 }
 
 /* " query b-e subject b-e" of a located pair: 1-based, inclusive; 0-0 for a score of 0 */
@@ -36,22 +37,45 @@ static void print_span(int32_t score, const uint32_t *c)
     else printf(" query 0-0 subject 0-0");
 }
 
+/* sw_locate_db; with -A sw_align_db, its CIGAR buffer sized by sum(query + subject length), which always suffices */
+static int locate_pairs(sw_handle_t *h, const sw_seqset_t *q, const sw_seqset_t *db, const uint32_t *row,
+                        const uint64_t *index, size_t n, int align, int32_t *score, uint32_t *coord, uint64_t **off,
+                        uint32_t **ops)
+{
+    size_t cap = 0, count = 0, i;
+    if (!align) return sw_locate_db(h, row, index, n, score, coord);
+    for (i = 0; i < n; ++i) cap += (size_t)q->len[row[i]] + db->len[index[i]];
+    *off = (uint64_t *)malloc((n + 1) * sizeof **off);
+    *ops = (uint32_t *)malloc((cap + 1) * sizeof **ops);
+    if (!*off || !*ops) return SW_ENOMEM;
+    return sw_align_db(h, row, index, n, score, coord, *off, *ops, cap, &count);
+}
+
+/* " cigar <CIGAR>" of aligned pair i: SAM text of its BAM ops, "*" for none */
+static void print_cigar(const uint64_t *off, const uint32_t *ops, size_t i)
+{
+    uint64_t k;
+    printf(" cigar ");
+    if (off[i] == off[i + 1]) printf("*");
+    for (k = off[i]; k < off[i + 1]; ++k) printf("%u%c", ops[k] >> 4, "MIDNSHP=X"[ops[k] & 15]);
+}
+
 int main(int argc, char **argv)
 {
     const char *qf = NULL, *lf = NULL, *of = NULL, *rf = NULL;
-    int timeout_s = 10, ngpus = 1, opt, rc, i, min_score = 0, subject_best = 0, locate = 0;
+    int timeout_s = 10, ngpus = 1, opt, rc, i, min_score = 0, subject_best = 0, locate = 0, align = 0;
     sw_params_t p;
     sw_handle_t *h = NULL;
     sw_seqset_t *q = NULL, *db = NULL;
     int32_t *scores = NULL, *hscore = NULL, *bscore = NULL, *bsecond = NULL, *lscore = NULL;
-    uint32_t *hrow = NULL, *brow = NULL, *lcoord = NULL;
-    uint64_t *hindex = NULL, *bindex = NULL;
+    uint32_t *hrow = NULL, *brow = NULL, *lcoord = NULL, *aops = NULL;
+    uint64_t *hindex = NULL, *bindex = NULL, *aoff = NULL;
     size_t nhits = 0;
     int gpu_ids[64];
     static struct option lo[] = {{"timeout", required_argument, 0, 't'}, {"query", required_argument, 0, 'q'},
                                  {"library", required_argument, 0, 'l'}, {"help", no_argument, 0, 'h'}, {0, 0, 0, 0}};
     sw_default_params(&p);
-    while ((opt = getopt_long(argc, argv, "ht:q:l:o:R:m:x:g:e:w:G:T:BL", lo, NULL)) >= 0) {
+    while ((opt = getopt_long(argc, argv, "ht:q:l:o:R:m:x:g:e:w:G:T:BLA", lo, NULL)) >= 0) {
         switch (opt) {
             case 'q': qf = optarg; break;
             case 'l': lf = optarg; break;
@@ -67,6 +91,7 @@ int main(int argc, char **argv)
             case 'T': min_score = atoi(optarg); break;
             case 'B': subject_best = 1; break;
             case 'L': locate = 1; break;
+            case 'A': align = locate = 1; break;
             case 'h': usage(argv[0]); return 0;
             default: usage(argv[0]); return -1;
         }
@@ -83,7 +108,8 @@ int main(int argc, char **argv)
         return -1;
     }
     if (locate && min_score <= 0 && !subject_best) {
-        printf("-L locates the pairs -T or -B prints: it needs one of them\n");
+        printf(align ? "-A aligns the pairs -T or -B prints: it needs one of them\n"
+                     : "-L locates the pairs -T or -B prints: it needs one of them\n");
         usage(argv[0]);
         return -1;
     }
@@ -123,15 +149,16 @@ int main(int argc, char **argv)
             lscore = (int32_t *)malloc((nhits + 1) * sizeof *lscore);
             lcoord = (uint32_t *)malloc((nhits + 1) * 4 * sizeof *lcoord);
             if (!lscore || !lcoord) { rc = SW_ENOMEM; goto fail; }
-            if ((rc = sw_locate_db(h, hrow, hindex, nhits, lscore, lcoord)) != SW_OK) goto fail;
+            if ((rc = locate_pairs(h, q, db, hrow, hindex, nhits, align, lscore, lcoord, &aoff, &aops)) != SW_OK) goto fail;
         }
         for (i = 0; (size_t)i < nhits; ++i) {
             printf("%s x %s result: %d, biased: %d(0x%04x)", q->name[hrow[i]], db->name[hindex[i]],
                    (int)hscore[i], (int)hscore[i] + 2048, (unsigned)(hscore[i] + 2048));
             if (locate) print_span(lscore[i], lcoord + 4 * (size_t)i);
+            if (align) print_cigar(aoff, aops, (size_t)i);
             printf("\n");
         }
-        free(hrow); free(hindex); free(hscore); free(lscore); free(lcoord); sw_destroy(h); sw_seqset_free(q); sw_seqset_free(db);
+        free(hrow); free(hindex); free(hscore); free(lscore); free(lcoord); free(aoff); free(aops); sw_destroy(h); sw_seqset_free(q); sw_seqset_free(db);
         return 0;
     }
     if (subject_best) {
@@ -148,14 +175,15 @@ int main(int argc, char **argv)
             lcoord = (uint32_t *)malloc((db->n + 1) * 4 * sizeof *lcoord);
             if (!bindex || !lscore || !lcoord) { rc = SW_ENOMEM; goto fail; }
             for (i = 0; (size_t)i < db->n; ++i) bindex[i] = (uint64_t)i;
-            if ((rc = sw_locate_db(h, brow, bindex, db->n, lscore, lcoord)) != SW_OK) goto fail;
+            if ((rc = locate_pairs(h, q, db, brow, bindex, db->n, align, lscore, lcoord, &aoff, &aops)) != SW_OK) goto fail;
         }
         for (i = 0; (size_t)i < db->n; ++i) {
             printf("%s best %s result: %d, second: %d", db->name[i], q->name[brow[i]], (int)bscore[i], (int)bsecond[i]);
             if (locate) print_span(lscore[i], lcoord + 4 * (size_t)i);
+            if (align) print_cigar(aoff, aops, (size_t)i);
             printf("\n");
         }
-        free(bscore); free(bsecond); free(brow); free(bindex); free(lscore); free(lcoord); sw_destroy(h); sw_seqset_free(q); sw_seqset_free(db);
+        free(bscore); free(bsecond); free(brow); free(bindex); free(lscore); free(lcoord); free(aoff); free(aops); sw_destroy(h); sw_seqset_free(q); sw_seqset_free(db);
         return 0;
     }
     scores = (int32_t *)calloc(q->n * db->n + 1, sizeof(int32_t));
@@ -191,6 +219,6 @@ fail:
     if (rc == SW_ECUDA) printf(" [%s]", sw_last_cuda_error_string(h));
     printf("\n");
     free(scores); free(hrow); free(hindex); free(hscore); free(bscore); free(bsecond); free(brow); free(bindex); free(lscore); free(lcoord);
-    sw_destroy(h); sw_seqset_free(q); sw_seqset_free(db);
+    free(aoff); free(aops); sw_destroy(h); sw_seqset_free(q); sw_seqset_free(db);
     return -1;
 }

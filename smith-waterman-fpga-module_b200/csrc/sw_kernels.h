@@ -257,6 +257,24 @@ struct SwLocateLaunch {
 };
 cudaError_t sw_launch_locate(cudaStream_t st, const SwLocateLaunch &L);
 
+/* CIGAR of the located best alignment of selected pairs (sw_locate.cu, sw_align_db): one thread per pair of
+ * loc.pairs[job0 .. job1).  loc.score / loc.coord hold sw_launch_locate's results for those pairs (read here).  Each
+ * pair with score > 0 stores 4 direction bits per cell of its rectangle in trace[trace_off[i] ..], ceil(m / 16) * n
+ * words for an m x n rectangle, and writes its run-length BAM ops to ops[ops_off[i] ..], at most m + n - 1 of them,
+ * and their count to nops[i] (0 for score 0).  loc.scratch as for sw_launch_locate. */
+struct SwAlignLaunch {
+    SwLocateLaunch loc{};
+    uint32_t job0 = 0, job1 = 0;
+    const uint64_t *trace_off = nullptr;
+    uint64_t *trace = nullptr;
+    uint64_t trace_words = 0;
+    const uint64_t *ops_off = nullptr;
+    uint32_t *ops = nullptr;
+    uint64_t ops_elems = 0;
+    uint32_t *nops = nullptr;
+};
+cudaError_t sw_launch_align(cudaStream_t st, const SwAlignLaunch &L);
+
 cudaError_t sw_launch_build_tp(cudaStream_t st, const SwDevDb &db);
 
 /* Per-query arg-max over subjects of a materialised int32 matrix (first index reaching the max). */
